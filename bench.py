@@ -14,6 +14,8 @@ Timed with CUDA events on the library's stream (pcb_timer_*), max over ranks, in
   lobpcg      seconds to converge the lowest 10 bands (tol 1e-4) for the rank's k-points, warm-started like bandgap()
   passes      device time of each of the five kernels of one block apply (pcb_apply_timed)
   cpu_baseline the oracle's NumPy/pocketfft restatement of the same apply on the host cores (bounded sample)
+With --dump-outputs DIR, rank 0 also writes the result of the last timed step to DIR (see dump_outputs): the inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import importlib
@@ -219,6 +221,20 @@ def timed_passes(pcb, op, X, Y, m, reps=5):
         L.check(L.lib().pcb_apply_timed(op.h, L.APPLY_H, m, L.ptr_array(X.ptrs), L.ptr_array(Y.ptrs), buf, C.byref(npass)), "pcb_apply_timed")
         acc += np.array(buf[:8])
     return [float(v) / reps for v in acc[:npass.value]]
+
+
+def dump_outputs(out_dir, Y, seed=0):
+    """Writes the result of the last timed step, Y = H X (R x m complex128 on the device), as float64 .npy files:
+      H_X_sample.npy        (rows, m, 2) real and imaginary parts of Y at `rows` sorted row indices drawn with a fixed seed
+                            (32 MiB: 131072 rows at m = 16), the same rows for the same N and m in every run
+      H_X_column_norms.npy  (m,) the 2-norm of every column of the whole of Y"""
+    Yh = Y.get()
+    R, m = Yh.shape
+    rows = min(R, (32 << 20) // (16 * m))
+    idx = np.sort(np.random.default_rng(seed).choice(R, size=rows, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "H_X_sample.npy"), np.ascontiguousarray(Yh[idx]).view(np.float64).reshape(rows, m, 2))
+    np.save(os.path.join(out_dir, "H_X_column_norms.npy"), np.linalg.norm(Yh, axis=0))
 
 
 def paper2_dielectric_leg(pcb, ctx, n, m, steps, warmup, peak):
@@ -448,7 +464,13 @@ def main():
     ap.add_argument("--no-paper2", action="store_true", help="skip the Paper-2 dielectric legs")
     ap.add_argument("--no-large-grid", action="store_true", help="N > 1: skip the large-grid (NCCL) leg")
     ap.add_argument("--cpu-full", action="store_true", help="CPU baseline per SURVEY 8(d): also the C1 solve (N=48) and 3 LOBPCG iterations at N=120 on the host")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step (seeded row sample + column norms, float64 .npy) to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.mode == "large-grid"):
+        ap.error("--dump-outputs applies to the CUDA k-path benchmark only")
     if args.impl == "reference":
         return run_reference(args)
     if args.mode == "large-grid":
@@ -484,6 +506,8 @@ def main():
     launches = ctx.launches() - l0
     dist.barrier()
     ms_total = dist.max(ms_total)
+    if args.dump_outputs and dist.rank == 0:
+        dump_outputs(args.dump_outputs, Y)
     if sampler:      # keep the identical load running so that nvidia-smi (50 ms period) gets enough samples of this workload
         t_end = time.perf_counter() + 0.6
         while time.perf_counter() < t_end:
