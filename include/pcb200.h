@@ -99,9 +99,10 @@ int pcb_op_create(pcb_ctx* ctx, const double* tables, double gamma, double shift
 int pcb_op_update(pcb_op* op, const double* tables, double gamma, double shift, double pshift, pcb_diel* diel);
 void pcb_op_destroy(pcb_op* op);
 
-/* Y_j = op(X_j), j < ncols.  in[j] == out[j] (in place) is allowed for every mode except PCB_APPLY_H (which re-reads X in
- * its last pass), PCB_APPLY_A / PCB_APPLY_M with the cross-DoF dielectric (out serves as work space of the plane halves / the
- * stencil gathers); the call fails with -2 in those cases.  Distinct columns must not overlap. */
+/* Y_j = op(X_j), j < ncols.  in[j] == out[j] (in place) is allowed for every mode except PCB_APPLY_H outside the plane mode
+ * (which re-reads X in its last pass), PCB_APPLY_A with the cross-DoF dielectric on the plane halves and PCB_APPLY_M with the
+ * cross-DoF dielectric (out serves as work space of the plane halves / the stencil gathers); the call fails with -2 in those
+ * cases, before anything is enqueued: no output column is written.  Distinct columns must not overlap. */
 int pcb_apply(pcb_op* op, int mode, int ncols, const void* const* in, void* const* out);
 
 /* Y_host = op(X_host): the reference-facing call with host arrays -- x_host, y_host are the reference's row-major (3N^3, k)
@@ -151,6 +152,10 @@ int pcb_update_resid(pcb_op* op, int m, int nl, void* const* s, void* const* hs,
 int pcb_update_resid_start(pcb_op* op, int m, int nl, void* const* s, void* const* hs, void* const* p_out, void* const* hp_out, const void* E,
                            const double* lambda, void* const* w_out);
 int pcb_update_resid_wait(pcb_op* op, int m, double* norms2);
+/* the last tiled block kernel pcb_gram2 / pcb_gram2_top / pcb_update / pcb_update_resid planned on this context: its name (e.g.
+ * "k_gram2", "k_update<32,1,3>", "k_update_res"), the CTAs it was launched with and the row tiles they share (test and measurement
+ * aid: which instantiation and how many tiles per CTA a shape selects) */
+int pcb_block_launch_info(pcb_ctx* ctx, char* name, int cap, long long* grid, long long* tiles);
 /* out[j] = a_j^H b_j (complex128 on the host) -- diag(x^H y) of numerical_experiments.py:105-111, environment.dots */
 int pcb_coldots(pcb_ctx* ctx, int ncols, const void* const* a, const void* const* b, void* out);
 /* y_j = alpha x_j + beta y_j */

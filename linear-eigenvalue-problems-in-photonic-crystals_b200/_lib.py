@@ -62,6 +62,7 @@ SIGNATURES = {
     "pcb_update_resid": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_void_pp, c_void_pp, c_void_pp, c_void_pp, C.c_void_p, c_double_p, c_void_pp, c_double_p]),
     "pcb_update_resid_start": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_void_pp, c_void_pp, c_void_pp, c_void_pp, C.c_void_p, c_double_p, c_void_pp]),
     "pcb_update_resid_wait": (C.c_int, [C.c_void_p, C.c_int, c_double_p]),
+    "pcb_block_launch_info": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]),
     "pcb_coldots": (C.c_int, [C.c_void_p, C.c_int, c_void_pp, c_void_pp, C.c_void_p]),
     "pcb_axpby": (C.c_int, [C.c_void_p, C.c_int, c_void_pp, c_void_pp, C.c_double, C.c_double]),
     "pcb_geometry_mask": (C.c_int, [C.c_void_p, C.c_int, c_double_p, C.c_void_p, C.c_void_p]),

@@ -88,6 +88,8 @@ struct pcb_ctx {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     cudaEvent_t order_ev[PCB_ORDER_EVENTS] = {};   // pcb_ctx_record / pcb_ctx_wait: stream ordering between contexts, created on first use
     long long launches = 0;
+    char blk_name[32] = "";         // the last tiled block kernel (Gram / update) planned on this context: pcb_block_launch_info
+    long long blk_grid = 0, blk_tiles = 0;
     int sms = 148;
     int use_plane = 1;              // PCB200_PLANE=0 forces the five-pass operator (A/B measurements)
     int use_plane_coupled = 1;      // PCB200_PLANE_COUPLED=0: coupled 3x3 dielectric on the five-pass path
@@ -147,6 +149,11 @@ static int ensure_dsmall(pcb_ctx* c, size_t bytes) { return ensure(c, &c->dsmall
 static int ensure_scratch(pcb_ctx* c, size_t bytes) { return ensure(c, (void**)&c->scratch, &c->scratch_bytes, bytes, false); }
 
 #define PCB_HOST_CH 8      // columns per pipeline chunk: 8 x 16 B = 128-byte rows, the narrowest 2-D copy that still runs at PCIe speed
+
+static void note_block(pcb_ctx* c, const char* name, long long grid, long long tiles) {
+    snprintf(c->blk_name, sizeof c->blk_name, "%s", name);
+    c->blk_grid = grid; c->blk_tiles = tiles;
+}
 
 static int grid_for(pcb_ctx* c, long long items, int per_block, int waves) {
     long long b = (items + per_block - 1) / per_block;
@@ -639,6 +646,25 @@ static int apply_structure(const pcb_op* o) {
     return diel == PCB_DIEL_CROSSDOF ? PCB_STRUCT_CROSS7 : PCB_STRUCT_FIVE;
 }
 
+// In-place columns (in[j] == out[j]) are refused where the pass structure re-reads X after writing `out` (H outside the plane
+// mode) or uses `out` as work space (cross-DoF plane halves, cross-DoF M).  Every column is checked before anything is enqueued:
+// a refused call returns -2 with all output columns untouched, also when the aliased column sits in a later launch chunk.
+static bool refuses_inplace_AH(int mode, int st) {
+    return (mode == PCB_APPLY_H && st != PCB_STRUCT_PLANE) || st == PCB_STRUCT_CROSS5 || st == PCB_STRUCT_CROSS4;
+}
+static int check_inplace(const pcb_op* o, int mode, int ncols, const void* const* in, void* const* out, const char* fn) {
+    bool refused = false;
+    if (mode == PCB_APPLY_M) refused = (o->d.diel == PCB_DIEL_CROSSDOF);
+    else if (mode == PCB_APPLY_A || mode == PCB_APPLY_H) refused = refuses_inplace_AH(mode, apply_structure(o));
+    if (!refused) return 0;
+    for (int j = 0; j < ncols; ++j)
+        if (in[j] == out[j]) {
+            pcb_set_error("%s: in[%d] == out[%d]; this mode re-reads X / uses out as work space here, use distinct columns", fn, j, j);
+            return -2;
+        }
+    return 0;
+}
+
 // A / H on kc columns (cols.in -> cols.out).  dist: the x passes read / write the slabs of all ranks through o->d.dist
 // (large-grid mode over peer memory); cols.in then holds the local X copies and cols.out local work columns.
 // (dist bit 0: the input columns are distributed, bit 1: the output columns are.)
@@ -651,7 +677,7 @@ static int apply_AH(pcb_op* o, int mode, PcbCols& cols, int kc, int j0, int dist
     const int last_t = (mode == PCB_APPLY_A) ? (dout ? PCB_PASS_XINV_A_TD : PCB_PASS_XINV_A_T) : (dout ? PCB_PASS_XINV_H_TD : PCB_PASS_XINV_H_T);
     int st = apply_structure(o);
     if (dist && c->zsplit) st = (o->d.diel == PCB_DIEL_CROSSDOF) ? PCB_STRUCT_CROSS7 : PCB_STRUCT_FIVE;      // no peer-memory x passes on split tiles
-    if ((mode == PCB_APPLY_H && st != PCB_STRUCT_PLANE) || st == PCB_STRUCT_CROSS5 || st == PCB_STRUCT_CROSS4 || dist)
+    if (refuses_inplace_AH(mode, st) || dist)      // (pcb_apply has checked all its columns already; pcb_apply_dist has not)
         for (int j = 0; j < kc; ++j)
             if (cols.in[j] == cols.out[j]) {
                 pcb_set_error("pcb_apply: in[%d] == out[%d]; this pass structure re-reads X / uses out as work space, use distinct columns", j0 + j, j0 + j);
@@ -715,6 +741,7 @@ int pcb_apply(pcb_op* o, int mode, int ncols, const void* const* in, void* const
         pcb_set_error("pcb_apply: mode %d needs whole columns; a slab context only supports PCB_APPLY_P (gather with pcb_slab_exchange)", mode);
         return -2;
     }
+    if (int rc = check_inplace(o, mode, ncols, in, out, "pcb_apply")) return rc;
     for (int j0 = 0; j0 < ncols; j0 += PCB_MAXC) {
         const int kc = (ncols - j0 < PCB_MAXC) ? ncols - j0 : PCB_MAXC;
         PcbCols cols;
@@ -741,10 +768,7 @@ int pcb_apply(pcb_op* o, int mode, int ncols, const void* const* in, void* const
                 c->launches++;
             } break;
             case PCB_APPLY_M:
-                if (cross) {
-                    for (int j = 0; j < kc; ++j) PCB_CHECK_ARG(cols.in[j] != cols.out[j], "cross-DoF dielectric cannot run in place");
-                    if (launch_crossdof(o, kc, cols.in, cols.out)) return -1;
-                }
+                if (cross && launch_crossdof(o, kc, cols.in, cols.out)) return -1;      // (in place refused by check_inplace)
                 for (int j = 0; j < kc && !cross; ++j) {
                     dim3 grid((unsigned)grid_for(c, c->nn, 256, 8), 1, 1);
                     PCB_LAUNCH(k_diel_point, grid, dim3(256, 1, 1), 0, c->stream, o->d, cols.in[j], cols.out[j]);
@@ -771,6 +795,7 @@ int pcb_apply(pcb_op* o, int mode, int ncols, const void* const* in, void* const
 int pcb_apply_timed(pcb_op* o, int mode, int ncols, const void* const* in, void* const* out, float* pass_ms, int* npass) {
     PCB_CHECK_ARG(o && in && out && pass_ms && npass && ncols > 0 && ncols <= PCB_MAXC, "bad arguments (ncols <= 32)");
     PCB_CHECK_ARG(mode == PCB_APPLY_A || mode == PCB_APPLY_H, "mode must be PCB_APPLY_A or PCB_APPLY_H");
+    if (int rc = check_inplace(o, mode, ncols, in, out, "pcb_apply_timed")) return rc;
     pcb_ctx* c = o->ctx;
     PCB_CUDA_OK(cudaSetDevice(c->device));
     PcbCols cols;
@@ -978,6 +1003,7 @@ int pcb_gram2_top(pcb_ctx* c, int n, int ntop, const void* const* s, const void*
         PCB_CUDA_OK(cudaGetLastError());
         c->launches++;
     }
+    note_block(c, "k_gram2", gx, ntiles);
     cplx* dout = (cplx*)c->dsmall;
     const int ne = 2 * nc * nc;
     PCB_LAUNCH(k_gram_finish, dim3((unsigned)((ne + 127) / 128), 1, 1), dim3(128, 1, 1), 0, c->stream, (const cplx*)c->partial, (int)gx, nt, ttop, dout);
@@ -1069,6 +1095,7 @@ static int update_impl(pcb_ctx* c, pcb_op* o, int m, int nl, void* const* s, voi
 #ifndef PCB_EMU
             if (smem_f > 48 * 1024) PCB_CUDA_OK(cudaFuncSetAttribute(k_update_res, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_f));
 #endif
+            note_block(c, "k_update_res", gxf, nt);
             PCB_LAUNCH(k_update_res, dim3((unsigned)gxf, 1, 1), dim3(PCB_UPDRES_THREADS, 1, 1), smem_f, c->stream, o->d, Sin, HSin, X, HX, P, HP, rs, dE, m, kx, kp, MPp, c->partial);
             PCB_CUDA_OK(cudaGetLastError());
             double* dout = c->partial + (size_t)gxf * 16;
@@ -1096,12 +1123,12 @@ static int update_impl(pcb_ctx* c, pcb_op* o, int m, int nl, void* const* s, voi
 #else
 #define PCB_UPD_GO(K) PCB_LAUNCH(K, grid, block, smem, c->stream, Sin, HSin, X, HX, P, HP, dE, m, kx, kp, MPp, c->R)
 #endif
-    if (deep) PCB_UPD_GO((k_update<32, 1, 3>));
-    else if (wide) PCB_UPD_GO((k_update<48, 1>));
-    else if (big && JW == 1) PCB_UPD_GO((k_update<32, 1>));
-    else if (big) PCB_UPD_GO((k_update<32, 2>));
-    else if (JW == 1) PCB_UPD_GO((k_update<16, 1>));
-    else PCB_UPD_GO((k_update<16, 2>));
+    if (deep) { PCB_UPD_GO((k_update<32, 1, 3>)); note_block(c, "k_update<32,1,3>", gx, ntiles); }
+    else if (wide) { PCB_UPD_GO((k_update<48, 1>)); note_block(c, "k_update<48,1>", gx, ntiles); }
+    else if (big && JW == 1) { PCB_UPD_GO((k_update<32, 1>)); note_block(c, "k_update<32,1>", gx, ntiles); }
+    else if (big) { PCB_UPD_GO((k_update<32, 2>)); note_block(c, "k_update<32,2>", gx, ntiles); }
+    else if (JW == 1) { PCB_UPD_GO((k_update<16, 1>)); note_block(c, "k_update<16,1>", gx, ntiles); }
+    else { PCB_UPD_GO((k_update<16, 2>)); note_block(c, "k_update<16,2>", gx, ntiles); }
     PCB_CUDA_OK(cudaGetLastError());
     c->launches++;
     if (o) {      // wide blocks: two kernels
@@ -1129,6 +1156,13 @@ int pcb_update_resid_wait(pcb_op* o, int m, double* norms2) {
         memcpy(norms2, (char*)c->hstage + sizeof(cplx) * 2 * PCB_MAXL * PCB_MAXL, sizeof(double) * m);
     } else memcpy(norms2, c->pending_norms, sizeof(double) * m);
     c->pending_state = 0;
+    return 0;
+}
+
+int pcb_block_launch_info(pcb_ctx* c, char* name, int cap, long long* grid, long long* tiles) {
+    PCB_CHECK_ARG(c && name && cap > 0 && grid && tiles, "bad arguments");
+    snprintf(name, (size_t)cap, "%s", c->blk_name);
+    *grid = c->blk_grid; *tiles = c->blk_tiles;
     return 0;
 }
 
