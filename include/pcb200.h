@@ -43,7 +43,9 @@ enum {
     PCB_APPLY_M = 5,     /* Diels(x) in real space          discretization.py:352-453                             */
     PCB_APPLY_KA = 6,    /* A_block_kernel(x, D_A)           pcfft.py:32-43 / _kernels.py:43-71                   */
     PCB_APPLY_KAH = 7,   /* A_block_kernel(x, -conj(D_A))    pcfft.py:148                                         */
-    PCB_APPLY_KB = 8     /* H_block_kernel(x, D_B) = gamma K_B x   pcfft.py:18-30,176 / _kernels.py:13-41         */
+    PCB_APPLY_KB = 8,    /* H_block_kernel(x, D_B) = gamma K_B x   pcfft.py:18-30,176 / _kernels.py:13-41         */
+    PCB_APPLY_DFIELD = 9, /* D = FFT3(K_A^H x): the real-space field of AMA (pcfft.py:148-149), natural layout        */
+    PCB_APPLY_EFIELD = 10 /* E = M D (the dielectric applied to that field), natural layout                          */
 };
 
 const char* pcb_last_error(void);
@@ -102,7 +104,9 @@ void pcb_op_destroy(pcb_op* op);
 /* Y_j = op(X_j), j < ncols.  in[j] == out[j] (in place) is allowed for every mode except PCB_APPLY_H outside the plane mode
  * (which re-reads X in its last pass), PCB_APPLY_A with the cross-DoF dielectric on the plane halves and PCB_APPLY_M with the
  * cross-DoF dielectric (out serves as work space of the plane halves / the stencil gathers); the call fails with -2 in those
- * cases, before anything is enqueued: no output column is written.  Distinct columns must not overlap. */
+ * cases, before anything is enqueued: no output column is written.  Distinct columns must not overlap.
+ * PCB_APPLY_DFIELD / PCB_APPLY_EFIELD (forward x, y, z passes; EFIELD then M point-wise in place on out, or the cross-DoF stencil
+ * from the context's scratch into out) read X only in their first pass: in place is allowed for every dielectric. */
 int pcb_apply(pcb_op* op, int mode, int ncols, const void* const* in, void* const* out);
 
 /* Y_host = op(X_host): the reference-facing call with host arrays -- x_host, y_host are the reference's row-major (3N^3, k)
@@ -120,6 +124,16 @@ int pcb_apply_host(pcb_op* op, int mode, int k, const void* x_host, long long ld
  * (x, y, z forward, stencil, z, y, x inverse), npass <- 7.
  * pass_ms must hold 8 floats.  Measurement aid for bench.py's per-pass roofline; not used by the solver. */
 int pcb_apply_timed(pcb_op* op, int mode, int ncols, const void* const* in, void* const* out, float* pass_ms, int* npass);
+
+/* Electric energy of modes in the dielectric.  For column x_j let D = FFT3(K_A^H x_j) (unnormalised, = PCB_APPLY_DFIELD) and
+ * E = M D, rows r = c N^3 + p:  e_tot[j] = Re sum_r conj(D_r) E_r / N^3 (= x_j^H A x_j, independent of gamma and the shift) and
+ * e_in[j] = the same sum over the rows in Omega_1 (bit c of the dielectric mask at cell p: the edge DoFs of ind_e); e_in = 0 without
+ * a dielectric.  e_in / e_tot is the fraction f of the mode's electric energy inside the dielectric (0 <= f <= 1 for the chiral M;
+ * the pseudochiral M couples rows, so a single row's term may be negative and f may leave [0, 1] slightly).  e_in, e_tot: HOST
+ * arrays of ncols doubles; x is read only.  Any ncols (launches of 32 columns); the reduction has a fixed grid and order, so a
+ * column gives the same bits at any width and on every call.  Runs the forward passes of A (the plane layout where A runs in plane
+ * mode, else the natural layout) into the context's scratch and a reduction kernel over them.  A slab context fails with -2. */
+int pcb_field_energy(pcb_op* op, int ncols, const void* const* x, double* e_in, double* e_tot);
 
 /* LOBPCG block kernels
  * pcb_residual: r_j = lambda_j x_j - hx_j (lobpcg.py:394-395); norms2[j] = ||r_j||^2 (environment.norms :131-143);

@@ -694,20 +694,17 @@ __global__ void __launch_bounds__(256) k_diel_point(PcbOp op, const cplx* __rest
 
 // K > 0: 2K taps known at compile time (K = 1 is the reference's default, discretization.py:403); K = 0: runtime st.k.
 // One thread per grid point and column (blockIdx.y): all three output components (gather form); out of place.
+// The gather at one grid point p of the natural layout: y = (M X)(p) from the point's own values d[c] = X[c nn + p] and its
+// stencil neighbours; mp = mask byte of p.  Shared by k_diel_crossdof and k_field_energy.
 template <int K>
-__global__ void __launch_bounds__(256) k_diel_crossdof(PcbOp op, PcbStencil st, PcbCols cols) {
+PCB_D void pcb_crossdof_gather(const PcbOp& op, const PcbStencil& st, const cplx* __restrict__ X, long long p, unsigned mp,
+                               const cplx d[3], cplx y[3]) {
     const int N = op.N;
     const long long nn = op.nn;
-    const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= nn) return;
-    const cplx* __restrict__ X = cols.in[blockIdx.y];
-    cplx* __restrict__ Y = cols.out[blockIdx.y];
     const int i[3] = {(int)(p % N), (int)((p / N) % N), (int)(p / ((long long)N * N))};
     const long long stride[3] = {1, N, (long long)N * N};
-    const unsigned mp = __ldg(op.mask + p);
-    cplx y[3];
     PCB_UNROLL
-    for (int c = 0; c < 3; ++c) y[c] = cscale(X[c * nn + p], ((mp >> c) & 1u) ? op.ediag[c] : 1.0);
+    for (int c = 0; c < 3; ++c) y[c] = cscale(d[c], ((mp >> c) & 1u) ? op.ediag[c] : 1.0);
     // pairs (a,b): (0,1) c-axis 2, ct-axis 1;  (0,2) c-axis 2, ct-axis 0;  (1,2) c-axis 1, ct-axis 0
     constexpr int PA[3] = {0, 0, 1}, PB[3] = {1, 2, 2}, CAX[3] = {2, 2, 1}, TAX[3] = {1, 0, 0};
     const int kk = K > 0 ? K : st.k;
@@ -752,6 +749,21 @@ __global__ void __launch_bounds__(256) k_diel_crossdof(PcbOp op, PcbStencil st, 
         y[a] = cfma(e, sa, y[a]);
         y[b] = cfmac(e, sb, y[b]);
     }
+}
+
+// K > 0: 2K taps known at compile time (K = 1 is the reference's default, discretization.py:403); K = 0: runtime st.k.
+// One thread per grid point and column (blockIdx.y): all three output components (gather form); out of place.
+template <int K>
+__global__ void __launch_bounds__(256) k_diel_crossdof(PcbOp op, PcbStencil st, PcbCols cols) {
+    const long long nn = op.nn;
+    const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= nn) return;
+    const cplx* __restrict__ X = cols.in[blockIdx.y];
+    cplx* __restrict__ Y = cols.out[blockIdx.y];
+    const unsigned mp = __ldg(op.mask + p);
+    const cplx d[3] = {X[p], X[nn + p], X[2 * nn + p]};
+    cplx y[3];
+    pcb_crossdof_gather<K>(op, st, X, p, mp, d, y);
     PCB_UNROLL
     for (int c = 0; c < 3; ++c) Y[c * nn + p] = y[c];
 }
@@ -761,22 +773,19 @@ __global__ void __launch_bounds__(256) k_diel_crossdof(PcbOp op, PcbStencil st, 
 // cols.wrk (output of the forward half of the plane pass), writes cols.out (input of the inverse half).  For the Good-Thomas
 // plans (N = 72, 120) coord is multiplication by a constant mod N, so a +-1 neighbour along i1 is a constant slot shift and the
 // gathers of a warp (lanes along col) stay contiguous.
+// The gather at slot position pt of the plane-slot layout: y = (M X)(pt), d[c] = X[c nn + pt], mp = maskp[pt] (bits 0-3 are read).
+// Shared by k_diel_crossdof_t and k_field_energy_t.
 template <int K>
-__global__ void __launch_bounds__(256) k_diel_crossdof_t(PcbOp op, PcbStencil st, PcbCols cols) {
+PCB_D void pcb_crossdof_gather_t(const PcbOp& op, const PcbStencil& st, const cplx* __restrict__ X, long long pt, unsigned mp,
+                                 const cplx d[3], cplx y[3]) {
     const int N = op.N;
     const long long nn = op.nn;
-    const long long pt = (long long)blockIdx.x * blockDim.x + threadIdx.x;      // position in the slot layout
-    if (pt >= nn) return;
-    const cplx* __restrict__ X = cols.wrk[blockIdx.y];
-    cplx* __restrict__ Y = cols.out[blockIdx.y];
     const int* __restrict__ ctab = op.ctab;
     const int scol = (int)(pt % N), srow = (int)((pt / N) % N);
     const int i[3] = {(int)(pt / ((long long)N * N)), __ldg(ctab + scol), __ldg(ctab + 2 * N + srow)};
     const unsigned char* __restrict__ maskp = op.maskp;      // the byte mask in the same slot order (k_mask_plane): coalesced
-    const unsigned mp = __ldg(maskp + pt);
-    cplx y[3];
     PCB_UNROLL
-    for (int c = 0; c < 3; ++c) y[c] = cscale(X[c * nn + pt], ((mp >> c) & 1u) ? op.ediag[c] : 1.0);
+    for (int c = 0; c < 3; ++c) y[c] = cscale(d[c], ((mp >> c) & 1u) ? op.ediag[c] : 1.0);
     constexpr int PA[3] = {0, 0, 1}, PB[3] = {1, 2, 2}, CAX[3] = {2, 2, 1}, TAX[3] = {1, 0, 0};
     const int kk = K > 0 ? K : st.k;
     const int taps = 2 * kk;
@@ -815,8 +824,91 @@ __global__ void __launch_bounds__(256) k_diel_crossdof_t(PcbOp op, PcbStencil st
         y[a] = cfma(e, sa, y[a]);
         y[b] = cfmac(e, sb, y[b]);
     }
+}
+
+template <int K>
+__global__ void __launch_bounds__(256) k_diel_crossdof_t(PcbOp op, PcbStencil st, PcbCols cols) {
+    const long long nn = op.nn;
+    const long long pt = (long long)blockIdx.x * blockDim.x + threadIdx.x;      // position in the slot layout
+    if (pt >= nn) return;
+    const cplx* __restrict__ X = cols.wrk[blockIdx.y];
+    cplx* __restrict__ Y = cols.out[blockIdx.y];
+    const unsigned mp = __ldg(op.maskp + pt);
+    const cplx d[3] = {X[pt], X[nn + pt], X[2 * nn + pt]};
+    cplx y[3];
+    pcb_crossdof_gather_t<K>(op, st, X, pt, mp, d, y);
     PCB_UNROLL
     for (int c = 0; c < 3; ++c) Y[c * nn + pt] = y[c];
+}
+
+// ---- electric energy of a mode in the dielectric (pcb_field_energy) ------------------------------------------------------
+// Input: D = FFT3(K_A^H x) in real space, one column per blockIdx.y.  Per cell, E = M D is formed in registers and
+//   e_tot += Re sum_c conj(D_c) E_c,   e_in += the same over the components c whose bit c of the mask is set (edge DoF in Omega_1).
+// partial[(blockIdx.x * ncols + j) * 2 + {0: e_in, 1: e_tot}] = this CTA's sums for column j.  The grid-stride loop runs over a
+// grid that does not depend on ncols, and both reduction stages have a fixed order: a column gets the same bits at any width.
+// DIEL: 0 none (e_in = 0, no mask), 1 chiral, 2 trivial (point-wise, pcb_diel_point), 3 cross-DoF (the stencil gather; K as in
+// k_diel_crossdof).
+PCB_D void pcb_energy_block_store(double ein, double etot, double* __restrict__ partial, int ncols) {
+    __shared__ double red[8][2];
+    ein = pcb_warp_sum(ein);
+    etot = pcb_warp_sum(etot);
+    const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
+    if (lane == 0) { red[warp][0] = ein; red[warp][1] = etot; }
+    __syncthreads();
+    if (threadIdx.x < 2) {
+        double v = 0.0;
+        for (int w = 0; w < 8; ++w) v += red[w][threadIdx.x];
+        partial[((long long)blockIdx.x * ncols + blockIdx.y) * 2 + threadIdx.x] = v;
+    }
+}
+PCB_D void pcb_energy_point(const cplx d[3], const cplx y[3], unsigned m, double& ein, double& etot) {
+    PCB_UNROLL
+    for (int c = 0; c < 3; ++c) {
+        const double t = fma(d[c].x, y[c].x, d[c].y * y[c].y);
+        etot += t;
+        if ((m >> c) & 1u) ein += t;
+    }
+}
+
+// natural layout [c][i2][i1][i0] (after the x, y, z forward passes); mask: op.mask
+template <int DIEL, int K>
+__global__ void __launch_bounds__(256) k_field_energy(PcbOp op, PcbStencil st, PcbCols cols, int ncols, double* __restrict__ partial) {
+    const long long nn = op.nn;
+    const cplx* __restrict__ X = cols.in[blockIdx.y];
+    double ein = 0.0, etot = 0.0;
+    for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < nn; p += (long long)gridDim.x * blockDim.x) {
+        const cplx d[3] = {X[p], X[nn + p], X[2 * nn + p]};
+        const unsigned m = DIEL ? (unsigned)__ldg(op.mask + p) : 0u;
+        cplx y[3];
+        if (DIEL == 3) pcb_crossdof_gather<K>(op, st, X, p, m, d, y);
+        else {
+            y[0] = d[0]; y[1] = d[1]; y[2] = d[2];
+            if (DIEL) pcb_diel_point(op, DIEL == 1 ? (m & 7u) : m, y);
+        }
+        pcb_energy_point(d, y, m, ein, etot);
+    }
+    pcb_energy_block_store(ein, etot, partial, ncols);
+}
+
+// plane-slot layout W'[c][i0][row][col] (after the x-forward pass and the forward half of the plane pass); mask: op.maskp, the
+// byte mask in the same slot order (bits 0-3; the cross-DoF activity bits 4-6 are not read)
+template <int DIEL, int K>
+__global__ void __launch_bounds__(256) k_field_energy_t(PcbOp op, PcbStencil st, PcbCols cols, int ncols, double* __restrict__ partial) {
+    const long long nn = op.nn;
+    const cplx* __restrict__ X = cols.in[blockIdx.y];
+    double ein = 0.0, etot = 0.0;
+    for (long long pt = (long long)blockIdx.x * blockDim.x + threadIdx.x; pt < nn; pt += (long long)gridDim.x * blockDim.x) {
+        const cplx d[3] = {X[pt], X[nn + pt], X[2 * nn + pt]};
+        const unsigned m = DIEL ? (unsigned)__ldg(op.maskp + pt) : 0u;
+        cplx y[3];
+        if (DIEL == 3) pcb_crossdof_gather_t<K>(op, st, X, pt, m, d, y);
+        else {
+            y[0] = d[0]; y[1] = d[1]; y[2] = d[2];
+            if (DIEL) pcb_diel_point(op, DIEL == 1 ? (m & 7u) : (m & 15u), y);
+        }
+        pcb_energy_point(d, y, m, ein, etot);
+    }
+    pcb_energy_block_store(ein, etot, partial, ncols);
 }
 
 // Set-up for the fused stencil-on-load: bit 4 + c of the slot-ordered mask byte = "component c at this point has a non-zero

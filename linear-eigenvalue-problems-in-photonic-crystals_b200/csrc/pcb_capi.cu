@@ -113,6 +113,7 @@ struct pcb_diel {
     unsigned* mbits2;       // five-sweep plane pass: bit words in its item order (k_mask_bits2); else null
     unsigned char* maskp2;  // five-sweep plane pass, coupled dielectric: byte mask in its slot order (k_mask_plane2); else null
     unsigned char* maskp;   // plane mode, coupled dielectric: byte mask in plane-slot order (k_mask_plane); else null
+    unsigned char* maskp_fe; // the same mask for pcb_field_energy where maskp does not exist: built by its first call in the plane layout
     int zsplit;             // the plane-mode form (ctx->zsplit) the slot-ordered masks were built for
     double ediag[3];
     cplx eoff[3];
@@ -458,7 +459,7 @@ int pcb_diel_create(pcb_ctx* c, int kind, const int64_t* ind_e, long long n_e, c
     PCB_CHECK_ARG(out && kind >= PCB_DIEL_NONE && kind <= PCB_DIEL_CROSSDOF, "bad kind");
     PCB_CUDA_OK(cudaSetDevice(c->device));
     pcb_diel* d = new pcb_diel;
-    d->ctx = c; d->kind = kind; d->mask = nullptr; d->mbits = nullptr; d->mbits2 = nullptr; d->maskp = nullptr; d->maskp2 = nullptr;
+    d->ctx = c; d->kind = kind; d->mask = nullptr; d->mbits = nullptr; d->mbits2 = nullptr; d->maskp = nullptr; d->maskp2 = nullptr; d->maskp_fe = nullptr;
     for (int i = 0; i < 3; ++i) { d->ediag[i] = ediag ? ediag[i] : 1.0; d->eoff[i] = eoff ? cmake(eoff[2 * i], eoff[2 * i + 1]) : cmake(0.0, 0.0); }
     d->st.k = 1; for (int i = 0; i < 8; ++i) d->st.w[i] = 0.0;
     if (kind == PCB_DIEL_CROSSDOF) {
@@ -544,6 +545,7 @@ void pcb_diel_destroy(pcb_diel* d) {
     if (d->maskp) cudaFree(d->maskp);
     if (d->mbits2) cudaFree(d->mbits2);
     if (d->maskp2) cudaFree(d->maskp2);
+    if (d->maskp_fe) cudaFree(d->maskp_fe);
     delete d;
 }
 
@@ -649,6 +651,8 @@ static int apply_structure(const pcb_op* o) {
 // In-place columns (in[j] == out[j]) are refused where the pass structure re-reads X after writing `out` (H outside the plane
 // mode) or uses `out` as work space (cross-DoF plane halves, cross-DoF M).  Every column is checked before anything is enqueued:
 // a refused call returns -2 with all output columns untouched, also when the aliased column sits in a later launch chunk.
+// PCB_APPLY_DFIELD / PCB_APPLY_EFIELD read x only in their first pass (the cross-DoF stencil of EFIELD reads the forward passes'
+// output from the scratch), so they take in[j] == out[j] in every pass structure.
 static bool refuses_inplace_AH(int mode, int st) {
     return (mode == PCB_APPLY_H && st != PCB_STRUCT_PLANE) || st == PCB_STRUCT_CROSS5 || st == PCB_STRUCT_CROSS4;
 }
@@ -731,6 +735,30 @@ static int apply_AH(pcb_op* o, int mode, PcbCols& cols, int kc, int j0, int dist
     return 0;
 }
 
+// D = FFT3(K_A^H x) (DFIELD) or E = M D (EFIELD) in the natural layout: the forward x (with K_A^H), y and z passes, then for E
+// the point-wise M in place on out, or the cross-DoF stencil from the scratch into out.
+static int apply_field(pcb_op* o, int mode, const PcbCols& cols, int kc) {
+    pcb_ctx* c = o->ctx;
+    const bool stencil = (mode == PCB_APPLY_EFIELD && o->d.diel == PCB_DIEL_CROSSDOF);
+    PcbCols f = cols;
+    if (stencil) {
+        if (ensure_scratch(c, sizeof(cplx) * (size_t)c->R * (size_t)kc)) return -1;
+        for (int j = 0; j < kc; ++j) f.out[j] = c->scratch + (size_t)j * c->R;
+    }
+    const int fwd[3] = {PCB_PASS_XFWD_SYM, PCB_PASS_YFWD, PCB_PASS_ZFWD};
+    for (int i = 0; i < 3; ++i) if (c->plan->pass(o->d, f, kc, fwd[i], c->tw, c->stream, c->sms)) return -1;
+    c->launches += 3;
+    if (mode != PCB_APPLY_EFIELD || o->d.diel == PCB_DIEL_NONE) return 0;
+    if (stencil) return launch_crossdof(o, kc, f.out, cols.out);
+    for (int j = 0; j < kc; ++j) {
+        dim3 grid((unsigned)grid_for(c, c->nn, 256, 8), 1, 1);
+        PCB_LAUNCH(k_diel_point, grid, dim3(256, 1, 1), 0, c->stream, o->d, cols.out[j], cols.out[j]);
+        PCB_CUDA_OK(cudaGetLastError());
+        c->launches++;
+    }
+    return 0;
+}
+
 int pcb_apply(pcb_op* o, int mode, int ncols, const void* const* in, void* const* out) {
     PCB_CHECK_ARG(o && in && out && ncols > 0, "bad arguments");
     pcb_ctx* c = o->ctx;
@@ -775,6 +803,9 @@ int pcb_apply(pcb_op* o, int mode, int ncols, const void* const* in, void* const
                     PCB_CUDA_OK(cudaGetLastError());
                     c->launches++;
                 }
+                break;
+            case PCB_APPLY_DFIELD: case PCB_APPLY_EFIELD:
+                if (int rc = apply_field(o, mode, cols, kc)) return rc;
                 break;
             case PCB_APPLY_KA: case PCB_APPLY_KAH: case PCB_APPLY_KB: {
                 dim3 grid((unsigned)grid_for(c, c->nn, 256, 8), (unsigned)kc, 1);
@@ -838,6 +869,109 @@ int pcb_apply_timed(pcb_op* o, int mode, int ncols, const void* const* in, void*
     PCB_EV_FREE;
 #undef PCB_EV_FREE
     *npass = n;
+    return 0;
+}
+
+// ---- electric energy of modes in the dielectric -------------------------------------------------------------------
+// The slot-ordered byte mask the plane-layout energy kernel reads: the dielectric's own maskp where it has one (coupled M on
+// clusters, cross-DoF: bits 0-3 are k_mask_plane's), else built here once and kept until pcb_diel_destroy.
+static const unsigned char* energy_slot_mask(pcb_op* o) {
+    pcb_diel* d = o->diel;
+    if (d->maskp) return d->maskp;
+    if (d->maskp_fe) return d->maskp_fe;
+    pcb_ctx* c = o->ctx;
+    unsigned char* mp = nullptr;
+    if (cudaMalloc(&mp, (size_t)c->nn) != cudaSuccess) { (void)cudaGetLastError(); pcb_set_error("pcb_field_energy: cudaMalloc of the slot mask failed"); return nullptr; }
+    PcbOp tmp;
+    memset(&tmp, 0, sizeof tmp);
+    tmp.N = c->N; tmp.nn = c->nn; tmp.nloc = c->nloc; tmp.mask = d->mask; tmp.maskp = mp; tmp.zsplit = d->zsplit;
+    PcbCols none;
+    memset(&none, 0, sizeof none);
+    if (c->plan->pass(tmp, none, 1, PCB_PASS_MASKPLANE, c->tw, c->stream, c->sms)) { cudaStreamSynchronize(c->stream); cudaFree(mp); return nullptr; }
+    c->launches++;
+    d->maskp_fe = mp;
+    return mp;
+}
+
+// e_in / e_tot of kc columns: forward passes into the scratch (the plane layout where A / H run in plane mode, else the natural
+// layout), the energy kernel over a fixed grid of gx CTAs per column, then the fixed-order sum of the partials into `dout`.
+static int field_energy_chunk(pcb_op* o, const PcbCols& cols, int kc, int plane, const unsigned char* smask, int gx, double* dout) {
+    pcb_ctx* c = o->ctx;
+    const PcbOpLaunch* pl = c->plan;
+    PcbCols f = cols, e;
+    memset(&e, 0, sizeof e);
+    for (int j = 0; j < kc; ++j) {
+        cplx* s = c->scratch + (size_t)j * c->R;
+        f.wrk[j] = s; f.out[j] = s; e.in[j] = s;
+    }
+    PcbOp d = o->d;
+    if (plane) {
+        // x forward -> transposed scratch, forward half of the plane pass in place: real-space D in the plane-slot layout
+        if (pl->pass(d, f, kc, PCB_PASS_XFWD_SYM_T, c->tw, c->stream, c->sms)) return -1;
+        if (pl->pass(d, f, kc, PCB_PASS_MID_FWD, c->tw, c->stream, c->sms)) return -1;
+        d.maskp = smask;
+    } else {
+        const int fwd[3] = {PCB_PASS_XFWD_SYM, PCB_PASS_YFWD, PCB_PASS_ZFWD};
+        for (int i = 0; i < 3; ++i) if (pl->pass(d, f, kc, fwd[i], c->tw, c->stream, c->sms)) return -1;
+        c->launches++;
+    }
+    c->launches += 2;
+    const PcbStencil st = d.sten;
+    const int k = st.k;
+    dim3 grid((unsigned)gx, (unsigned)kc, 1), blk(256, 1, 1);
+    double* part = c->partial;
+#define PCB_FE_GO(KERN)                                                                                             \
+    do {                                                                                                            \
+        switch (d.diel) {                                                                                           \
+            case PCB_DIEL_NONE: PCB_LAUNCH((KERN<0, 1>), grid, blk, 0, c->stream, d, st, e, kc, part); break;       \
+            case PCB_DIEL_CHIRAL: PCB_LAUNCH((KERN<1, 1>), grid, blk, 0, c->stream, d, st, e, kc, part); break;     \
+            case PCB_DIEL_TRIVIAL: PCB_LAUNCH((KERN<2, 1>), grid, blk, 0, c->stream, d, st, e, kc, part); break;    \
+            default:                                                                                                \
+                if (k == 1) PCB_LAUNCH((KERN<3, 1>), grid, blk, 0, c->stream, d, st, e, kc, part);                  \
+                else if (k == 2) PCB_LAUNCH((KERN<3, 2>), grid, blk, 0, c->stream, d, st, e, kc, part);             \
+                else PCB_LAUNCH((KERN<3, 0>), grid, blk, 0, c->stream, d, st, e, kc, part);                         \
+        }                                                                                                           \
+    } while (0)
+    if (plane) PCB_FE_GO(k_field_energy_t);
+    else PCB_FE_GO(k_field_energy);
+#undef PCB_FE_GO
+    PCB_CUDA_OK(cudaGetLastError());
+    PCB_LAUNCH(k_sum_partials, dim3(1, 1, 1), dim3(64, 1, 1), 0, c->stream, (const double*)part, gx, 2 * kc, dout);
+    PCB_CUDA_OK(cudaGetLastError());
+    c->launches += 2;
+    return 0;
+}
+
+int pcb_field_energy(pcb_op* o, int ncols, const void* const* x, double* e_in, double* e_tot) {
+    PCB_CHECK_ARG(o && x && e_in && e_tot && ncols > 0, "bad arguments");
+    pcb_ctx* c = o->ctx;
+    PCB_CUDA_OK(cudaSetDevice(c->device));
+    if (c->nloc != c->nn) {
+        pcb_set_error("pcb_field_energy: needs whole columns; a slab context only supports PCB_APPLY_P (gather with pcb_slab_exchange)");
+        return -2;
+    }
+    PCB_CHECK_ARG(!o->diel || o->diel->zsplit == c->zsplit, "dielectric was created under the other plane-mode form (plane_split); re-create it");
+    // the layout of the A / H plane mode (apply_structure), for every dielectric kind
+    const int plane = (c->use_plane && (c->zsplit || c->plan->plane_split != 2)) ? 1 : 0;
+    const unsigned char* smask = nullptr;
+    if (plane && o->d.diel != PCB_DIEL_NONE && !(smask = energy_slot_mask(o))) return -1;
+    const int gx = grid_for(c, c->nn, 256, 4);      // fixed for the context: the same partials for a column at any width
+    const int kmax = ncols < PCB_MAXC ? ncols : PCB_MAXC;
+    if (ensure_partial(c, sizeof(double) * ((size_t)gx + 1) * 2 * PCB_MAXC)) return -1;
+    if (ensure_hstage(c, 65536)) return -1;
+    if (ensure_scratch(c, sizeof(cplx) * (size_t)c->R * (size_t)kmax)) return -1;
+    double* dout = c->partial + (size_t)gx * 2 * PCB_MAXC;
+    for (int j0 = 0; j0 < ncols; j0 += PCB_MAXC) {
+        const int kc = (ncols - j0 < PCB_MAXC) ? ncols - j0 : PCB_MAXC;
+        PcbCols cols;
+        memset(&cols, 0, sizeof cols);
+        for (int j = 0; j < kc; ++j) cols.in[j] = (const cplx*)x[j0 + j];
+        if (field_energy_chunk(o, cols, kc, plane, smask, gx, dout)) return -1;
+        PCB_CUDA_OK(cudaMemcpyAsync(c->hstage, dout, sizeof(double) * 2 * kc, cudaMemcpyDeviceToHost, c->stream));
+        PCB_CUDA_OK(cudaStreamSynchronize(c->stream));
+        const double* h = (const double*)c->hstage;
+        for (int j = 0; j < kc; ++j) { e_in[j0 + j] = h[2 * j] / (double)c->nn; e_tot[j0 + j] = h[2 * j + 1] / (double)c->nn; }
+    }
     return 0;
 }
 

@@ -4,7 +4,8 @@ uniform_initialization :33-71, pc_mfd_handle :73-85, recompute_normalize_print :
 and bandgap :313-496 keep their names, arguments, printed tables and the JSON checkpoint format
 ("<d_flag>_<n>_iterations" / "_frequencies", [0,0] = uncomputed, [-1,-1] = failed).  New here:
 ``kpath_chunks`` / ``bandgap_sharded`` distribute the k-path over the GPUs of a node, one k-chunk per
-process, with no data-path collective (SURVEY.md 8e-i).
+process, with no data-path collective (SURVEY.md 8e-i); ``energy_fraction`` / ``mode_fields`` tell where a band's
+electric energy lives (opt-in output of ``eigen_1p`` / ``bandgap`` with ``energy=True``).
 """
 import json
 import os
@@ -113,10 +114,40 @@ def recompute_normalize_print(lambdas_in, x, A_func, shift=0.0, scal=SCAL):
     return lambdas_pnt, lambdas_re
 
 
+def _operator_of(A_func, what):
+    if not isinstance(A_func, OperatorCallable):
+        raise TypeError(f"{what}: A_func must be the device operator callable returned by pc_mfd_handle, got "
+                        f"{type(A_func).__name__} (the energies are reduced on the device; there is no host path)")
+    return A_func.op
+
+
+def energy_fraction(x, A_func):
+    """Fraction f = e_in / e_tot of each column's electric energy that lies in the dielectric (Omega_1), with
+    D = FFT3(K_A^H x), E = M D, e_tot = Re D^H E / N^3 (= x^H A x) and e_in the same sum over the edge DoFs in Omega_1
+    (pcb_field_energy).  x: DeviceBlock or host array (3n^3, k); A_func: the first callable of pc_mfd_handle.
+
+    0 <= f <= 1 for the chiral M; the pseudochiral M couples rows, so f may leave [0, 1] slightly there.  f = 0 without a
+    dielectric.  For the chiral M, dlambda/deps = -lambda f / eps (Hellmann-Feynman).  Within a degenerate set of bands f of a
+    single vector depends on the basis the solver returned; the sum over the set does not."""
+    e_in, e_tot = _operator_of(A_func, "energy_fraction").field_energy(x)
+    return e_in / e_tot
+
+
+def mode_fields(x, A_func, which="D"):
+    """Real-space fields of the columns of x as a new DeviceBlock in the natural layout: which = "D" gives D = FFT3(K_A^H x),
+    "E" gives E = M D.  ``.get()[:, j].reshape(3, n, n, n)`` is column j indexed [c][i2][i1][i0]."""
+    op = _operator_of(A_func, "mode_fields")
+    if which not in ("D", "E"):
+        raise ValueError('which must be "D" or "E"')
+    return op.apply(L.APPLY_DFIELD if which == "D" else L.APPLY_EFIELD,
+                    x if isinstance(x, DeviceBlock) else DeviceBlock.from_host(op.ctx, x))
+
+
 def eigen_1p(n, d_flag, alpha, type="chiral", nev=NEV, solver=lobpcg_sep_softlock, cpu_x0=False, x0=None, seed=None,
-             tol=TOL, eps_opt=0):
+             tol=TOL, eps_opt=0, energy=False):
     """Eigenvalues at one lattice vector (numerical_experiments.py:209-247).  Prints like the reference and
-    additionally returns a dict (lambdas, x, info, omega_pnt, omega_re, residuals, shift)."""
+    additionally returns a dict (lambdas, x, info, omega_pnt, omega_re, residuals, shift); with ``energy=True`` also
+    "energy_fraction", the fraction of the electric energy in the dielectric of the first nev bands (energy_fraction)."""
     alpha = np.asarray(alpha, dtype=float)
     a_fft, b_fft, inv_fft, x_rand, shift = uniform_initialization(n, d_flag, alpha, nev=nev, seed=seed)
     if x0 is None:
@@ -137,16 +168,37 @@ def eigen_1p(n, d_flag, alpha, type="chiral", nev=NEV, solver=lobpcg_sep_softloc
     say(lambdas_pnt)
     say(f"\n{RESET}")
     w_pnt, w_re = recompute_normalize_print(lambdas_pnt[:nev], x[:, :nev], A_func, shift=shift)
-    return {"lambdas": lambdas_pnt, "x": x, "info": iters, "omega_pnt": w_pnt, "omega_re": w_re,
-            "residuals": recompute_normalize_print.last_residuals, "shift": shift}
+    out = {"lambdas": lambdas_pnt, "x": x, "info": iters, "omega_pnt": w_pnt, "omega_re": w_re,
+           "residuals": recompute_normalize_print.last_residuals, "shift": shift}
+    if energy:
+        out["energy_fraction"] = energy_fraction(x[:, :nev], A_func)
+    return out
 
 
 # ---------------------------------------------------------------------------------------------
 # Band structure along the k-path
 # ---------------------------------------------------------------------------------------------
-def _load_or_init_record(path_bandgap, var_it, var_fq, n_k, type, d_flag, n):
+def _load_or_init_record(path_bandgap, var_it, var_fq, n_k, type, d_flag, n, var_en=None, nev=NEV):
     """JSON checkpoint logic of bandgap() (numerical_experiments.py:355-408).
-    Returns (gap_lib, uncomputed indices or None, done flag)."""
+    Returns (gap_lib, uncomputed indices or None, done flag).  var_en (energy=True): the energy-fraction key; a row
+    counts as done only when its energy row is filled too (rows of a file written without energies are recomputed)."""
+    gap_lib, uncomputed, done = _load_or_init_record_its(path_bandgap, var_it, var_fq, n_k, type, d_flag, n)
+    if var_en is None:
+        return gap_lib, uncomputed, done
+    rec = gap_lib.get(var_en)
+    if rec is None or len(rec) != n_k:
+        rec = gap_lib[var_en] = [[0] * nev for _ in range(n_k)]
+    if uncomputed is None:
+        return gap_lib, None, False
+    missing = [i for i, a in enumerate(rec) if all(v == 0 for v in a) or all(v == -1 for v in a)]
+    missing = [i for i in missing if i not in set(uncomputed)]
+    if missing:
+        say(f"{YELLOW}Following indices have no energy fractions yet: {missing}.{RESET}")
+    todo = sorted(set(uncomputed) | set(missing))
+    return gap_lib, todo, not todo
+
+
+def _load_or_init_record_its(path_bandgap, var_it, var_fq, n_k, type, d_flag, n):
     fresh_it, fresh_fq = [[0] * 2 for _ in range(n_k)], [[0] * NEV for _ in range(n_k)]
     if not os.path.exists(path_bandgap):
         say("The bandgap of type ", d_flag, " has no previous record.")
@@ -178,12 +230,16 @@ def _load_or_init_record(path_bandgap, var_it, var_fq, n_k, type, d_flag, n):
 
 
 def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indices=None, nev=NEV, seed=None,
-            path=None, tol=TOL / SCAL / SCAL, only=None):
+            path=None, tol=TOL / SCAL / SCAL, only=None, energy=False):
     """Band structure along the lattice's k-path, one warm-started LOBPCG solve per point, checkpointed to
     JSON after every point (numerical_experiments.py:313-496).  Returns the list of failed indices.
-    `nev` (default NEV), `seed` (reproducible random starts) and `path` (output file) are additions."""
+    `nev` (default NEV), `seed` (reproducible random starts) and `path` (output file) are additions.
+    `energy=True` also records, per k-point, the fraction of the electric energy in the dielectric of its nev bands
+    (energy_fraction) under "<d_flag>_<n>_energy_fraction" ([0]*nev uncomputed, [-1]*nev failed)."""
     t_all = time.time()
     timing = {"setup": 0.0, "assemble": 0.0, "solver": 0.0, "postprocess": 0.0, "checkpoint": 0.0}
+    if energy:
+        timing["energy"] = 0.0
     bandgap.last_timing = timing          # wall seconds by phase (where a band-structure run spends its time)
     ct, sym_points = diel.diel_info(d_flag)
     alphas = diel.kpath(d_flag, GAP)
@@ -195,10 +251,12 @@ def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indice
 
     path_bandgap = path or (OUTPUT_PATH + type + "/bandgap_" + d_flag + ".json")
     var_it, var_fq = f"{d_flag}_{n}_iterations", f"{d_flag}_{n}_frequencies"
-    gap_lib, uncomputed, done = _load_or_init_record(path_bandgap, var_it, var_fq, n_k, type, d_flag, n)
+    var_en = f"{d_flag}_{n}_energy_fraction" if energy else None
+    gap_lib, uncomputed, done = _load_or_init_record(path_bandgap, var_it, var_fq, n_k, type, d_flag, n, var_en, nev)
     if done:
         return []
     gap_rec_it, gap_rec_fq = gap_lib[var_it], gap_lib[var_fq]
+    gap_rec_en = gap_lib[var_en] if energy else None
     if indices is None:
         indices = list(range(n_k)) if uncomputed is None else uncomputed
         if only is not None:          # resume restricted to the given rows (the file may hold other ranks' empty rows)
@@ -246,6 +304,11 @@ def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indice
             t_s = time.time()
             _, lambdas_re = recompute_normalize_print(lambdas_pnt, x, A_func, relax_opt[0])
             timing["postprocess"] += time.time() - t_s
+            if energy:
+                t_s = time.time()
+                frac = energy_fraction(x[:, :nev], A_func)
+                timing["energy"] += time.time() - t_s
+                gap_rec_en[idx] = [float(v) for v in frac]
             gap_rec_it[idx] = [float(v) for v in iters[:2]]
             gap_rec_fq[idx] = [float(v) for v in lambdas_re]
         except Exception as e:          # same policy as the reference: record [-1,-1], restart from random
@@ -255,9 +318,13 @@ def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indice
             x = None
             gap_rec_it[idx] = [-1.0, -1.0]
             gap_rec_fq[idx] = [-1.0] * nev
+            if energy:
+                gap_rec_en[idx] = [-1.0] * nev
         del x0
         t_h = time.time()
         gap_lib[var_it], gap_lib[var_fq] = gap_rec_it, gap_rec_fq
+        if energy:
+            gap_lib[var_en] = gap_rec_en
         with open(path_bandgap, "w") as f:
             json.dump(gap_lib, f, indent=4)
         timing["checkpoint"] += time.time() - t_h
@@ -283,21 +350,26 @@ def kpath_chunks(n_k, world):
 
 
 def merge_records(parts, n_k, nev=NEV):
-    """Combine per-rank {"iterations": {idx: [it, s]}, "frequencies": {idx: [...]}} rows into full-path lists."""
+    """Combine per-rank {"iterations": {idx: [it, s]}, "frequencies": {idx: [...]}} rows into full-path lists.
+    When the parts carry "energy_fraction" rows (bandgap_sharded(..., energy=True)), a third list of them is returned too."""
     its, fqs = [[0, 0] for _ in range(n_k)], [[0] * nev for _ in range(n_k)]
+    ens = [[0] * nev for _ in range(n_k)] if any("energy_fraction" in p for p in parts) else None
     for p in parts:
         for idx, row in p["iterations"].items():
             its[int(idx)] = row
         for idx, row in p["frequencies"].items():
             fqs[int(idx)] = row
-    return its, fqs
+        for idx, row in p.get("energy_fraction", {}).items():
+            ens[int(idx)] = row
+    return (its, fqs) if ens is None else (its, fqs, ens)
 
 
 def bandgap_sharded(n, d_flag, rank, world, type=TYPE0, eps_opt=0, nev=NEV, seed=1000, out_dir=None, indices=None,
-                    gather=None, tol=TOL / SCAL / SCAL, retry=1):
+                    gather=None, tol=TOL / SCAL / SCAL, retry=1, energy=False):
     """k-path sharding over `world` processes (one GPU each): rank r solves chunk r of the path (or of `indices`)
     into its own JSON file; with `gather` (callable: obj -> list of objs on rank 0, e.g. a torch.distributed
-    gather_object wrapper) rank 0 merges all rows into the reference-format file.  No collective touches the data path."""
+    gather_object wrapper) rank 0 merges all rows into the reference-format file.  No collective touches the data path.
+    energy=True: bandgap(..., energy=True) on every rank, and the energy-fraction rows are merged as well."""
     all_idx = list(range(diel.kpath(d_flag, GAP).shape[0])) if indices is None else list(indices)
     mine = [all_idx[i] for i in kpath_chunks(len(all_idx), world)[rank]]
     out_dir = out_dir or (OUTPUT_PATH + type + "/")
@@ -305,7 +377,8 @@ def bandgap_sharded(n, d_flag, rank, world, type=TYPE0, eps_opt=0, nev=NEV, seed
     part_path = os.path.join(out_dir, f"bandgap_{d_flag}.rank{rank}.json")
     if os.path.exists(part_path):
         os.remove(part_path)
-    errs = bandgap(n, d_flag, type=type, eps_opt=eps_opt, indices=mine, nev=nev, seed=seed, path=part_path, tol=tol) if mine else []
+    errs = bandgap(n, d_flag, type=type, eps_opt=eps_opt, indices=mine, nev=nev, seed=seed, path=part_path, tol=tol,
+                   energy=energy) if mine else []
     # A warm start can make [X W] numerically rank deficient (e.g. the point after Gamma, whose zero modes are pure gradients):
     # the reference records [-1,-1] and recomputes such rows from a random start when bandgap() is called again
     # (numerical_experiments.py:370-390); do that second call here.
@@ -313,26 +386,33 @@ def bandgap_sharded(n, d_flag, rank, world, type=TYPE0, eps_opt=0, nev=NEV, seed
         if not errs:
             break
         errs = bandgap(n, d_flag, type=type, eps_opt=eps_opt, indices=None, nev=nev, seed=seed + 7919 * (attempt + 1),
-                       path=part_path, tol=tol, only=errs)
+                       path=part_path, tol=tol, only=errs, energy=energy)
     rows = {"iterations": {}, "frequencies": {}, "errors": errs}
+    if energy:
+        rows["energy_fraction"] = {}
     if mine:
         with open(part_path) as f:
             lib = json.load(f)
         for idx in mine:
             rows["iterations"][idx] = lib[f"{d_flag}_{n}_iterations"][idx]
             rows["frequencies"][idx] = lib[f"{d_flag}_{n}_frequencies"][idx]
+            if energy:
+                rows["energy_fraction"][idx] = lib[f"{d_flag}_{n}_energy_fraction"][idx]
     if gather is None:
         return rows
     parts = gather(rows)
     if rank == 0:
         n_k = diel.kpath(d_flag, GAP).shape[0]
-        its, fqs = merge_records(parts, n_k, nev)
+        merged = merge_records(parts, n_k, nev)
+        its, fqs = merged[0], merged[1]
         final = os.path.join(out_dir, f"bandgap_{d_flag}.json")
         lib = {}
         if os.path.exists(final):
             with open(final) as f:
                 lib = json.load(f)
         lib[f"{d_flag}_{n}_iterations"], lib[f"{d_flag}_{n}_frequencies"] = its, fqs
+        if len(merged) == 3:
+            lib[f"{d_flag}_{n}_energy_fraction"] = merged[2]
         with open(final, "w") as f:
             json.dump(lib, f, indent=4)
     return rows

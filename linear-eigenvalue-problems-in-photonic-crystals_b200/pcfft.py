@@ -104,6 +104,17 @@ class Operator:
         return np.sqrt(out)
 
 
+    def field_energy(self, X):
+        """(e_in, e_tot) per column, NumPy arrays: e_tot = Re D^H M D / N^3 = x^H A x and e_in the same sum over the rows in
+        Omega_1 (the edge DoFs of the dielectric), with D = FFT3(K_A^H x) -- see pcb_field_energy in include/pcb200.h.
+        X: a DeviceBlock on this operator's context (column views welcome) or a host array (3n^3, k) / (3n^3,), uploaded."""
+        X, _ = devarray.as_block(self.ctx, X)
+        e_in, e_tot = np.zeros(X.k), np.zeros(X.k)
+        if X.k:
+            L.check(self._lib.pcb_field_energy(self.h, X.k, L.ptr_array(X.ptrs), e_in.ctypes.data_as(L.c_double_p),
+                                               e_tot.ctypes.data_as(L.c_double_p)), "pcb_field_energy")
+        return e_in, e_tot
+
     def update_resid(self, m, n_loc, s_loc, hs_loc, P, HP, E, lambdas, W):
         """_sep_update_after_rr (lobpcg.py:1248-1270) fused with the next iteration's residual, norms and preconditioner
         (:394-397,442): returns ||lambda_j x_j - hx_j||_2 of the UPDATED X, HX; W receives K_P^-1 of those residuals."""
