@@ -45,7 +45,8 @@ enum {
     PCB_APPLY_KAH = 7,   /* A_block_kernel(x, -conj(D_A))    pcfft.py:148                                         */
     PCB_APPLY_KB = 8,    /* H_block_kernel(x, D_B) = gamma K_B x   pcfft.py:18-30,176 / _kernels.py:13-41         */
     PCB_APPLY_DFIELD = 9, /* D = FFT3(K_A^H x): the real-space field of AMA (pcfft.py:148-149), natural layout        */
-    PCB_APPLY_EFIELD = 10 /* E = M D (the dielectric applied to that field), natural layout                          */
+    PCB_APPLY_EFIELD = 10, /* E = M D (the dielectric applied to that field), natural layout                         */
+    PCB_APPLY_EFOURIER = 11 /* E^ = IFFT3(M FFT3(K_A^H x)): AMA before its last K_A (A x = K_A E^), natural layout   */
 };
 
 const char* pcb_last_error(void);
@@ -55,6 +56,7 @@ int pcb_supported_sizes(int* sizes, int cap);  /* returns how many grid sizes N 
 
 int pcb_ctx_create(int device, int N, pcb_ctx** ctx);
 void pcb_ctx_destroy(pcb_ctx* ctx);
+long long pcb_ctx_trim(pcb_ctx* ctx);               /* frees the context's cached E^ columns of pcb_band_velocity; returns the bytes freed */
 int pcb_sync(pcb_ctx* ctx);
 int pcb_launch_count(pcb_ctx* ctx, long long* n);   /* kernels launched by this context so far */
 /* pass-structure switches (A/B measurements, tests): "plane", "plane_coupled", "plane_cross" (0 / 1 / 2), "mid_five" (-1 auto, 0, 1),
@@ -106,7 +108,8 @@ void pcb_op_destroy(pcb_op* op);
  * cross-DoF dielectric (out serves as work space of the plane halves / the stencil gathers); the call fails with -2 in those
  * cases, before anything is enqueued: no output column is written.  Distinct columns must not overlap.
  * PCB_APPLY_DFIELD / PCB_APPLY_EFIELD (forward x, y, z passes; EFIELD then M point-wise in place on out, or the cross-DoF stencil
- * from the context's scratch into out) read X only in their first pass: in place is allowed for every dielectric. */
+ * from the context's scratch into out) read X only in their first pass: in place is allowed for every dielectric.
+ * PCB_APPLY_EFOURIER runs the passes of PCB_APPLY_A (the last x pass without K_A) and follows its in-place rule. */
 int pcb_apply(pcb_op* op, int mode, int ncols, const void* const* in, void* const* out);
 
 /* Y_host = op(X_host): the reference-facing call with host arrays -- x_host, y_host are the reference's row-major (3N^3, k)
@@ -134,6 +137,19 @@ int pcb_apply_timed(pcb_op* op, int mode, int ncols, const void* const* in, void
  * column gives the same bits at any width and on every call.  Runs the forward passes of A (the plane layout where A runs in plane
  * mode, else the natural layout) into the context's scratch and a reduction kernel over them.  A slab context fails with -2. */
 int pcb_field_energy(pcb_op* op, int ncols, const void* const* x, double* e_in, double* e_tot);
+
+/* Band velocity matrices (Hellmann-Feynman).  The symbols depend on the k-point alpha only through the Bloch term of the diagonal
+ * tables, dK_c/dalpha_d = delta_cd tau_d[i_d]; dtables = tau as a HOST array [3][N] complex128 (FourierSymbols.dtables).  With
+ * E^ = PCB_APPLY_EFOURIER of x and, for d, a, b cyclic, W_d[i][j] = x_i^H ((tau_d e_d) x E^_j)
+ *     = sum_q tau_d[q_d] (conj(x_i,b) E^_j,a - conj(x_i,a) E^_j,b),
+ * the call returns V_d = W_d + W_d^H = X^H (dA/dalpha_d) X (Hermitian): V HOST, [3][ncols][ncols] complex128 row-major;
+ * xx[j] = x_j^H x_j and xax[j] = Re x_j^H A x_j = Re sum_q conj(x_j) . (K x E^_j) (HOST doubles), so that
+ * dlambda_j/dalpha_d = V_d[j][j] / xx[j] for a band that is not degenerate.  1 <= ncols <= 32 (the solver's block width); x is
+ * read only.  Runs the passes of A with a plain last x pass into a buffer of ncols columns kept by the context (released by
+ * pcb_ctx_trim), then the reduction kernel over a grid that depends on the context only and a fixed-order sum: entry (d, i, j)
+ * gets the same bits at any width (V of a subset of columns is the matching sub-block of a wider call) and on every call.
+ * ncols > 32 and slab contexts fail with -2, before anything is written to V, xx or xax. */
+int pcb_band_velocity(pcb_op* op, int ncols, const void* const* x, const double* dtables, void* V, double* xx, double* xax);
 
 /* LOBPCG block kernels
  * pcb_residual: r_j = lambda_j x_j - hx_j (lobpcg.py:394-395); norms2[j] = ||r_j||^2 (environment.norms :131-143);

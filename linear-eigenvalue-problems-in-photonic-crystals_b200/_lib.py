@@ -64,6 +64,8 @@ SIGNATURES = {
     "pcb_update_resid_wait": (C.c_int, [C.c_void_p, C.c_int, c_double_p]),
     "pcb_block_launch_info": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]),
     "pcb_field_energy": (C.c_int, [C.c_void_p, C.c_int, c_void_pp, c_double_p, c_double_p]),
+    "pcb_band_velocity": (C.c_int, [C.c_void_p, C.c_int, c_void_pp, c_double_p, C.c_void_p, c_double_p, c_double_p]),
+    "pcb_ctx_trim": (C.c_longlong, [C.c_void_p]),
     "pcb_coldots": (C.c_int, [C.c_void_p, C.c_int, c_void_pp, c_void_pp, C.c_void_p]),
     "pcb_axpby": (C.c_int, [C.c_void_p, C.c_int, c_void_pp, c_void_pp, C.c_double, C.c_double]),
     "pcb_geometry_mask": (C.c_int, [C.c_void_p, C.c_int, c_double_p, C.c_void_p, C.c_void_p]),
@@ -80,7 +82,7 @@ SIGNATURES = {
     "pcb_slab_exchange": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), c_void_pp, c_void_pp]),
 }
 
-APPLY_FFT, APPLY_IFFT, APPLY_A, APPLY_H, APPLY_P, APPLY_M, APPLY_KA, APPLY_KAH, APPLY_KB, APPLY_DFIELD, APPLY_EFIELD = range(11)
+APPLY_FFT, APPLY_IFFT, APPLY_A, APPLY_H, APPLY_P, APPLY_M, APPLY_KA, APPLY_KAH, APPLY_KB, APPLY_DFIELD, APPLY_EFIELD, APPLY_EFOURIER = range(12)
 DIEL_NONE, DIEL_CHIRAL, DIEL_TRIVIAL, DIEL_CROSSDOF = range(4)
 
 

@@ -911,6 +911,153 @@ __global__ void __launch_bounds__(256) k_field_energy_t(PcbOp op, PcbStencil st,
     pcb_energy_block_store(ein, etot, partial, ncols);
 }
 
+// ---- band velocity matrices (pcb_band_velocity) ---------------------------------------------------------------------------
+// Input: X (cols.in) and E^ = IFFT3(M FFT3(K_A^H x)) (cols.out), natural layout; tau = dK_d/dalpha_d, [3][N] complex (device).
+// For d, a, b cyclic:  W_d[i][j] = sum_q conj(x_i,b) F_j,d,a - conj(x_i,a) F_j,d,b  with  F_j,d,c = tau_d[q_d] E^_j,c
+// (tau folded into E^ while staging), plus xx[j] = sum |x_j|^2 and xax[j] = Re sum conj(x_j) . (K x E^_j) on the diagonal blocks.
+// blockIdx.y = (I, J), a pair of blocks of PCB_BV_B columns (X_I against E^_J); blockIdx.x strides over chunks of PCB_BV_P
+// points.  A chunk is staged [c or m][column][point] in shared memory (+1 point pad: the staging stores and the broadcast loads
+// of the register tiles are conflict-free); slice s of the chunk (points s P/S .. (s+1) P/S - 1) belongs to warps 2s, 2s+1, whose
+// 64 lanes hold the 256 entries of the block as 2 x 2 register tiles (rows it + 8 ki, columns jt + 8 kj) for all three d.
+// Determinism: an entry (d, i, j) is summed over the CTA's chunks in order, within a chunk over its slice's points in order,
+// then over the S slices in order, then over the CTAs in order (k_sum_partials).  None of this depends on ncols or on (I, J):
+// a column pair gets the same bits at any width.  partial[blockIdx.x * E + e], E = 6 n^2 + 2 n doubles:
+// e = 2 ((d n + i) n + j) + {re, im} for W, 6 n^2 + j for xx, 6 n^2 + n + j for xax.
+#define PCB_BV_B 16
+#define PCB_BV_P 32
+#define PCB_BV_S 4
+#define PCB_BV_NT 256
+#define PCB_BV_LD (PCB_BV_P + 1)
+#define PCB_BV_SMEM ((3 + 6) * PCB_BV_B * PCB_BV_LD * (int)sizeof(cplx))
+#ifdef PCB_EMU
+#define PCB_BV_ROLLED
+#else
+#define PCB_BV_ROLLED _Pragma("unroll 1")
+#endif
+__global__ void __launch_bounds__(PCB_BV_NT, 2) k_band_velocity(PcbOp op, PcbCols cols, const cplx* __restrict__ tau, int ncols,
+                                                                int nb, double* __restrict__ partial) {
+    static_assert(PCB_BV_B == 16 && PCB_BV_NT == 256 && PCB_BV_S * 2 * 32 == PCB_BV_NT, "tile mapping below assumes these");
+    constexpr int B = PCB_BV_B, P = PCB_BV_P, S = PCB_BV_S, LD = PCB_BV_LD, PS = P / S;
+    PCB_DYN_SMEM(cplx, sm);
+    cplx* __restrict__ Xs = sm;                     // [c][i][p]
+    cplx* __restrict__ Fs = sm + 3 * B * LD;        // [m = 2 d + {0: a, 1: b}][j][p]
+    __shared__ double red[2][PCB_BV_NT / 32][2];
+    const int N = op.N;
+    const long long nn = op.nn;
+    const int I = blockIdx.y / nb, J = blockIdx.y % nb;
+    const bool diag = (I == J);
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int s = warp >> 1, t = (warp & 1) * 32 + lane;
+    const int it = t >> 3, jt = t & 7;              // a warp reads 4 distinct rows and 8 distinct columns per load: broadcasts
+    const long long nchunks = (nn + P - 1) / P;
+    cplx acc[3][2][2];
+    PCB_UNROLL
+    for (int d = 0; d < 3; ++d)
+        PCB_UNROLL
+        for (int ki = 0; ki < 2; ++ki)
+            PCB_UNROLL
+            for (int kj = 0; kj < 2; ++kj) acc[d][ki][kj] = cmake(0.0, 0.0);
+    double axx0 = 0.0, axx1 = 0.0, axax0 = 0.0, axax1 = 0.0;      // xx, xax of the columns staged as r = 0, 1
+    for (long long ch = blockIdx.x; ch < nchunks; ch += gridDim.x) {
+        // stage: thread = (point lane, columns warp and warp + 8); zero rows past the last column / point
+        const long long q = ch * P + lane;
+        const bool qok = q < nn;
+        const int i0 = (int)(q % N), i1 = (int)((q / N) % N), i2 = (int)(q / ((long long)N * N));
+        cplx tq[3] = {cmake(0.0, 0.0), cmake(0.0, 0.0), cmake(0.0, 0.0)};
+        if (qok) { tq[0] = __ldg(tau + i0); tq[1] = __ldg(tau + N + i1); tq[2] = __ldg(tau + 2 * N + i2); }
+        Sym3 sy;
+        if (diag && qok) sy = pcb_symbol(op.T, N, i0, i1, i2);
+        PCB_BV_ROLLED
+        for (int r = 0; r < 2; ++r) {
+            const int jl = warp + 8 * r;
+            const int ci = I * B + jl, cj = J * B + jl;
+            cplx xv[3], ev[3];
+            PCB_UNROLL
+            for (int c = 0; c < 3; ++c) {
+                xv[c] = (qok && ci < ncols) ? cols.in[ci][c * nn + q] : cmake(0.0, 0.0);
+                ev[c] = (qok && cj < ncols) ? cols.out[cj][c * nn + q] : cmake(0.0, 0.0);
+                Xs[(c * B + jl) * LD + lane] = xv[c];
+            }
+            PCB_UNROLL
+            for (int d = 0; d < 3; ++d) {
+                const int a = (d + 1) % 3, b = (d + 2) % 3;
+                Fs[((2 * d) * B + jl) * LD + lane] = cmul(tq[d], ev[a]);
+                Fs[((2 * d + 1) * B + jl) * LD + lane] = cmul(tq[d], ev[b]);
+            }
+            if (diag && qok) {      // (I == J: xv and ev belong to the same column)
+                cplx z[3];
+                pcb_cross(sy.k, ev, z);
+                double sxx = 0.0, sxax = 0.0;
+                PCB_UNROLL
+                for (int c = 0; c < 3; ++c) {
+                    sxx += cabs2(xv[c]);
+                    sxax += fma(xv[c].x, z[c].x, xv[c].y * z[c].y);
+                }
+                if (r == 0) { axx0 += sxx; axax0 += sxax; } else { axx1 += sxx; axax1 += sxax; }
+            }
+        }
+        __syncthreads();
+        // accumulate: this slice's points in order, 2 x 2 tile x 3 directions = 24 complex FMAs per point and lane
+        PCB_BV_ROLLED
+        for (int u = 0; u < PS; ++u) {
+            const int p = s * PS + u;
+            cplx xv[3][2];
+            PCB_UNROLL
+            for (int c = 0; c < 3; ++c)
+                PCB_UNROLL
+                for (int ki = 0; ki < 2; ++ki) xv[c][ki] = Xs[(c * B + it + 8 * ki) * LD + p];
+            PCB_UNROLL
+            for (int d = 0; d < 3; ++d) {
+                const int a = (d + 1) % 3, b = (d + 2) % 3;
+                cplx fa[2], fb[2];
+                PCB_UNROLL
+                for (int kj = 0; kj < 2; ++kj) {
+                    fa[kj] = Fs[((2 * d) * B + jt + 8 * kj) * LD + p];
+                    fb[kj] = Fs[((2 * d + 1) * B + jt + 8 * kj) * LD + p];
+                }
+                PCB_UNROLL
+                for (int ki = 0; ki < 2; ++ki)
+                    PCB_UNROLL
+                    for (int kj = 0; kj < 2; ++kj)
+                        acc[d][ki][kj] = cfmac(cneg(xv[a][ki]), fb[kj], cfmac(xv[b][ki], fa[kj], acc[d][ki][kj]));
+            }
+        }
+        __syncthreads();
+    }
+    // slices -> CTA (fixed order) through shared memory: red_w[s][d][i][j]
+    cplx* __restrict__ rw = sm;
+    PCB_UNROLL
+    for (int d = 0; d < 3; ++d)
+        PCB_UNROLL
+        for (int ki = 0; ki < 2; ++ki)
+            PCB_UNROLL
+            for (int kj = 0; kj < 2; ++kj) rw[((s * 3 + d) * B + it + 8 * ki) * B + jt + 8 * kj] = acc[d][ki][kj];
+    PCB_UNROLL
+    for (int r = 0; r < 2; ++r) {
+        const double vx = pcb_warp_sum(r ? axx1 : axx0), va = pcb_warp_sum(r ? axax1 : axax0);
+        if (lane == 0) { red[r][warp][0] = vx; red[r][warp][1] = va; }
+    }
+    __syncthreads();
+    const long long E = 6LL * ncols * ncols + 2LL * ncols;
+    double* __restrict__ out = partial + (long long)blockIdx.x * E;
+    for (int e = tid; e < 3 * B * B; e += PCB_BV_NT) {
+        const int d = e / (B * B), i = (e / B) % B, j = e % B;
+        const int gi = I * B + i, gj = J * B + j;
+        if (gi >= ncols || gj >= ncols) continue;
+        cplx v = rw[(d * B + i) * B + j];
+        PCB_UNROLL
+        for (int sl = 1; sl < S; ++sl) v = cadd(v, rw[((sl * 3 + d) * B + i) * B + j]);
+        const long long o = 2LL * (((long long)d * ncols + gi) * ncols + gj);
+        out[o] = v.x;
+        out[o + 1] = v.y;
+    }
+    if (diag && tid < 2 * B) {
+        const int jl = tid % B, which = tid / B;       // column jl was staged by warp jl % 8, r = jl / 8
+        const int gj = I * B + jl;
+        if (gj < ncols) out[6LL * ncols * ncols + (long long)which * ncols + gj] = red[jl / 8][jl % 8][which];
+    }
+}
+
 // Set-up for the fused stencil-on-load: bit 4 + c of the slot-ordered mask byte = "component c at this point has a non-zero
 // cross-DoF coupling term" (its own DoF or any tap of a pair with eps_ab != 0 lies in Omega_1) -- elsewhere M is the identity
 // for that component and the plane pass touches nothing.  src: k_mask_plane's bytes (bits 0-3), dst: the same plus bits 4-6.

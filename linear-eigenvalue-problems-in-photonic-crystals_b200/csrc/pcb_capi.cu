@@ -85,6 +85,8 @@ struct pcb_ctx {
     size_t dsmall_bytes = 0;
     cplx* scratch = nullptr;        // work columns (cross-DoF dielectric, block transposes)
     size_t scratch_bytes = 0;
+    cplx* bv_buf = nullptr;         // pcb_band_velocity: the tau tables + E^ of its columns; released by pcb_ctx_trim
+    size_t bv_bytes = 0;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     cudaEvent_t order_ev[PCB_ORDER_EVENTS] = {};   // pcb_ctx_record / pcb_ctx_wait: stream ordering between contexts, created on first use
     long long launches = 0;
@@ -286,6 +288,7 @@ void pcb_ctx_destroy(pcb_ctx* c) {
     if (c->partial) cudaFree(c->partial);
     if (c->dsmall) cudaFree(c->dsmall);
     if (c->scratch) cudaFree(c->scratch);
+    if (c->bv_buf) cudaFree(c->bv_buf);
     if (c->hstage) cudaFreeHost(c->hstage);
     if (c->hp_buf) cudaFree(c->hp_buf);
     if (c->s_h2d) cudaStreamDestroy(c->s_h2d);
@@ -296,6 +299,15 @@ void pcb_ctx_destroy(pcb_ctx* c) {
     if (c->ev1) cudaEventDestroy(c->ev1);
     if (c->stream) cudaStreamDestroy(c->stream);
     delete c;
+}
+long long pcb_ctx_trim(pcb_ctx* c) {
+    if (!c || !c->bv_buf) return 0;
+    cudaSetDevice(c->device);
+    cudaStreamSynchronize(c->stream);
+    cudaFree(c->bv_buf);
+    const long long freed = (long long)c->bv_bytes;
+    c->bv_buf = nullptr; c->bv_bytes = 0;
+    return freed;
 }
 int pcb_sync(pcb_ctx* c) { PCB_CUDA_OK(cudaStreamSynchronize(c->stream)); PCB_CUDA_OK(cudaGetLastError()); return 0; }
 int pcb_launch_count(pcb_ctx* c, long long* n) { *n = c->launches; return 0; }
@@ -660,6 +672,7 @@ static int check_inplace(const pcb_op* o, int mode, int ncols, const void* const
     bool refused = false;
     if (mode == PCB_APPLY_M) refused = (o->d.diel == PCB_DIEL_CROSSDOF);
     else if (mode == PCB_APPLY_A || mode == PCB_APPLY_H) refused = refuses_inplace_AH(mode, apply_structure(o));
+    else if (mode == PCB_APPLY_EFOURIER) refused = refuses_inplace_AH(PCB_APPLY_A, apply_structure(o));      // A's passes, A's rule
     if (!refused) return 0;
     for (int j = 0; j < ncols; ++j)
         if (in[j] == out[j]) {
@@ -672,13 +685,18 @@ static int check_inplace(const pcb_op* o, int mode, int ncols, const void* const
 // A / H on kc columns (cols.in -> cols.out).  dist: the x passes read / write the slabs of all ranks through o->d.dist
 // (large-grid mode over peer memory); cols.in then holds the local X copies and cols.out local work columns.
 // (dist bit 0: the input columns are distributed, bit 1: the output columns are.)
+// mode PCB_APPLY_EFOURIER runs the passes of A with a plain inverse x pass last (no K_A): out = IFFT3(M FFT3(K_A^H x)).
+static int last_pass(int mode, bool dout, bool trn) {
+    if (mode == PCB_APPLY_EFOURIER) return trn ? PCB_PASS_XINV_T : PCB_PASS_XINV;
+    if (mode == PCB_APPLY_A) return trn ? (dout ? PCB_PASS_XINV_A_TD : PCB_PASS_XINV_A_T) : (dout ? PCB_PASS_XINV_A_D : PCB_PASS_XINV_A);
+    return trn ? (dout ? PCB_PASS_XINV_H_TD : PCB_PASS_XINV_H_T) : (dout ? PCB_PASS_XINV_H_D : PCB_PASS_XINV_H);
+}
 static int apply_AH(pcb_op* o, int mode, PcbCols& cols, int kc, int j0, int dist) {
     pcb_ctx* c = o->ctx;
     const PcbOpLaunch* pl = c->plan;
     const bool din = dist & 1, dout = dist & 2;
     const int first = din ? PCB_PASS_XFWD_SYM_D : PCB_PASS_XFWD_SYM, first_t = din ? PCB_PASS_XFWD_SYM_TD : PCB_PASS_XFWD_SYM_T;
-    const int last = (mode == PCB_APPLY_A) ? (dout ? PCB_PASS_XINV_A_D : PCB_PASS_XINV_A) : (dout ? PCB_PASS_XINV_H_D : PCB_PASS_XINV_H);
-    const int last_t = (mode == PCB_APPLY_A) ? (dout ? PCB_PASS_XINV_A_TD : PCB_PASS_XINV_A_T) : (dout ? PCB_PASS_XINV_H_TD : PCB_PASS_XINV_H_T);
+    const int last = last_pass(mode, dout, false), last_t = last_pass(mode, dout, true);
     int st = apply_structure(o);
     if (dist && c->zsplit) st = (o->d.diel == PCB_DIEL_CROSSDOF) ? PCB_STRUCT_CROSS7 : PCB_STRUCT_FIVE;      // no peer-memory x passes on split tiles
     if (refuses_inplace_AH(mode, st) || dist)      // (pcb_apply has checked all its columns already; pcb_apply_dist has not)
@@ -782,7 +800,7 @@ int pcb_apply(pcb_op* o, int mode, int ncols, const void* const* in, void* const
                 if (pl->apply(o->d, cols, kc, mode == PCB_APPLY_FFT ? 0 : 1, c->tw, c->stream, c->sms)) return -1;
                 c->launches += 3;
                 break;
-            case PCB_APPLY_A: case PCB_APPLY_H:
+            case PCB_APPLY_A: case PCB_APPLY_H: case PCB_APPLY_EFOURIER:
                 if (int rc = apply_AH(o, mode, cols, kc, j0, 0)) return rc;
                 break;
             case PCB_APPLY_P: {
@@ -972,6 +990,66 @@ int pcb_field_energy(pcb_op* o, int ncols, const void* const* x, double* e_in, d
         const double* h = (const double*)c->hstage;
         for (int j = 0; j < kc; ++j) { e_in[j0 + j] = h[2 * j] / (double)c->nn; e_tot[j0 + j] = h[2 * j + 1] / (double)c->nn; }
     }
+    return 0;
+}
+
+// ---- band velocity matrices (Hellmann-Feynman) ---------------------------------------------------------------------
+// E^ = PCB_APPLY_EFOURIER of the ncols columns into the context's bv_buf (behind the tau tables), k_band_velocity over a grid
+// fixed by the context, the fixed-order sum of its partials; V_d = W_d + W_d^H is formed on the host.
+int pcb_band_velocity(pcb_op* o, int ncols, const void* const* x, const double* dtables, void* V, double* xx, double* xax) {
+    PCB_CHECK_ARG(o && x && dtables && V && xx && xax && ncols > 0, "bad arguments");
+    PCB_CHECK_ARG(ncols <= PCB_MAXC, "ncols > 32: call per block of at most 32 columns");
+    pcb_ctx* c = o->ctx;
+    PCB_CUDA_OK(cudaSetDevice(c->device));
+    if (c->nloc != c->nn) {
+        pcb_set_error("pcb_band_velocity: needs whole columns; a slab context only supports PCB_APPLY_P (gather with pcb_slab_exchange)");
+        return -2;
+    }
+    PCB_CHECK_ARG(!o->diel || o->diel->zsplit == c->zsplit, "dielectric was created under the other plane-mode form (plane_split); re-create it");
+    const int N = c->N;
+    const size_t need = sizeof(cplx) * (3 * (size_t)N + (size_t)c->R * (size_t)ncols);      // grows with the widest call so far
+    if (c->bv_bytes < need) {
+        if (c->bv_buf) { PCB_CUDA_OK(cudaStreamSynchronize(c->stream)); PCB_CUDA_OK(cudaFree(c->bv_buf)); c->bv_buf = nullptr; c->bv_bytes = 0; }
+        PCB_CUDA_OK(cudaMalloc(&c->bv_buf, need));
+        c->bv_bytes = need;
+    }
+    cplx* tau = c->bv_buf;
+    cplx* ehat = c->bv_buf + 3 * (size_t)N;
+    const long long nchunks = (c->nn + PCB_BV_P - 1) / PCB_BV_P;
+    const int gx = (int)(nchunks < 2LL * c->sms ? nchunks : 2LL * c->sms);      // fixed for the context: the same partials at any width
+    const int nb = (ncols + PCB_BV_B - 1) / PCB_BV_B;
+    const long long E = 6LL * ncols * ncols + 2LL * ncols;
+    if (ensure_partial(c, sizeof(double) * ((size_t)gx + 1) * (size_t)E)) return -1;
+    double* dout = c->partial + (size_t)gx * (size_t)E;
+    PCB_CUDA_OK(cudaMemcpyAsync(tau, dtables, sizeof(cplx) * 3 * (size_t)N, cudaMemcpyHostToDevice, c->stream));
+    PcbCols cols;
+    memset(&cols, 0, sizeof cols);
+    for (int j = 0; j < ncols; ++j) { cols.in[j] = (const cplx*)x[j]; cols.out[j] = ehat + (size_t)j * c->R; }
+    if (int rc = apply_AH(o, PCB_APPLY_EFOURIER, cols, ncols, 0, 0)) return rc;
+    PcbCols bv;
+    memset(&bv, 0, sizeof bv);
+    for (int j = 0; j < ncols; ++j) { bv.in[j] = cols.in[j]; bv.out[j] = cols.out[j]; }
+    if (PCB_BV_SMEM > 48 * 1024) PCB_CUDA_OK(cudaFuncSetAttribute(k_band_velocity, cudaFuncAttributeMaxDynamicSharedMemorySize, PCB_BV_SMEM));
+    PCB_LAUNCH(k_band_velocity, dim3((unsigned)gx, (unsigned)(nb * nb), 1), dim3(PCB_BV_NT, 1, 1), (size_t)PCB_BV_SMEM, c->stream,
+               o->d, bv, (const cplx*)tau, ncols, nb, c->partial);
+    PCB_CUDA_OK(cudaGetLastError());
+    PCB_LAUNCH(k_sum_partials, dim3((unsigned)((E + 63) / 64), 1, 1), dim3(64, 1, 1), 0, c->stream, (const double*)c->partial, gx, (int)E, dout);
+    PCB_CUDA_OK(cudaGetLastError());
+    c->launches += 2;
+    std::vector<double> h((size_t)E);
+    PCB_CUDA_OK(cudaMemcpyAsync(h.data(), dout, sizeof(double) * (size_t)E, cudaMemcpyDeviceToHost, c->stream));
+    PCB_CUDA_OK(cudaStreamSynchronize(c->stream));
+    double* v = (double*)V;
+    const size_t n = (size_t)ncols;
+    for (size_t d = 0; d < 3; ++d)
+        for (size_t i = 0; i < n; ++i)
+            for (size_t j = 0; j < n; ++j) {
+                const double* wij = &h[2 * ((d * n + i) * n + j)];
+                const double* wji = &h[2 * ((d * n + j) * n + i)];
+                v[2 * ((d * n + i) * n + j)] = wij[0] + wji[0];          // V = W + W^H
+                v[2 * ((d * n + i) * n + j) + 1] = wij[1] - wji[1];
+            }
+    for (size_t j = 0; j < n; ++j) { xx[j] = h[6 * n * n + j]; xax[j] = h[6 * n * n + n + j]; }
     return 0;
 }
 

@@ -1747,6 +1747,7 @@ enum { PCB_PASS_XFWD_SYM = 0, PCB_PASS_XFWD = 1, PCB_PASS_YFWD = 2, PCB_PASS_ZFW
        PCB_PASS_XFWD_SYM_TD = 23, PCB_PASS_XINV_A_TD = 24, PCB_PASS_XINV_H_TD = 25,
        // cross-DoF dielectric with the stencil fused into the inverse half of the plane pass (four kernels)
        PCB_PASS_MID_FWD_O = 26 /* forward half, planes -> cols.out */, PCB_PASS_MID_INV_ST = 27 /* stencil on load + inverse half, cols.out -> cols.wrk */,
-       PCB_PASS_MASKACTIVE = 28 /* set-up: bits 4-6 of op.maskp */, PCB_PASS_MASKPLANE2 = 29 /* set-up: op.mask -> (unsigned char*)op.maskp2 */ };
+       PCB_PASS_MASKACTIVE = 28 /* set-up: bits 4-6 of op.maskp */, PCB_PASS_MASKPLANE2 = 29 /* set-up: op.mask -> (unsigned char*)op.maskp2 */,
+       PCB_PASS_XINV_T = 30 /* plane mode: plain inverse x pass (1/N^3, no symbol) from the transposed work column */ };
 
 const PcbOpLaunch* pcb_find_plan(int N);

@@ -303,6 +303,7 @@ struct PlanePass<true, PP, ZS> {
             if (pass_id == PCB_PASS_XFWD_SYM_T) PCB_GO((k_xfwd<PP, LX, NT, 1, 1, 0, ZS>), GX, kStageXT);
             else if (pass_id == PCB_PASS_XINV_A_T) PCB_GO((k_xinv<PP, LX, NT, 1, 1, 0, ZS>), GX, kStageXT);
             else if (pass_id == PCB_PASS_XINV_H_T) PCB_GO((k_xinv<PP, LX, NT, 2, 1, 0, ZS>), GX, kStageXT);
+            else if (pass_id == PCB_PASS_XINV_T) PCB_GO((k_xinv<PP, LX, NT, 0, 1, 0, ZS>), GX, kStageXT);
             else if (pass_id == PCB_PASS_MID && (op.diel == PCB_DIEL_NONE || op.diel == PCB_DIEL_CHIRAL)) {
 #ifndef PCB_EMU
                 if (kTma) {
@@ -325,6 +326,7 @@ struct PlanePass<true, PP, ZS> {
         }
         else if (pass_id == PCB_PASS_XINV_A_T) PCB_GO((k_xinv<PP, LX, NT, 1, 1>), GX, kStageXT);
         else if (pass_id == PCB_PASS_XINV_H_T) PCB_GO((k_xinv<PP, LX, NT, 2, 1>), GX, kStageXT);
+        else if (pass_id == PCB_PASS_XINV_T) PCB_GO((k_xinv<PP, LX, NT, 0, 1>), GX, kStageXT);
         else if (pass_id == PCB_PASS_MASKBITS2 || pass_id == PCB_PASS_MASKPLANE2) return PlaneFive<(kPlaneFive && ZS == 1), PP>::go(op, cols, ncols, pass_id, tw, s, sms);
         else if (op.diel == PCB_DIEL_NONE || op.diel == PCB_DIEL_CHIRAL) {
             if (kPlaneFive && ZS == 1 && op.mid_five && (op.diel == PCB_DIEL_NONE || op.mbits2 != nullptr)) return PlaneFive<(kPlaneFive && ZS == 1), PP>::go(op, cols, ncols, pass_id, tw, s, sms);
@@ -366,6 +368,7 @@ int run_pass(const PcbOp& op, const PcbCols& cols, int ncols, int pass_id, const
         case PCB_PASS_XFWD_SYM_T: case PCB_PASS_MID: case PCB_PASS_XINV_A_T: case PCB_PASS_XINV_H_T: case PCB_PASS_MASKBITS:
         case PCB_PASS_MID_FWD: case PCB_PASS_MID_INV: case PCB_PASS_MASKPLANE: case PCB_PASS_COORDTAB: case PCB_PASS_MASKBITS2:
         case PCB_PASS_XFWD_SYM_TD: case PCB_PASS_XINV_A_TD: case PCB_PASS_XINV_H_TD: case PCB_PASS_MID_FWD_O: case PCB_PASS_MID_INV_ST: case PCB_PASS_MASKPLANE2:
+        case PCB_PASS_XINV_T:
             if (op.zsplit) return PlanePass<kPlaneSplit, P, 2>::go(op, cols, ncols, pass_id, tw, s, sms);
             return PlanePass<kPlane, P, 1>::go(op, cols, ncols, pass_id, tw, s, sms);
         default: pcb_set_error("unknown pass id %d", pass_id); return -1;

@@ -116,9 +116,10 @@ class Context:
         L.check(self._lib.pcb_free(self.h, ptr), "pcb_free")
 
     def trim(self):
-        """cudaFree every cached block; returns the number of bytes released."""
+        """cudaFree every cached block and the context's cached band-velocity columns (pcb_ctx_trim); returns the number of
+        bytes released."""
         cache = self.__dict__.get("_alloc_cache", {})
-        freed = 0
+        freed = int(self._lib.pcb_ctx_trim(self.h))
         for nbytes, lst in cache.items():
             while lst:
                 self._lib.pcb_free(self.h, lst.pop())

@@ -156,6 +156,12 @@ class FourierSymbols:
                 t[c, c] = t[c, c] + 1j * (self.alpha[c] / self.scal) * self.D0
         return t * self.factor
 
+    @property
+    def dtables(self):
+        """(3, N) derivatives of the tables by the k-point: dK_c/dalpha_d = delta_cd dtables[d][i_d].  alpha enters only the
+        Bloch term of the diagonal tables, so dtables[d] = 1j factor / scal D0 for every d and does not depend on alpha."""
+        return np.tile(1j * (self.factor / self.scal) * np.asarray(self.D0, dtype=np.complex128), (3, 1))
+
     def toarray(self):
         """The reference's dense a_fft (3 N^3,) -- tests / interoperability only."""
         t, N = self.tables, self.N

@@ -5,7 +5,8 @@ and bandgap :313-496 keep their names, arguments, printed tables and the JSON ch
 ("<d_flag>_<n>_iterations" / "_frequencies", [0,0] = uncomputed, [-1,-1] = failed).  New here:
 ``kpath_chunks`` / ``bandgap_sharded`` distribute the k-path over the GPUs of a node, one k-chunk per
 process, with no data-path collective (SURVEY.md 8e-i); ``energy_fraction`` / ``mode_fields`` tell where a band's
-electric energy lives (opt-in output of ``eigen_1p`` / ``bandgap`` with ``energy=True``).
+electric energy lives (opt-in output of ``eigen_1p`` / ``bandgap`` with ``energy=True``); ``group_velocity`` gives the bands'
+group velocities by Hellmann-Feynman (opt-in output with ``velocity=True``).
 """
 import json
 import os
@@ -143,11 +144,95 @@ def mode_fields(x, A_func, which="D"):
                     x if isinstance(x, DeviceBlock) else DeviceBlock.from_host(op.ctx, x))
 
 
+ZERO_MODE_FREQ = 1e-4      # bands below this printed frequency (omega scal / 2 pi: the zero modes at Gamma) get no velocity
+
+
+def _velocity_clusters(lam, degen_tol):
+    """Cluster label per band: bands whose lambda agree to a relative degen_tol, grouped transitively in ascending order."""
+    order = np.argsort(lam, kind="stable")
+    labels = np.empty(len(lam), dtype=int)
+    cur = 0
+    for r, j in enumerate(order):
+        if r > 0:
+            prev = lam[order[r - 1]]
+            if abs(lam[j] - prev) > degen_tol * max(abs(lam[j]), abs(prev)):
+                cur += 1
+        labels[j] = cur
+    return labels
+
+
+def _group_velocity(x, A_func, direction, side, degen_tol):
+    """(velocities, cluster labels) of group_velocity."""
+    from .orthogonalization import gram_pair
+    import scipy.linalg as sla
+    op = _operator_of(A_func, "group_velocity")
+    X, _ = devarray.as_block(op.ctx, x)
+    k = X.k
+    if k > 32:
+        raise ValueError("group_velocity: at most 32 columns per call (the solver's block width)")
+    if side not in (1, -1):
+        raise ValueError("side must be +1 or -1")
+    V, xx, xax = op.band_velocity(X)
+    lam = xax / xx
+    labels = _velocity_clusters(lam, degen_tol)
+    u = None
+    if direction is not None:
+        u = np.asarray(direction, dtype=float).reshape(3)
+        u = u / np.linalg.norm(u)
+    dlam = np.zeros((k, 3)) if u is None else np.zeros(k)
+    for lab in np.unique(labels):
+        S = [int(j) for j in np.flatnonzero(labels == lab)]      # in column order: the solver returns the bands ascending
+        if len(S) == 1:
+            j = S[0]
+            g = V[:, j, j].real / xx[j]
+            dlam[j] = g if u is None else u @ g
+            continue
+        Xs = X.cols(S)
+        G = gram_pair(Xs, Xs)[0]
+        VS = V[:, S][:, :, S]
+        if u is None:              # basis-independent: the trace average of G^-1 V_d over the cluster
+            g = np.array([np.trace(np.linalg.solve(G, VS[d])).real / len(S) for d in range(3)])
+            for j in S:
+                dlam[j] = g
+        else:                      # degenerate first-order perturbation theory along u
+            Vu = np.einsum("d,dij->ij", u, VS)
+            Vu = 0.5 * (Vu + Vu.conj().T)
+            mu = sla.eigh(Vu, G, eigvals_only=True)
+            mu = mu if side > 0 else mu[::-1]
+            for j, m in zip(S, mu):
+                dlam[j] = m
+    scal = op.a_fft.scal
+    omega = np.sqrt(np.maximum(lam, 0.0))
+    zero = omega * scal / (2 * pi) < ZERO_MODE_FREQ
+    with np.errstate(divide="ignore", invalid="ignore"):
+        vel = dlam / (2 * omega[:, None]) if u is None else dlam / (2 * omega)
+    vel[zero] = np.nan
+    return vel, labels
+
+
+def group_velocity(x, A_func, direction=None, side=+1, degen_tol=1e-6):
+    """Group velocities d omega / d alpha of the columns of x (eigenvectors of A_func at k-point alpha, omega = sqrt(lambda)),
+    by Hellmann-Feynman from the velocity matrices V_d = X^H (dA/dalpha_d) X of pcb_band_velocity.  x: DeviceBlock or host
+    array (3n^3, k), k <= 32; A_func: the first callable of pc_mfd_handle.  With SCAL = 1 and alpha in units of 1/a the
+    velocity is in units of c.
+
+    direction None: (k, 3) gradients.  Else (k,) derivatives along the normalised direction u.  Bands whose lambda agree to a
+    relative degen_tol (grouped transitively) form a cluster S: along u its velocities are the eigenvalues mu of
+    (sum_d u_d V_d)|_S c = mu G_S c, G_S = X_S^H X_S, assigned to the cluster's columns (the columns of x are taken to be
+    the bands in ascending order, as the solver returns them) in ascending order for the step
+    k -> k + h u (side=+1) and in descending order for the derivative from the -u side (side=-1: the bands are sorted at
+    k - h u, where omega ~ omega_0 - h mu).  Without a direction a cluster reports the basis-independent trace average
+    (1/|S|) tr(G_S^-1 V_d|_S).  Bands with omega scal / 2 pi < 1e-4 (the zero modes at Gamma) get NaN."""
+    return _group_velocity(x, A_func, direction, side, degen_tol)[0]
+
+
 def eigen_1p(n, d_flag, alpha, type="chiral", nev=NEV, solver=lobpcg_sep_softlock, cpu_x0=False, x0=None, seed=None,
-             tol=TOL, eps_opt=0, energy=False):
+             tol=TOL, eps_opt=0, energy=False, velocity=False):
     """Eigenvalues at one lattice vector (numerical_experiments.py:209-247).  Prints like the reference and
     additionally returns a dict (lambdas, x, info, omega_pnt, omega_re, residuals, shift); with ``energy=True`` also
-    "energy_fraction", the fraction of the electric energy in the dielectric of the first nev bands (energy_fraction)."""
+    "energy_fraction", the fraction of the electric energy in the dielectric of the first nev bands (energy_fraction); with
+    ``velocity=True`` also "group_velocity" (nev, 3), the gradients of group_velocity, and "velocity_cluster", its cluster
+    label per band (bands with the same label are degenerate and report the cluster's trace average)."""
     alpha = np.asarray(alpha, dtype=float)
     a_fft, b_fft, inv_fft, x_rand, shift = uniform_initialization(n, d_flag, alpha, nev=nev, seed=seed)
     if x0 is None:
@@ -172,29 +257,38 @@ def eigen_1p(n, d_flag, alpha, type="chiral", nev=NEV, solver=lobpcg_sep_softloc
            "residuals": recompute_normalize_print.last_residuals, "shift": shift}
     if energy:
         out["energy_fraction"] = energy_fraction(x[:, :nev], A_func)
+    if velocity:
+        out["group_velocity"], out["velocity_cluster"] = _group_velocity(x[:, :nev], A_func, None, +1, 1e-6)
     return out
 
 
 # ---------------------------------------------------------------------------------------------
 # Band structure along the k-path
 # ---------------------------------------------------------------------------------------------
-def _load_or_init_record(path_bandgap, var_it, var_fq, n_k, type, d_flag, n, var_en=None, nev=NEV):
+def _load_or_init_record(path_bandgap, var_it, var_fq, n_k, type, d_flag, n, var_en=None, nev=NEV, var_vel=None):
     """JSON checkpoint logic of bandgap() (numerical_experiments.py:355-408).
-    Returns (gap_lib, uncomputed indices or None, done flag).  var_en (energy=True): the energy-fraction key; a row
-    counts as done only when its energy row is filled too (rows of a file written without energies are recomputed)."""
+    Returns (gap_lib, uncomputed indices or None, done flag).  var_en (energy=True) / var_vel (velocity=True): the
+    energy-fraction / group-velocity keys; a row counts as done only when those rows are filled too (rows of a file written
+    without them are recomputed)."""
     gap_lib, uncomputed, done = _load_or_init_record_its(path_bandgap, var_it, var_fq, n_k, type, d_flag, n)
-    if var_en is None:
+    extra = [(v, what) for v, what in ((var_en, "energy fractions"), (var_vel, "group velocities")) if v is not None]
+    if not extra:
         return gap_lib, uncomputed, done
-    rec = gap_lib.get(var_en)
-    if rec is None or len(rec) != n_k:
-        rec = gap_lib[var_en] = [[0] * nev for _ in range(n_k)]
+    missing = set()
+    for var, what in extra:
+        rec = gap_lib.get(var)
+        if rec is None or len(rec) != n_k:
+            rec = gap_lib[var] = [[0] * nev for _ in range(n_k)]
+        if uncomputed is None:
+            continue
+        miss = [i for i, a in enumerate(rec) if all(v == 0 for v in a) or all(v == -1 for v in a)]
+        miss = [i for i in miss if i not in set(uncomputed)]
+        if miss:
+            say(f"{YELLOW}Following indices have no {what} yet: {miss}.{RESET}")
+        missing |= set(miss)
     if uncomputed is None:
         return gap_lib, None, False
-    missing = [i for i, a in enumerate(rec) if all(v == 0 for v in a) or all(v == -1 for v in a)]
-    missing = [i for i in missing if i not in set(uncomputed)]
-    if missing:
-        say(f"{YELLOW}Following indices have no energy fractions yet: {missing}.{RESET}")
-    todo = sorted(set(uncomputed) | set(missing))
+    todo = sorted(set(uncomputed) | missing)
     return gap_lib, todo, not todo
 
 
@@ -230,16 +324,22 @@ def _load_or_init_record_its(path_bandgap, var_it, var_fq, n_k, type, d_flag, n)
 
 
 def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indices=None, nev=NEV, seed=None,
-            path=None, tol=TOL / SCAL / SCAL, only=None, energy=False):
+            path=None, tol=TOL / SCAL / SCAL, only=None, energy=False, velocity=False):
     """Band structure along the lattice's k-path, one warm-started LOBPCG solve per point, checkpointed to
     JSON after every point (numerical_experiments.py:313-496).  Returns the list of failed indices.
     `nev` (default NEV), `seed` (reproducible random starts) and `path` (output file) are additions.
     `energy=True` also records, per k-point, the fraction of the electric energy in the dielectric of its nev bands
-    (energy_fraction) under "<d_flag>_<n>_energy_fraction" ([0]*nev uncomputed, [-1]*nev failed)."""
+    (energy_fraction) under "<d_flag>_<n>_energy_fraction" ([0]*nev uncomputed, [-1]*nev failed).
+    `velocity=True` records under "<d_flag>_<n>_group_velocity", per k-point, d omega / ds of its nev bands along the path
+    (group_velocity): point idx lies on segment s = idx // GAP with direction u_s = sym[s+1] - sym[s], and the derivative is
+    taken from that segment's start side (side=-1), so segment end points and crossings get the value the path arrives with.
+    Zero modes are written as null; the row sentinels are those of the energy fractions."""
     t_all = time.time()
     timing = {"setup": 0.0, "assemble": 0.0, "solver": 0.0, "postprocess": 0.0, "checkpoint": 0.0}
     if energy:
         timing["energy"] = 0.0
+    if velocity:
+        timing["velocity"] = 0.0
     bandgap.last_timing = timing          # wall seconds by phase (where a band-structure run spends its time)
     ct, sym_points = diel.diel_info(d_flag)
     alphas = diel.kpath(d_flag, GAP)
@@ -252,11 +352,14 @@ def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indice
     path_bandgap = path or (OUTPUT_PATH + type + "/bandgap_" + d_flag + ".json")
     var_it, var_fq = f"{d_flag}_{n}_iterations", f"{d_flag}_{n}_frequencies"
     var_en = f"{d_flag}_{n}_energy_fraction" if energy else None
-    gap_lib, uncomputed, done = _load_or_init_record(path_bandgap, var_it, var_fq, n_k, type, d_flag, n, var_en, nev)
+    var_vel = f"{d_flag}_{n}_group_velocity" if velocity else None
+    gap_lib, uncomputed, done = _load_or_init_record(path_bandgap, var_it, var_fq, n_k, type, d_flag, n, var_en, nev, var_vel)
     if done:
         return []
     gap_rec_it, gap_rec_fq = gap_lib[var_it], gap_lib[var_fq]
     gap_rec_en = gap_lib[var_en] if energy else None
+    gap_rec_vel = gap_lib[var_vel] if velocity else None
+    sym = diel.diel_info(d_flag, "sym").astype(float)
     if indices is None:
         indices = list(range(n_k)) if uncomputed is None else uncomputed
         if only is not None:          # resume restricted to the given rows (the file may hold other ranks' empty rows)
@@ -309,6 +412,12 @@ def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indice
                 frac = energy_fraction(x[:, :nev], A_func)
                 timing["energy"] += time.time() - t_s
                 gap_rec_en[idx] = [float(v) for v in frac]
+            if velocity:
+                t_s = time.time()
+                seg = sym[idx // GAP + 1] - sym[idx // GAP]
+                vel = group_velocity(x[:, :nev], A_func, direction=seg, side=-1)
+                timing["velocity"] += time.time() - t_s
+                gap_rec_vel[idx] = [None if np.isnan(v) else float(v) for v in vel]
             gap_rec_it[idx] = [float(v) for v in iters[:2]]
             gap_rec_fq[idx] = [float(v) for v in lambdas_re]
         except Exception as e:          # same policy as the reference: record [-1,-1], restart from random
@@ -320,11 +429,15 @@ def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indice
             gap_rec_fq[idx] = [-1.0] * nev
             if energy:
                 gap_rec_en[idx] = [-1.0] * nev
+            if velocity:
+                gap_rec_vel[idx] = [-1.0] * nev
         del x0
         t_h = time.time()
         gap_lib[var_it], gap_lib[var_fq] = gap_rec_it, gap_rec_fq
         if energy:
             gap_lib[var_en] = gap_rec_en
+        if velocity:
+            gap_lib[var_vel] = gap_rec_vel
         with open(path_bandgap, "w") as f:
             json.dump(gap_lib, f, indent=4)
         timing["checkpoint"] += time.time() - t_h
@@ -351,9 +464,11 @@ def kpath_chunks(n_k, world):
 
 def merge_records(parts, n_k, nev=NEV):
     """Combine per-rank {"iterations": {idx: [it, s]}, "frequencies": {idx: [...]}} rows into full-path lists.
-    When the parts carry "energy_fraction" rows (bandgap_sharded(..., energy=True)), a third list of them is returned too."""
+    When the parts carry "energy_fraction" rows (bandgap_sharded(..., energy=True)), a third list of them is returned too.
+    When they carry "group_velocity" rows (velocity=True), four lists are returned: (its, fqs, energy rows or None, velocity rows)."""
     its, fqs = [[0, 0] for _ in range(n_k)], [[0] * nev for _ in range(n_k)]
     ens = [[0] * nev for _ in range(n_k)] if any("energy_fraction" in p for p in parts) else None
+    vels = [[0] * nev for _ in range(n_k)] if any("group_velocity" in p for p in parts) else None
     for p in parts:
         for idx, row in p["iterations"].items():
             its[int(idx)] = row
@@ -361,15 +476,20 @@ def merge_records(parts, n_k, nev=NEV):
             fqs[int(idx)] = row
         for idx, row in p.get("energy_fraction", {}).items():
             ens[int(idx)] = row
+        for idx, row in p.get("group_velocity", {}).items():
+            vels[int(idx)] = row
+    if vels is not None:
+        return its, fqs, ens, vels
     return (its, fqs) if ens is None else (its, fqs, ens)
 
 
 def bandgap_sharded(n, d_flag, rank, world, type=TYPE0, eps_opt=0, nev=NEV, seed=1000, out_dir=None, indices=None,
-                    gather=None, tol=TOL / SCAL / SCAL, retry=1, energy=False):
+                    gather=None, tol=TOL / SCAL / SCAL, retry=1, energy=False, velocity=False):
     """k-path sharding over `world` processes (one GPU each): rank r solves chunk r of the path (or of `indices`)
     into its own JSON file; with `gather` (callable: obj -> list of objs on rank 0, e.g. a torch.distributed
     gather_object wrapper) rank 0 merges all rows into the reference-format file.  No collective touches the data path.
-    energy=True: bandgap(..., energy=True) on every rank, and the energy-fraction rows are merged as well."""
+    energy=True: bandgap(..., energy=True) on every rank, and the energy-fraction rows are merged as well; velocity=True the
+    same for the group-velocity rows."""
     all_idx = list(range(diel.kpath(d_flag, GAP).shape[0])) if indices is None else list(indices)
     mine = [all_idx[i] for i in kpath_chunks(len(all_idx), world)[rank]]
     out_dir = out_dir or (OUTPUT_PATH + type + "/")
@@ -378,7 +498,7 @@ def bandgap_sharded(n, d_flag, rank, world, type=TYPE0, eps_opt=0, nev=NEV, seed
     if os.path.exists(part_path):
         os.remove(part_path)
     errs = bandgap(n, d_flag, type=type, eps_opt=eps_opt, indices=mine, nev=nev, seed=seed, path=part_path, tol=tol,
-                   energy=energy) if mine else []
+                   energy=energy, velocity=velocity) if mine else []
     # A warm start can make [X W] numerically rank deficient (e.g. the point after Gamma, whose zero modes are pure gradients):
     # the reference records [-1,-1] and recomputes such rows from a random start when bandgap() is called again
     # (numerical_experiments.py:370-390); do that second call here.
@@ -386,10 +506,12 @@ def bandgap_sharded(n, d_flag, rank, world, type=TYPE0, eps_opt=0, nev=NEV, seed
         if not errs:
             break
         errs = bandgap(n, d_flag, type=type, eps_opt=eps_opt, indices=None, nev=nev, seed=seed + 7919 * (attempt + 1),
-                       path=part_path, tol=tol, only=errs, energy=energy)
+                       path=part_path, tol=tol, only=errs, energy=energy, velocity=velocity)
     rows = {"iterations": {}, "frequencies": {}, "errors": errs}
     if energy:
         rows["energy_fraction"] = {}
+    if velocity:
+        rows["group_velocity"] = {}
     if mine:
         with open(part_path) as f:
             lib = json.load(f)
@@ -398,6 +520,8 @@ def bandgap_sharded(n, d_flag, rank, world, type=TYPE0, eps_opt=0, nev=NEV, seed
             rows["frequencies"][idx] = lib[f"{d_flag}_{n}_frequencies"][idx]
             if energy:
                 rows["energy_fraction"][idx] = lib[f"{d_flag}_{n}_energy_fraction"][idx]
+            if velocity:
+                rows["group_velocity"][idx] = lib[f"{d_flag}_{n}_group_velocity"][idx]
     if gather is None:
         return rows
     parts = gather(rows)
@@ -411,8 +535,10 @@ def bandgap_sharded(n, d_flag, rank, world, type=TYPE0, eps_opt=0, nev=NEV, seed
             with open(final) as f:
                 lib = json.load(f)
         lib[f"{d_flag}_{n}_iterations"], lib[f"{d_flag}_{n}_frequencies"] = its, fqs
-        if len(merged) == 3:
+        if len(merged) >= 3 and merged[2] is not None:
             lib[f"{d_flag}_{n}_energy_fraction"] = merged[2]
+        if len(merged) == 4:
+            lib[f"{d_flag}_{n}_group_velocity"] = merged[3]
         with open(final, "w") as f:
             json.dump(lib, f, indent=4)
     return rows

@@ -115,6 +115,22 @@ class Operator:
                                                e_tot.ctypes.data_as(L.c_double_p)), "pcb_field_energy")
         return e_in, e_tot
 
+    def band_velocity(self, X):
+        """(V, xx, xax) of the columns of X (n <= 32): V (3, n, n) complex, V[d] = X^H (dA/dalpha_d) X (Hermitian), xx[j] =
+        x_j^H x_j, xax[j] = Re x_j^H A x_j -- see pcb_band_velocity in include/pcb200.h.  dA/dalpha_d comes from
+        FourierSymbols.dtables of this operator's symbols.  X: a DeviceBlock on this operator's context (column views welcome)
+        or a host array (3n^3, k) / (3n^3,), uploaded."""
+        X, _ = devarray.as_block(self.ctx, X)
+        n = X.k
+        V = np.zeros((3, n, n), dtype=np.complex128)
+        xx, xax = np.zeros(n), np.zeros(n)
+        if n:
+            dt = np.ascontiguousarray(self.a_fft.dtables, dtype=np.complex128)
+            L.check(self._lib.pcb_band_velocity(self.h, n, L.ptr_array(X.ptrs), dt.view(np.float64).ctypes.data_as(L.c_double_p),
+                                                V.ctypes.data, xx.ctypes.data_as(L.c_double_p),
+                                                xax.ctypes.data_as(L.c_double_p)), "pcb_band_velocity")
+        return V, xx, xax
+
     def update_resid(self, m, n_loc, s_loc, hs_loc, P, HP, E, lambdas, W):
         """_sep_update_after_rr (lobpcg.py:1248-1270) fused with the next iteration's residual, norms and preconditioner
         (:394-397,442): returns ||lambda_j x_j - hx_j||_2 of the UPDATED X, HX; W receives K_P^-1 of those residuals."""
