@@ -647,12 +647,15 @@ static int launch_crossdof_t(pcb_op* o, int kc, const PcbCols& cols) {
 }
 
 // Pass structure of an A / H apply (DESIGN.md 3): 0 plane mode (3 passes), 1 five passes, 2 five passes split around the
-// cross-DoF stencil (7 kernels), 3 plane mode split around the stencil on the slot layout (5 kernels)
+// cross-DoF stencil (7 kernels), 3 plane mode split around the stencil on the slot layout (5 kernels), 4 plane halves with the
+// stencil fused into the inverse half (4 kernels)
 enum { PCB_STRUCT_PLANE = 0, PCB_STRUCT_FIVE = 1, PCB_STRUCT_CROSS7 = 2, PCB_STRUCT_CROSS5 = 3, PCB_STRUCT_CROSS4 = 4 };
+// A / H of this context run on the plane layout (transposed scratch columns) for every dielectric kind that has a plane structure
+static bool plane_layout(const pcb_ctx* c) { return c->use_plane && (c->zsplit || c->plan->plane_split != 2); }
 static int apply_structure(const pcb_op* o) {
     const pcb_ctx* c = o->ctx;
     const int diel = o->d.diel;
-    if (c->use_plane && (c->zsplit || c->plan->plane_split != 2)) {
+    if (plane_layout(c)) {
         if (diel == PCB_DIEL_NONE || diel == PCB_DIEL_CHIRAL) return PCB_STRUCT_PLANE;
         if (diel == PCB_DIEL_TRIVIAL && c->use_plane_coupled && (c->zsplit ? c->plan->plane_split_coupled : c->plan->plane_coupled)) return PCB_STRUCT_PLANE;
         if (diel == PCB_DIEL_CROSSDOF && c->use_plane_cross) return c->use_plane_cross == 2 ? PCB_STRUCT_CROSS5 : PCB_STRUCT_CROSS4;
@@ -682,92 +685,107 @@ static int check_inplace(const pcb_op* o, int mode, int ncols, const void* const
     return 0;
 }
 
-// A / H on kc columns (cols.in -> cols.out).  dist: the x passes read / write the slabs of all ranks through o->d.dist
-// (large-grid mode over peer memory); cols.in then holds the local X copies and cols.out local work columns.
-// (dist bit 0: the input columns are distributed, bit 1: the output columns are.)
+// One kernel of an apply: a pass id, or the cross-DoF stencil on the natural layout (STENCIL: scratch -> out) or on the
+// plane-slot layout (STENCIL_T: cols.wrk -> out).  The columns it runs on: IO in -> out; SCR in -> the scratch (a natural-layout
+// pass with the scratch as its `out`); WRK in / out with the scratch as the transposed work columns cols.wrk (plane layout).
+enum { PCB_STEP_STENCIL = -1, PCB_STEP_STENCIL_T = -2 };
+enum { PCB_COLS_IO = 0, PCB_COLS_SCR = 1, PCB_COLS_WRK = 2 };
+struct PcbStep { int kern, cols; };
+struct PcbSteps { int n; PcbStep s[7]; };
+
 // mode PCB_APPLY_EFOURIER runs the passes of A with a plain inverse x pass last (no K_A): out = IFFT3(M FFT3(K_A^H x)).
+// dist bit 0: the first x pass reads the input slabs of all ranks through o->d.dist, bit 1: the last x pass writes the output slabs.
 static int last_pass(int mode, bool dout, bool trn) {
     if (mode == PCB_APPLY_EFOURIER) return trn ? PCB_PASS_XINV_T : PCB_PASS_XINV;
     if (mode == PCB_APPLY_A) return trn ? (dout ? PCB_PASS_XINV_A_TD : PCB_PASS_XINV_A_T) : (dout ? PCB_PASS_XINV_A_D : PCB_PASS_XINV_A);
     return trn ? (dout ? PCB_PASS_XINV_H_TD : PCB_PASS_XINV_H_T) : (dout ? PCB_PASS_XINV_H_D : PCB_PASS_XINV_H);
 }
-static int apply_AH(pcb_op* o, int mode, PcbCols& cols, int kc, int j0, int dist) {
-    pcb_ctx* c = o->ctx;
-    const PcbOpLaunch* pl = c->plan;
+static PcbSteps structure_steps(int st, int mode, int dist) {
     const bool din = dist & 1, dout = dist & 2;
     const int first = din ? PCB_PASS_XFWD_SYM_D : PCB_PASS_XFWD_SYM, first_t = din ? PCB_PASS_XFWD_SYM_TD : PCB_PASS_XFWD_SYM_T;
     const int last = last_pass(mode, dout, false), last_t = last_pass(mode, dout, true);
+    enum { IO = PCB_COLS_IO, SCR = PCB_COLS_SCR, WRK = PCB_COLS_WRK };
+    switch (st) {
+        case PCB_STRUCT_PLANE:      // x forward -> transposed scratch, fused y/z/M/z/y on (i1,i2) planes, x inverse -> out
+            // (Round 2, measured and removed: running the three passes on chunks of 1 / 2 / 4 columns so that the scratch of a chunk
+            // (83 MB per column) could stay in the 126 MB L2 between the passes: 2.76 / 2.44 / 2.22 ms instead of 2.02 ms per 16
+            // columns -- the per-chunk launches lose more in partial waves (360 planes per column on 148 SMs) than L2 residency returns.)
+            return {3, {{first_t, WRK}, {PCB_PASS_MID, WRK}, {last_t, WRK}}};
+        case PCB_STRUCT_CROSS4:     // x forward -> scratch, forward half of the plane pass scratch -> out (real-space planes, slot
+                                    // layout), inverse half with the stencil applied on load out -> scratch, x inverse scratch -> out
+            return {4, {{first_t, WRK}, {PCB_PASS_MID_FWD_O, WRK}, {PCB_PASS_MID_INV_ST, WRK}, {last_t, WRK}}};
+        case PCB_STRUCT_CROSS5:     // x forward -> scratch, forward half of the plane pass in place, stencil scratch -> out (slot
+                                    // layout), inverse half out -> scratch, x inverse scratch -> out
+            return {5, {{first_t, WRK}, {PCB_PASS_MID_FWD, WRK}, {PCB_STEP_STENCIL_T, WRK}, {PCB_PASS_MID_INV, WRK}, {last_t, WRK}}};
+        case PCB_STRUCT_CROSS7:     // cross-DoF M is a stencil in real space: forward passes into scratch, M scratch -> out, inverse in place
+            return {7, {{first, SCR}, {PCB_PASS_YFWD, SCR}, {PCB_PASS_ZFWD, SCR}, {PCB_STEP_STENCIL, SCR},
+                        {PCB_PASS_ZINV, IO}, {PCB_PASS_YINV, IO}, {last, IO}}};
+        default:
+            return {5, {{first, IO}, {PCB_PASS_YFWD, IO}, {PCB_PASS_ZMID, IO}, {PCB_PASS_YINV, IO}, {last, IO}}};
+    }
+}
+// The kernels of an A / H / EFOURIER apply in launch order
+static PcbSteps apply_steps(const pcb_op* o, int mode, int dist) {
     int st = apply_structure(o);
-    if (dist && c->zsplit) st = (o->d.diel == PCB_DIEL_CROSSDOF) ? PCB_STRUCT_CROSS7 : PCB_STRUCT_FIVE;      // no peer-memory x passes on split tiles
-    if (refuses_inplace_AH(mode, st) || dist)      // (pcb_apply has checked all its columns already; pcb_apply_dist has not)
+    if (dist && o->ctx->zsplit) st = (o->d.diel == PCB_DIEL_CROSSDOF) ? PCB_STRUCT_CROSS7 : PCB_STRUCT_FIVE;      // no peer-memory x passes on split tiles
+    return structure_steps(st, mode, dist);
+}
+// The forward half of a layout, D = FFT3(K_A^H x): the steps of its split structure (CROSS5 on the plane layout, CROSS7 on the
+// natural layout) before the stencil
+static PcbSteps forward_steps(bool plane) {
+    PcbSteps p = structure_steps(plane ? PCB_STRUCT_CROSS5 : PCB_STRUCT_CROSS7, PCB_APPLY_A, 0);
+    p.n = 0;
+    while (p.s[p.n].kern >= 0) ++p.n;
+    return p;
+}
+
+// Runs the steps on kc columns (cols.in -> cols.out) with the context's scratch where a step uses it, counting one launch per
+// kernel.  ev (pcb_apply_timed): ev[0] is recorded once the scratch is set up, ev[i + 1] after step i.
+static int run_steps(pcb_op* o, const PcbSteps& p, PcbCols cols, int kc, cudaEvent_t* ev = nullptr) {
+    pcb_ctx* c = o->ctx;
+    bool scratch = false;
+    for (int i = 0; i < p.n; ++i) scratch |= (p.s[i].cols != PCB_COLS_IO);
+    PcbCols sc = cols;
+    if (scratch) {
+        if (ensure_scratch(c, sizeof(cplx) * (size_t)c->R * (size_t)kc)) return -1;
+        for (int j = 0; j < kc; ++j) cols.wrk[j] = sc.wrk[j] = sc.out[j] = c->scratch + (size_t)j * c->R;
+    }
+    if (ev) PCB_CUDA_OK(cudaEventRecord(ev[0], c->stream));
+    for (int i = 0; i < p.n; ++i) {
+        const int k = p.s[i].kern;
+        if (k == PCB_STEP_STENCIL) { if (launch_crossdof(o, kc, sc.out, cols.out)) return -1; }
+        else if (k == PCB_STEP_STENCIL_T) { if (launch_crossdof_t(o, kc, cols)) return -1; }
+        else {
+            if (c->plan->pass(o->d, p.s[i].cols == PCB_COLS_SCR ? sc : cols, kc, k, c->tw, c->stream, c->sms)) return -1;
+            c->launches++;
+        }
+        if (ev) PCB_CUDA_OK(cudaEventRecord(ev[i + 1], c->stream));
+    }
+    return 0;
+}
+
+// A / H on kc columns (cols.in -> cols.out).  dist: the x passes read / write the slabs of all ranks through o->d.dist
+// (large-grid mode over peer memory); cols.in then holds the local X copies and cols.out local work columns.
+static int apply_AH(pcb_op* o, int mode, const PcbCols& cols, int kc, int j0, int dist) {
+    if (refuses_inplace_AH(mode, apply_structure(o)) || dist)      // (pcb_apply has checked all its columns already; pcb_apply_dist has not)
         for (int j = 0; j < kc; ++j)
             if (cols.in[j] == cols.out[j]) {
                 pcb_set_error("pcb_apply: in[%d] == out[%d]; this pass structure re-reads X / uses out as work space, use distinct columns", j0 + j, j0 + j);
                 return -2;
             }
-    if (st == PCB_STRUCT_PLANE) {
-        // three passes: x forward -> transposed scratch, fused y/z/M/z/y on (i1,i2) planes, x inverse -> out
-        if (ensure_scratch(c, sizeof(cplx) * (size_t)c->R * (size_t)kc)) return -1;
-        for (int j = 0; j < kc; ++j) cols.wrk[j] = c->scratch + (size_t)j * c->R;
-        const int seq[3] = {first_t, PCB_PASS_MID, last_t};
-        // (Round 2, measured and removed: running the three passes on chunks of 1 / 2 / 4 columns so that the scratch of a chunk
-        // (83 MB per column) could stay in the 126 MB L2 between the passes: 2.76 / 2.44 / 2.22 ms instead of 2.02 ms per 16 columns --
-        // the per-chunk launches lose more in partial waves (360 planes per column on 148 SMs) than L2 residency returns.)
-        for (int i = 0; i < 3; ++i) if (pl->pass(o->d, cols, kc, seq[i], c->tw, c->stream, c->sms)) return -1;
-        c->launches += 3;
-    } else if (st == PCB_STRUCT_CROSS4) {
-        // x forward -> scratch, forward half of the plane pass scratch -> out (real-space planes, slot layout), inverse half with
-        // the stencil applied on load out -> scratch, x inverse scratch -> out
-        if (ensure_scratch(c, sizeof(cplx) * (size_t)c->R * (size_t)kc)) return -1;
-        for (int j = 0; j < kc; ++j) cols.wrk[j] = c->scratch + (size_t)j * c->R;
-        const int seq[4] = {first_t, PCB_PASS_MID_FWD_O, PCB_PASS_MID_INV_ST, last_t};
-        for (int i = 0; i < 4; ++i) if (pl->pass(o->d, cols, kc, seq[i], c->tw, c->stream, c->sms)) return -1;
-        c->launches += 4;
-    } else if (st == PCB_STRUCT_CROSS5) {
-        // x forward -> scratch, forward half of the plane pass in place, stencil scratch -> out (slot layout),
-        // inverse half out -> scratch, x inverse scratch -> out
-        if (ensure_scratch(c, sizeof(cplx) * (size_t)c->R * (size_t)kc)) return -1;
-        for (int j = 0; j < kc; ++j) cols.wrk[j] = c->scratch + (size_t)j * c->R;
-        if (pl->pass(o->d, cols, kc, first_t, c->tw, c->stream, c->sms)) return -1;
-        if (pl->pass(o->d, cols, kc, PCB_PASS_MID_FWD, c->tw, c->stream, c->sms)) return -1;
-        if (launch_crossdof_t(o, kc, cols)) return -1;
-        if (pl->pass(o->d, cols, kc, PCB_PASS_MID_INV, c->tw, c->stream, c->sms)) return -1;
-        if (pl->pass(o->d, cols, kc, last_t, c->tw, c->stream, c->sms)) return -1;
-        c->launches += 4;   // + the stencil launch counted in launch_crossdof_t
-    } else if (st == PCB_STRUCT_FIVE) {
-        const int seq[5] = {first, PCB_PASS_YFWD, PCB_PASS_ZMID, PCB_PASS_YINV, last};
-        for (int i = 0; i < 5; ++i) if (pl->pass(o->d, cols, kc, seq[i], c->tw, c->stream, c->sms)) return -1;
-        c->launches += 5;
-    } else {
-        // cross-DoF M is a stencil in real space: forward passes into scratch, M scratch -> out, inverse in place
-        if (ensure_scratch(c, sizeof(cplx) * (size_t)c->R * (size_t)kc)) return -1;
-        PcbCols tmp = cols;
-        for (int j = 0; j < kc; ++j) tmp.out[j] = c->scratch + (size_t)j * c->R;
-        const int fwd[3] = {first, PCB_PASS_YFWD, PCB_PASS_ZFWD};
-        for (int i = 0; i < 3; ++i) if (pl->pass(o->d, tmp, kc, fwd[i], c->tw, c->stream, c->sms)) return -1;
-        if (launch_crossdof(o, kc, tmp.out, cols.out)) return -1;
-        const int inv[3] = {PCB_PASS_ZINV, PCB_PASS_YINV, last};
-        for (int i = 0; i < 3; ++i) if (pl->pass(o->d, cols, kc, inv[i], c->tw, c->stream, c->sms)) return -1;
-        c->launches += 6;   // + the stencil launch counted in launch_crossdof
-    }
-    return 0;
+    return run_steps(o, apply_steps(o, mode, dist), cols, kc);
 }
 
-// D = FFT3(K_A^H x) (DFIELD) or E = M D (EFIELD) in the natural layout: the forward x (with K_A^H), y and z passes, then for E
-// the point-wise M in place on out, or the cross-DoF stencil from the scratch into out.
+// D = FFT3(K_A^H x) (DFIELD) or E = M D (EFIELD) in the natural layout: the forward half, then for E the point-wise M in place
+// on out, or the cross-DoF stencil from the scratch into out.
 static int apply_field(pcb_op* o, int mode, const PcbCols& cols, int kc) {
     pcb_ctx* c = o->ctx;
     const bool stencil = (mode == PCB_APPLY_EFIELD && o->d.diel == PCB_DIEL_CROSSDOF);
-    PcbCols f = cols;
-    if (stencil) {
-        if (ensure_scratch(c, sizeof(cplx) * (size_t)c->R * (size_t)kc)) return -1;
-        for (int j = 0; j < kc; ++j) f.out[j] = c->scratch + (size_t)j * c->R;
-    }
-    const int fwd[3] = {PCB_PASS_XFWD_SYM, PCB_PASS_YFWD, PCB_PASS_ZFWD};
-    for (int i = 0; i < 3; ++i) if (c->plan->pass(o->d, f, kc, fwd[i], c->tw, c->stream, c->sms)) return -1;
-    c->launches += 3;
-    if (mode != PCB_APPLY_EFIELD || o->d.diel == PCB_DIEL_NONE) return 0;
-    if (stencil) return launch_crossdof(o, kc, f.out, cols.out);
+    PcbSteps p = forward_steps(false);
+    if (stencil) p.s[p.n++] = {PCB_STEP_STENCIL, PCB_COLS_SCR};
+    else for (int i = 0; i < p.n; ++i) p.s[i].cols = PCB_COLS_IO;      // D straight into out
+    if (run_steps(o, p, cols, kc)) return -1;
+    if (mode != PCB_APPLY_EFIELD || o->d.diel == PCB_DIEL_NONE || stencil) return 0;
     for (int j = 0; j < kc; ++j) {
         dim3 grid((unsigned)grid_for(c, c->nn, 256, 8), 1, 1);
         PCB_LAUNCH(k_diel_point, grid, dim3(256, 1, 1), 0, c->stream, o->d, cols.out[j], cols.out[j]);
@@ -849,44 +867,16 @@ int pcb_apply_timed(pcb_op* o, int mode, int ncols, const void* const* in, void*
     PCB_CUDA_OK(cudaSetDevice(c->device));
     PcbCols cols;
     for (int j = 0; j < ncols; ++j) { cols.in[j] = (const cplx*)in[j]; cols.out[j] = (cplx*)out[j]; }
-    const int st = apply_structure(o);
-    const int last = mode == PCB_APPLY_A ? PCB_PASS_XINV_A : PCB_PASS_XINV_H, last_t = mode == PCB_APPLY_A ? PCB_PASS_XINV_A_T : PCB_PASS_XINV_H_T;
-    // kernels of the structure in launch order; -1 / -2 = the cross-DoF stencil (natural / slot layout); up to 7 entries
-    enum { STENCIL = -1, STENCIL_T = -2 };
-    int seq[7] = {PCB_PASS_XFWD_SYM, PCB_PASS_YFWD, PCB_PASS_ZMID, PCB_PASS_YINV, last, 0, 0};
-    int n = 5;
-    if (st != PCB_STRUCT_FIVE) if (ensure_scratch(c, sizeof(cplx) * (size_t)c->R * (size_t)ncols)) return -1;
-    PcbCols fwd = cols;      // CROSS7: the forward passes run on the scratch columns
-    if (st == PCB_STRUCT_PLANE) {
-        for (int j = 0; j < ncols; ++j) cols.wrk[j] = c->scratch + (size_t)j * c->R;
-        seq[0] = PCB_PASS_XFWD_SYM_T; seq[1] = PCB_PASS_MID; seq[2] = last_t; n = 3;
-    } else if (st == PCB_STRUCT_CROSS4) {
-        for (int j = 0; j < ncols; ++j) cols.wrk[j] = c->scratch + (size_t)j * c->R;
-        seq[0] = PCB_PASS_XFWD_SYM_T; seq[1] = PCB_PASS_MID_FWD_O; seq[2] = PCB_PASS_MID_INV_ST; seq[3] = last_t; n = 4;
-    } else if (st == PCB_STRUCT_CROSS5) {
-        for (int j = 0; j < ncols; ++j) cols.wrk[j] = c->scratch + (size_t)j * c->R;
-        seq[0] = PCB_PASS_XFWD_SYM_T; seq[1] = PCB_PASS_MID_FWD; seq[2] = STENCIL_T; seq[3] = PCB_PASS_MID_INV; seq[4] = last_t; n = 5;
-    } else if (st == PCB_STRUCT_CROSS7) {
-        for (int j = 0; j < ncols; ++j) fwd.out[j] = c->scratch + (size_t)j * c->R;
-        seq[0] = PCB_PASS_XFWD_SYM; seq[1] = PCB_PASS_YFWD; seq[2] = PCB_PASS_ZFWD; seq[3] = STENCIL; seq[4] = PCB_PASS_ZINV; seq[5] = PCB_PASS_YINV; seq[6] = last; n = 7;
-    }
+    const PcbSteps p = apply_steps(o, mode, 0);
     cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
 #define PCB_EV_FREE do { for (int q = 0; q < 8; ++q) if (ev[q]) cudaEventDestroy(ev[q]); } while (0)
     for (int i = 0; i < 8; ++i) PCB_CUDA_OK_OR(cudaEventCreate(&ev[i]), PCB_EV_FREE);
-    PCB_CUDA_OK_OR(cudaEventRecord(ev[0], c->stream), PCB_EV_FREE);
-    for (int i = 0; i < n; ++i) {
-        int rc;
-        if (seq[i] == STENCIL) rc = launch_crossdof(o, ncols, fwd.out, cols.out);
-        else if (seq[i] == STENCIL_T) rc = launch_crossdof_t(o, ncols, cols);
-        else { rc = c->plan->pass(o->d, (st == PCB_STRUCT_CROSS7 && i < 3) ? fwd : cols, ncols, seq[i], c->tw, c->stream, c->sms); c->launches++; }
-        if (rc) { cudaStreamSynchronize(c->stream); PCB_EV_FREE; return -1; }
-        PCB_CUDA_OK_OR(cudaEventRecord(ev[i + 1], c->stream), PCB_EV_FREE);
-    }
-    PCB_CUDA_OK_OR(cudaEventSynchronize(ev[n]), PCB_EV_FREE);
-    for (int i = 0; i < n; ++i) PCB_CUDA_OK_OR(cudaEventElapsedTime(&pass_ms[i], ev[i], ev[i + 1]), PCB_EV_FREE);
+    if (run_steps(o, p, cols, ncols, ev)) { cudaStreamSynchronize(c->stream); PCB_EV_FREE; return -1; }
+    PCB_CUDA_OK_OR(cudaEventSynchronize(ev[p.n]), PCB_EV_FREE);
+    for (int i = 0; i < p.n; ++i) PCB_CUDA_OK_OR(cudaEventElapsedTime(&pass_ms[i], ev[i], ev[i + 1]), PCB_EV_FREE);
     PCB_EV_FREE;
 #undef PCB_EV_FREE
-    *npass = n;
+    *npass = p.n;
     return 0;
 }
 
@@ -913,27 +903,14 @@ static const unsigned char* energy_slot_mask(pcb_op* o) {
 
 // e_in / e_tot of kc columns: forward passes into the scratch (the plane layout where A / H run in plane mode, else the natural
 // layout), the energy kernel over a fixed grid of gx CTAs per column, then the fixed-order sum of the partials into `dout`.
-static int field_energy_chunk(pcb_op* o, const PcbCols& cols, int kc, int plane, const unsigned char* smask, int gx, double* dout) {
+static int field_energy_chunk(pcb_op* o, const PcbCols& cols, int kc, bool plane, const unsigned char* smask, int gx, double* dout) {
     pcb_ctx* c = o->ctx;
-    const PcbOpLaunch* pl = c->plan;
-    PcbCols f = cols, e;
+    if (run_steps(o, forward_steps(plane), cols, kc)) return -1;
+    PcbCols e;
     memset(&e, 0, sizeof e);
-    for (int j = 0; j < kc; ++j) {
-        cplx* s = c->scratch + (size_t)j * c->R;
-        f.wrk[j] = s; f.out[j] = s; e.in[j] = s;
-    }
+    for (int j = 0; j < kc; ++j) e.in[j] = c->scratch + (size_t)j * c->R;
     PcbOp d = o->d;
-    if (plane) {
-        // x forward -> transposed scratch, forward half of the plane pass in place: real-space D in the plane-slot layout
-        if (pl->pass(d, f, kc, PCB_PASS_XFWD_SYM_T, c->tw, c->stream, c->sms)) return -1;
-        if (pl->pass(d, f, kc, PCB_PASS_MID_FWD, c->tw, c->stream, c->sms)) return -1;
-        d.maskp = smask;
-    } else {
-        const int fwd[3] = {PCB_PASS_XFWD_SYM, PCB_PASS_YFWD, PCB_PASS_ZFWD};
-        for (int i = 0; i < 3; ++i) if (pl->pass(d, f, kc, fwd[i], c->tw, c->stream, c->sms)) return -1;
-        c->launches++;
-    }
-    c->launches += 2;
+    if (plane) d.maskp = smask;
     const PcbStencil st = d.sten;
     const int k = st.k;
     dim3 grid((unsigned)gx, (unsigned)kc, 1), blk(256, 1, 1);
@@ -969,8 +946,7 @@ int pcb_field_energy(pcb_op* o, int ncols, const void* const* x, double* e_in, d
         return -2;
     }
     PCB_CHECK_ARG(!o->diel || o->diel->zsplit == c->zsplit, "dielectric was created under the other plane-mode form (plane_split); re-create it");
-    // the layout of the A / H plane mode (apply_structure), for every dielectric kind
-    const int plane = (c->use_plane && (c->zsplit || c->plan->plane_split != 2)) ? 1 : 0;
+    const bool plane = plane_layout(c);
     const unsigned char* smask = nullptr;
     if (plane && o->d.diel != PCB_DIEL_NONE && !(smask = energy_slot_mask(o))) return -1;
     const int gx = grid_for(c, c->nn, 256, 4);      // fixed for the context: the same partials for a column at any width

@@ -152,9 +152,6 @@ PCB_D void pcb_bulk_load(void* smem_dst, const void* gsrc, unsigned bytes, unsig
 PCB_D void pcb_bulk_store(void* gdst, const void* smem_src, unsigned bytes) {
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;\n" ::"l"(gdst), "r"(pcb_smem_u32(smem_src)), "r"(bytes) : "memory");
 }
-PCB_D void pcb_bulk_prefetch_l2(const void* gsrc, unsigned bytes) {      // TMA prefetch of a contiguous chunk into L2 (no shared-memory destination)
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;\n" ::"l"(gsrc), "r"(bytes) : "memory");
-}
 PCB_D void pcb_bulk_commit() { asm volatile("cp.async.bulk.commit_group;\n" ::: "memory"); }
 PCB_D void pcb_bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;\n" ::: "memory"); }
 PCB_D void pcb_fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory"); }
@@ -471,10 +468,7 @@ __global__ void __launch_bounds__(NT, (ZS == 2 ? (P::R1 <= 8 ? PCB_XINV_ZS_CTAS 
         for (int l = tid; l < 3 * lines; l += NT)
             pcb_prefetch_l2(reinterpret_cast<const char*>(X + (l / lines) * nn + (long long)row0 * N) + (l % lines) * 128);
     }
-#ifndef PCB_XINV_ZS_PF
-#define PCB_XINV_ZS_PF 1
-#endif
-    if (MODE == 2 && ZS == 2 && PCB_XINV_ZS_PF) {   // ... 3 x ZS chunks of LH rows
+    if (MODE == 2 && ZS == 2) {   // ... 3 x ZS chunks of LH rows
         constexpr int lines = (LH * N * (int)sizeof(cplx) + 127) / 128;
         for (int l = tid; l < 3 * ZS * lines; l += NT) {
             const int ch = l / lines;
@@ -879,11 +873,10 @@ __global__ void k_mask_bits(PcbOp op, unsigned* __restrict__ out) {
 // operator drops from 11 to 7 column transfers per op-apply.  DIEL: 0 identity, 1 component-wise (chiral); the coupled
 // 3x3 dielectrics need all three components of a point and stay on the five-pass path.
 // ---------------------------------------------------------------------------------------
-// TMA = 1 (default on the device): the rows of a plane are moved by bulk copies -- cp.async.bulk, one elected lane per warp
+// TMA = 1 (the device build): the rows of a plane are moved by bulk copies -- cp.async.bulk, one elected lane per warp
 // issues eight row copies against the warp's own mbarrier; the store goes back the same way after a proxy fence -- instead
 // of per-element cp.async / LDS + STG loops: 960 LDGSTS and 960 LDS+STG per warp and plane leave the LSU queue, which the
-// radix steps need (N = 120, 16 columns: 0.884 -> 0.818 ms; PCB200_MID_TMA=0 selects the loop form, which is also what the
-// host-emulation build runs).
+// radix steps need (N = 120, 16 columns: 0.884 -> 0.818 ms).  TMA = 0, the loop form, is what the host-emulation build runs.
 // (Round 2, measured and removed: the radix-R1 steps with two items per lane in flight -- either both loaded before both
 // butterflies, or software-pipelined so that item i+1's loads go out before item i's stores; the shared-memory plane carries no
 // restrict information, so the compiler keeps each trip's loads behind the previous trip's stores.  At the 128-register cap of
@@ -1368,7 +1361,7 @@ __global__ void k_mask_bits2(PcbOp op, unsigned* __restrict__ out) {
 // DIEL = 2: the coupled 3x3 dielectric on clusters of three CTAs, exactly as in k_mid<2>: sweep C is split at real space --
 // forward radix-R2 + diagonal -> plane, cluster barrier, off-diagonal terms at the coupled points of this CTA's third of the rows
 // through distributed shared memory (byte mask in this kernel's slot order, op.maskp2), cluster barrier, inverse radix-R2.
-template <class P, int DIEL, int TMA = 0, int PF = 0>
+template <class P, int DIEL, int TMA = 0>
 __global__ void __launch_bounds__(Mid2<P>::NTHR, 1) k_mid2(PcbOp op, PcbCols cols, const cplx* __restrict__ tw, int ncols) {
     typedef Mid2<P> M2;
     constexpr int N = P::N, R2 = P::R2, LD = N + 1, NTHR = M2::NTHR, CI = M2::CI;
@@ -1416,16 +1409,6 @@ __global__ void __launch_bounds__(Mid2<P>::NTHR, 1) k_mid2(PcbOp op, PcbCols col
                 for (int r = 0; r < nrw; ++r) {
                     const int row = M2::rho(r & 7, 2 * warp + (r >> 3));
                     pcb_bulk_load(pl + row * LD, base + (long long)row * N, N * (unsigned)sizeof(cplx), mybar);
-                }
-                if (PF && DIEL != 2) {      // the rows this warp will load for the CTA's next plane: ask L2 for them now (one TMA prefetch per row)
-                    const int np = pid + gridDim.x;
-                    if (np < 3 * N * ncols) {
-                        const cplx* nb = cols.wrk[np / (3 * N)] + ((np / N) % 3) * nn + (long long)(np % N) * N * N;
-                        for (int r = 0; r < nrw; ++r) {
-                            const int row = M2::rho(r & 7, 2 * warp + (r >> 3));
-                            pcb_bulk_prefetch_l2(nb + (long long)row * N, N * (unsigned)sizeof(cplx));
-                        }
-                    }
                 }
             }
         } else

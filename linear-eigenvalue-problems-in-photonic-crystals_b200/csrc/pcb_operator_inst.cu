@@ -24,18 +24,12 @@ constexpr int kStageX = LX * kRowBytes;               // one x-tile (three compo
 constexpr int NTX = (LX * P::R2 <= 64) ? 64 : NT;
 constexpr int kSmemL = 3 * P::N * 8 * (int)sizeof(cplx);
 constexpr int kSmemZ = 2 * kSmemL;                       // two stages
-// ... else (N >= 160) single-stage tiles with 2-3 CTAs of 256 threads per SM.  (Round 2, measured: when two stages still fit ONCE,
-// one CTA of 512 threads per SM with the cp.async double buffer -- the same 16 warps and pipeline depth per SM as the small
-// sizes, no spills -- is slower: N = 160, 16 columns 2.09 vs 1.79 ms, N = 256, 8 columns 4.08 vs 3.31 ms; build with
-// -DPCB_ZMID_WIDE=1 to get that form.)
-#ifndef PCB_ZMID_WIDE
-#define PCB_ZMID_WIDE 0
-#endif
+// ... else (N >= 160) single-stage tiles with 2-3 CTAs of 256 threads per SM.  (Round 2, measured and removed: when two stages still
+// fit ONCE, one CTA of 512 threads per SM with the cp.async double buffer -- the same 16 warps and pipeline depth per SM as the small
+// sizes, no spills -- is slower: N = 160, 16 columns 2.09 vs 1.79 ms, N = 256, 8 columns 4.08 vs 3.31 ms.)
 constexpr bool kZTwice = 2 * (kSmemZ + 1024) <= 224 * 1024;
-constexpr bool kZWide = !kZTwice && PCB_ZMID_WIDE && (kSmemZ + 1024 <= 227 * 1024);
-constexpr int NSTZ = (kZTwice || kZWide) ? 2 : 1;         // ... else single-stage tiles, still several CTAs per SM
+constexpr int NSTZ = kZTwice ? 2 : 1;         // ... else single-stage tiles, still several CTAs per SM
 constexpr int kSmemZU = NSTZ * kSmemL;
-constexpr int NTZ = kZWide ? 512 : NTP;
 
 template <class K>
 int set_smem(K kern, int bytes) {
@@ -96,6 +90,15 @@ constexpr bool kPlaneSplitCoupled = false;
 #else
 constexpr bool kPlaneSplitCoupled = kPlaneSplit;      // coupled 3x3 M on clusters of three CTAs, one half plane per cluster
 #endif
+// plane passes (k_mid / k_mid2) move their rows by TMA bulk copies on the device (one mbarrier per warp behind the plane, at most
+// 128 bytes) and by row loops under host emulation
+#ifdef PCB_EMU
+constexpr int kTma = 0;
+#else
+constexpr int kTma = 1;
+#endif
+static_assert(!kPlane || kSmemMid + 128 <= 232448, "whole plane + mbarriers exceed a CTA's shared memory");
+static_assert(!kPlaneSplit || (P::N / 2) * (P::N + 1) * (int)sizeof(cplx) + 128 <= 232448, "half plane + mbarriers exceed a CTA's shared memory");
 constexpr int kStageXT = 3 * LX * (P::R1 * P::R2P + 1) * (int)sizeof(cplx);
 
 constexpr int GX = (P::N * P::N + LX - 1) / LX;          // x tiles per column
@@ -119,7 +122,6 @@ int launch_cluster3(K kfn, int threads, int smem, int planes, const PcbOp& op, c
     if (max_clusters == 0) {
         cfg.gridDim = dim3(3 * 148, 1, 1);
         PCB_CUDA_OK(cudaOccupancyMaxActiveClusters(&max_clusters, kfn, &cfg));
-        if (const char* ev = getenv("PCB200_MID_CLUSTERS")) { const int v = atoi(ev); if (v >= 1 && v < max_clusters) max_clusters = v; }
         if (getenv("PCB200_DEBUG")) fprintf(stderr, "[pcb200] plane pass, coupled M, N = %d, %d threads: %d co-resident clusters of 3 CTAs (%d SMs)\n", N, threads, max_clusters, sms);
         if (max_clusters < 1) { pcb_set_error("plane mode: no 3-CTA cluster of the plane pass fits on this device"); max_clusters = 0; return -1; }
     }
@@ -150,7 +152,7 @@ struct PlaneFive<true, PP> {
             PCB_CUDA_OK(cudaGetLastError());
             return 0;
         }
-        constexpr int smem_tma = PP::N * (PP::N + 1) * (int)sizeof(cplx) + 128;
+        constexpr int smem = PP::N * (PP::N + 1) * (int)sizeof(cplx) + (kTma ? 128 : 0);
         if (pass_id == PCB_PASS_MASKPLANE2) {
             const long long total = (long long)PP::N * PP::N * PP::N;
             PCB_LAUNCH((k_mask_plane2<PP>), dim3((unsigned)((total + 255) / 256), 1, 1), dim3(256, 1, 1), 0, s, op, const_cast<unsigned char*>(op.maskp2));
@@ -159,37 +161,12 @@ struct PlaneFive<true, PP> {
         }
 #ifndef PCB_EMU
         if (op.diel == PCB_DIEL_TRIVIAL) {
-            if (smem_tma > 232448 || PP::N % 3 != 0) { pcb_set_error("five-sweep plane pass: coupled M not available for N = %d", PP::N); return -1; }
-            return launch_cluster3(k_mid2<PP, 2, 1>, M2::NTHR, smem_tma, PP::N * ncols, op, cols, tw, ncols, s, sms, PP::N);
-        }
-        if (smem_tma <= 232448) {
-            static const char* evpf = getenv("PCB200_MID_PF");      // PCB200_MID_PF=1: TMA prefetch of the CTA's next plane into L2
-            if (evpf && evpf[0] == '1') {
-                if (op.diel == PCB_DIEL_NONE) PCB_GO_P((k_mid2<PP, 0, 1, 1>), M2::NTHR, 3 * PP::N, smem_tma, 1);
-                else PCB_GO_P((k_mid2<PP, 1, 1, 1>), M2::NTHR, 3 * PP::N, smem_tma, 1);
-                return 0;
-            }
-            if (op.diel == PCB_DIEL_NONE) PCB_GO_P((k_mid2<PP, 0, 1>), M2::NTHR, 3 * PP::N, smem_tma, 1);
-            else PCB_GO_P((k_mid2<PP, 1, 1>), M2::NTHR, 3 * PP::N, smem_tma, 1);
-            return 0;
+            if (PP::N % 3 != 0) { pcb_set_error("five-sweep plane pass: coupled M not available for N = %d", PP::N); return -1; }
+            return launch_cluster3(k_mid2<PP, 2, 1>, M2::NTHR, smem, PP::N * ncols, op, cols, tw, ncols, s, sms, PP::N);
         }
 #endif
-        if (op.diel == PCB_DIEL_NONE) PCB_GO_P((k_mid2<PP, 0, 0>), M2::NTHR, 3 * PP::N, smem_tma - 128, 1);
-        else PCB_GO_P((k_mid2<PP, 1, 0>), M2::NTHR, 3 * PP::N, smem_tma - 128, 1);
-        return 0;
-    }
-};
-
-template <bool OK, class PP>
-struct XFwd2 { static int go(const PcbOp&, const PcbCols&, int, const cplx*, cudaStream_t) { return -1; } };
-template <class PP>
-struct XFwd2<true, PP> {
-    static int go(const PcbOp& op, const PcbCols& cols, int ncols, const cplx* tw, cudaStream_t s) {
-        auto kfn = k_xfwd2<PP, LX, NT>;
-        if (set_smem(kfn, kStageXT)) return -1;
-        dim3 grid((unsigned)((GX + 1) / 2), (unsigned)ncols, 1);
-        PCB_LAUNCH(kfn, grid, dim3(NT, 1, 1), (size_t)kStageXT, s, op, cols, tw);
-        PCB_CUDA_OK(cudaGetLastError());
+        if (op.diel == PCB_DIEL_NONE) PCB_GO_P((k_mid2<PP, 0, kTma>), M2::NTHR, 3 * PP::N, smem, 1);
+        else PCB_GO_P((k_mid2<PP, 1, kTma>), M2::NTHR, 3 * PP::N, smem, 1);
         return 0;
     }
 };
@@ -260,68 +237,43 @@ struct PlanePass<true, PP, ZS> {
             PCB_CUDA_OK(cudaGetLastError());
             return 0;
         }
-        constexpr bool kTma = kSmemMidZ + 128 <= 232448;
+// plane pass on whole (ZS = 1) or half (ZS = 2) planes: one CTA per plane, N / ZS / 8 warps
+#define PCB_GO_MID(DIEL, HALF, STEN) PCB_GO_P((k_mid<PP, DIEL, kTma, HALF, STEN, ZS>), PP::N / ZS / 8 * 32, 3 * PP::N * ZS, kSmemMidZ + (kTma ? 128 : 0), 1)
         if (pass_id == PCB_PASS_MID_FWD_O || pass_id == PCB_PASS_MID_INV_ST) {      // ... with the stencil fused into the inverse half
             const int k = op.sten.k;
-#ifndef PCB_EMU
-            if (kTma) {
-                if (pass_id == PCB_PASS_MID_FWD_O) PCB_GO_P((k_mid<PP, 0, 1, 1, 1, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ + 128, 1);
-                else if (k == 1) PCB_GO_P((k_mid<PP, 0, 1, 2, 3, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ + 128, 1);
-                else if (k == 2) PCB_GO_P((k_mid<PP, 0, 1, 2, 5, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ + 128, 1);
-                else PCB_GO_P((k_mid<PP, 0, 1, 2, 1, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ + 128, 1);
-                return 0;
-            }
-#endif
-            if (pass_id == PCB_PASS_MID_FWD_O) PCB_GO_P((k_mid<PP, 0, 0, 1, 1, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ, 1);
-            else if (k == 1) PCB_GO_P((k_mid<PP, 0, 0, 2, 3, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ, 1);
-            else if (k == 2) PCB_GO_P((k_mid<PP, 0, 0, 2, 5, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ, 1);
-            else PCB_GO_P((k_mid<PP, 0, 0, 2, 1, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ, 1);
+            if (pass_id == PCB_PASS_MID_FWD_O) PCB_GO_MID(0, 1, 1);
+            else if (k == 1) PCB_GO_MID(0, 2, 3);
+            else if (k == 2) PCB_GO_MID(0, 2, 5);
+            else PCB_GO_MID(0, 2, 1);
             return 0;
         }
         if (pass_id == PCB_PASS_MID_FWD || pass_id == PCB_PASS_MID_INV) {      // halves of the plane pass (cross-DoF dielectric)
-#ifndef PCB_EMU
-            if (kTma) {
-                if (pass_id == PCB_PASS_MID_FWD) PCB_GO_P((k_mid<PP, 0, 1, 1, 0, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ + 128, 1);
-                else PCB_GO_P((k_mid<PP, 0, 1, 2, 0, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ + 128, 1);
-                return 0;
-            }
-#endif
-            if (pass_id == PCB_PASS_MID_FWD) PCB_GO_P((k_mid<PP, 0, 0, 1, 0, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ, 1);
-            else PCB_GO_P((k_mid<PP, 0, 0, 2, 0, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ, 1);
+            if (pass_id == PCB_PASS_MID_FWD) PCB_GO_MID(0, 1, 0);
+            else PCB_GO_MID(0, 2, 0);
             return 0;
         }
 #ifndef PCB_EMU
         if (pass_id == PCB_PASS_MID && op.diel == PCB_DIEL_TRIVIAL) {
             // coupled 3x3 M: clusters of three CTAs (one component each) exchanging the coupled points through DSMEM
-            static_assert(!kPlaneCoupled || kTma, "the cluster form of the plane pass uses the TMA row copies");
             return Coupled<(ZS == 1 ? kPlaneCoupled : kPlaneSplitCoupled), PP, ZS>::go(op, cols, ncols, pass_id, tw, s, sms);
         }
 #endif
         if (pass_id == PCB_PASS_XFWD_SYM_TD || pass_id == PCB_PASS_XINV_A_TD || pass_id == PCB_PASS_XINV_H_TD)
             return XDist<ZS == 1, PP>::go(op, cols, ncols, pass_id, tw, s);
-        if (ZS == 2) {      // z-split plane mode: x passes with the split tiles, plane pass on half planes
+        if constexpr (ZS == 2) {      // z-split plane mode: x passes with the split tiles, plane pass on half planes
             if (pass_id == PCB_PASS_XFWD_SYM_T) PCB_GO((k_xfwd<PP, LX, NT, 1, 1, 0, ZS>), GX, kStageXT);
             else if (pass_id == PCB_PASS_XINV_A_T) PCB_GO((k_xinv<PP, LX, NT, 1, 1, 0, ZS>), GX, kStageXT);
             else if (pass_id == PCB_PASS_XINV_H_T) PCB_GO((k_xinv<PP, LX, NT, 2, 1, 0, ZS>), GX, kStageXT);
             else if (pass_id == PCB_PASS_XINV_T) PCB_GO((k_xinv<PP, LX, NT, 0, 1, 0, ZS>), GX, kStageXT);
-            else if (pass_id == PCB_PASS_MID && (op.diel == PCB_DIEL_NONE || op.diel == PCB_DIEL_CHIRAL)) {
-#ifndef PCB_EMU
-                if (kTma) {
-                    if (op.diel == PCB_DIEL_NONE) PCB_GO_P((k_mid<PP, 0, 1, 0, 0, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ + 128, 1);
-                    else PCB_GO_P((k_mid<PP, 1, 1, 0, 0, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ + 128, 1);
-                    return 0;
-                }
-#endif
-                if (op.diel == PCB_DIEL_NONE) PCB_GO_P((k_mid<PP, 0, 0, 0, 0, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ, 1);
-                else PCB_GO_P((k_mid<PP, 1, 0, 0, 0, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ, 1);
-            }
+            else if (pass_id == PCB_PASS_MID && op.diel == PCB_DIEL_NONE) PCB_GO_MID(0, 0, 0);
+            else if (pass_id == PCB_PASS_MID && op.diel == PCB_DIEL_CHIRAL) PCB_GO_MID(1, 0, 0);
             else { pcb_set_error("z-split plane mode: pass %d / dielectric type %d not supported", pass_id, op.diel); return -1; }
             return 0;
         }
         if (pass_id == PCB_PASS_XFWD_SYM_T) {
-            static const char* ev2 = getenv("PCB200_XFWD2");      // default: two tiles per CTA, the second tile's loads behind the first tile's radix-R2 phase (PCB200_XFWD2=0: one tile per CTA)
-            // (N = 48: 0.058 vs 0.051 ms -- below N = 64 one tile per CTA stays)
-            if (LX * PP::R2 <= NT && PP::N >= 64 && !(ev2 && ev2[0] == '0')) { if (XFwd2<(LX * PP::R2 <= NT && PP::N >= 64 && ZS == 1), PP>::go(op, cols, ncols, tw, s)) return -1; }
+            // from N = 64 on two tiles per CTA, the second tile's loads behind the first tile's radix-R2 phase (N = 48: 0.058 vs
+            // 0.051 ms -- below N = 64 one tile per CTA stays)
+            if constexpr (LX * PP::R2 <= NT && PP::N >= 64 && ZS == 1) PCB_GO((k_xfwd2<PP, LX, NT>), (GX + 1) / 2, kStageXT);
             else PCB_GO((k_xfwd<PP, LX, NT, 1, 1>), GX, kStageXT);
         }
         else if (pass_id == PCB_PASS_XINV_A_T) PCB_GO((k_xinv<PP, LX, NT, 1, 1>), GX, kStageXT);
@@ -330,18 +282,12 @@ struct PlanePass<true, PP, ZS> {
         else if (pass_id == PCB_PASS_MASKBITS2 || pass_id == PCB_PASS_MASKPLANE2) return PlaneFive<(kPlaneFive && ZS == 1), PP>::go(op, cols, ncols, pass_id, tw, s, sms);
         else if (op.diel == PCB_DIEL_NONE || op.diel == PCB_DIEL_CHIRAL) {
             if (kPlaneFive && ZS == 1 && op.mid_five && (op.diel == PCB_DIEL_NONE || op.mbits2 != nullptr)) return PlaneFive<(kPlaneFive && ZS == 1), PP>::go(op, cols, ncols, pass_id, tw, s, sms);
-            static const char* ev = getenv("PCB200_MID_TMA");
-            const bool tma = !(ev && ev[0] == '0') && kSmemMidZ + 128 <= 232448;      // default; PCB200_MID_TMA=0: cp.async / LDS+STG row loops
-            if (tma) {
-                if (op.diel == PCB_DIEL_NONE) PCB_GO_P((k_mid<PP, 0, 1, 0, 0, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ + 128, 1);
-                else PCB_GO_P((k_mid<PP, 1, 1, 0, 0, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ + 128, 1);
-            } else {
-                if (op.diel == PCB_DIEL_NONE) PCB_GO_P((k_mid<PP, 0, 0, 0, 0, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ, 1);
-                else PCB_GO_P((k_mid<PP, 1, 0, 0, 0, ZS>), (PP::N / ZS / 8 * 32), 3 * PP::N * ZS, kSmemMidZ, 1);
-            }
+            if (op.diel == PCB_DIEL_NONE) PCB_GO_MID(0, 0, 0);
+            else PCB_GO_MID(1, 0, 0);
         }
         else { pcb_set_error("plane mode: dielectric type %d not supported", op.diel); return -1; }
         return 0;
+#undef PCB_GO_MID
     }
 };
 
@@ -360,9 +306,9 @@ int run_pass(const PcbOp& op, const PcbCols& cols, int ncols, int pass_id, const
         case PCB_PASS_XINV_A_D:   PCB_GO((k_xinv<P, LX, NT, 1, 0, 1>), GX, kStageX); break;
         case PCB_PASS_XINV_H_D:   PCB_GO((k_xinv<P, LX, NT, 2, 0, 1>), GX, kStageX); break;
         case PCB_PASS_ZMID:
-            if (op.diel == PCB_DIEL_NONE) PCB_GO_P((k_zmid<P, 0, NTZ, NSTZ>), NTZ, GL, kSmemZU, 3);
-            else if (op.diel == PCB_DIEL_CHIRAL) PCB_GO_P((k_zmid<P, 1, NTZ, NSTZ>), NTZ, GL, kSmemZU, 3);
-            else if (op.diel == PCB_DIEL_TRIVIAL) PCB_GO_P((k_zmid<P, 2, NTZ, NSTZ>), NTZ, GL, kSmemZU, 2);
+            if (op.diel == PCB_DIEL_NONE) PCB_GO_P((k_zmid<P, 0, NTP, NSTZ>), NTP, GL, kSmemZU, 3);
+            else if (op.diel == PCB_DIEL_CHIRAL) PCB_GO_P((k_zmid<P, 1, NTP, NSTZ>), NTP, GL, kSmemZU, 3);
+            else if (op.diel == PCB_DIEL_TRIVIAL) PCB_GO_P((k_zmid<P, 2, NTP, NSTZ>), NTP, GL, kSmemZU, 2);
             else { pcb_set_error("zmid: dielectric type %d has no fused z pass", op.diel); return -1; }
             break;
         case PCB_PASS_XFWD_SYM_T: case PCB_PASS_MID: case PCB_PASS_XINV_A_T: case PCB_PASS_XINV_H_T: case PCB_PASS_MASKBITS:

@@ -101,6 +101,11 @@ def _rel(got, want, floor):
     return np.abs(got - want) / np.maximum(np.abs(want), floor)
 
 
+def _plane_layout(N, options):
+    """A / H run on the plane layout: N % 8 == 0 up to N = 160 (whole or half planes), unless the plane mode is switched off."""
+    return options.get("plane", 1) != 0 and N % 8 == 0 and N <= 160
+
+
 def _with_options(pkg, N, options, fn):
     ctx = pkg.get_context(N)
     try:
@@ -158,8 +163,11 @@ def _check_case(pkg, oc, case, ncols=3, widths=True):
             assert np.all((f >= 0.0) & (f <= 1.0)), f
         # 4. x is read only; a repeated call gives the same bits; a host array is uploaded
         assert np.array_equal(X.get(), x)
+        n0 = ctx.launches()
         again = op.field_energy(X)
         assert np.array_equal(again[0], e_in) and np.array_equal(again[1], e_tot)
+        # the forward half of A's layout (x forward + forward plane half, or x, y and z forward), the energy kernel, the sum
+        assert ctx.launches() - n0 == (2 if _plane_layout(N, options) else 3) + 2, ctx.launches() - n0
         host = op.field_energy(x[:, :1])
         assert host[0][0] == e_in[0] and host[1][0] == e_tot[0]
         if widths:

@@ -79,9 +79,11 @@ def _apply_rc(pkg, op, mode, X, Y):
     return pkg._lib.lib().pcb_apply(op.h, mode, X.k, pkg._lib.ptr_array(X.ptrs), pkg._lib.ptr_array(Y.ptrs))
 
 
-def _apply_timed_rc(pkg, op, mode, X, Y):
+def _apply_timed(pkg, op, mode, X, Y):
+    """pcb_apply_timed: (return code, number of kernels timed)."""
     ms, n = (C.c_float * 8)(), C.c_int()
-    return pkg._lib.lib().pcb_apply_timed(op.h, mode, X.k, pkg._lib.ptr_array(X.ptrs), pkg._lib.ptr_array(Y.ptrs), ms, C.byref(n))
+    rc = pkg._lib.lib().pcb_apply_timed(op.h, mode, X.k, pkg._lib.ptr_array(X.ptrs), pkg._lib.ptr_array(Y.ptrs), ms, C.byref(n))
+    return rc, n.value
 
 
 def _colerr(got, want):
@@ -154,6 +156,13 @@ EMU_CASES = [
 _DEFAULT_OPTIONS = {"mid_five": -1, "plane_cross": 1, "plane_split": 0}
 
 
+def _kernels(struct, N, options):
+    """Kernels of one A / H apply of at most 32 columns, the cross-DoF stencil kernel included."""
+    if struct == STRUCT_CROSS_PLANE:      # stencil fused into the inverse plane half (4), or its own kernel between the halves (5):
+        return 5 if options.get("plane_cross", 2 if N >= 160 else 1) == 2 else 4      # the default of the z-split sizes N >= 160
+    return {STRUCT_PLANE: 3, STRUCT_FIVE: 5, STRUCT_CROSS7: 7}[struct]
+
+
 def _case_id(c):
     opt = "".join(f"-{k}{v}" for k, v in c[4].items())
     return f"N{c[0]}-{c[1]}-{c[2] or 'vacuum'}{opt}"
@@ -194,8 +203,15 @@ def _operator_widths_on(pkg, oc, ctx, case, widths, timed_width):
             op.apply_into(mode, X.cols(range(w)), Y.cols(range(w)))
             eq = _same(pkg, Y1.cols(range(w)), Y.cols(range(w)))
             assert eq.all(), (name, w, np.flatnonzero(~eq))
-        # pcb_apply_timed runs the kernels bench.py's per-pass table reports: the same numbers as pcb_apply
-        L.check(_apply_timed_rc(pkg, op, mode, X.cols(range(timed_width)), Y.cols(range(timed_width))), "pcb_apply_timed")
+        # pcb_apply_timed runs the kernels bench.py's per-pass table reports: the same kernels and numbers as pcb_apply
+        kernels = _kernels(struct, N, options)
+        n0 = ctx.launches()
+        L.check(_apply_rc(pkg, op, mode, X.cols(range(timed_width)), Y.cols(range(timed_width))), "pcb_apply")
+        assert ctx.launches() - n0 == kernels, (name, "pcb_apply launches", ctx.launches() - n0)
+        n0 = ctx.launches()
+        rc, npass = _apply_timed(pkg, op, mode, X.cols(range(timed_width)), Y.cols(range(timed_width)))
+        L.check(rc, "pcb_apply_timed")
+        assert npass == kernels and ctx.launches() - n0 == kernels, (name, "pcb_apply_timed", npass, ctx.launches() - n0)
         assert _same(pkg, Y1.cols(range(timed_width)), Y.cols(range(timed_width))).all(), (name, "timed")
         Y.assign(X)
         rc = _apply_rc(pkg, op, mode, Y, Y)
@@ -218,7 +234,7 @@ def _refused_alias_leaves_outputs(pkg, op, mode, X, Y, j_alias, timed=0):
     probe = (pkg.pcfft.column_norms(X.cols([j_alias])), pkg.pcfft.column_dots(X.cols([j_alias]), X.cols([0])))
     out = pkg.devarray.DeviceBlock(Y.ctx, _owners=Y._owners, _ptrs=Y.ptrs[:k])
     out.ptrs[j_alias] = X.ptrs[j_alias]
-    rc = (_apply_timed_rc if timed else _apply_rc)(pkg, op, mode, X.cols(range(k)), out)
+    rc = _apply_timed(pkg, op, mode, X.cols(range(k)), out)[0] if timed else _apply_rc(pkg, op, mode, X.cols(range(k)), out)
     assert rc == -2, ("aliased column", j_alias, rc)
     assert b"in[" in pkg._lib.lib().pcb_last_error()
     Y.ctx.sync()
