@@ -30,8 +30,10 @@ typedef struct pcb_diel pcb_diel;   /* dielectric M: bit mask of Omega_1 + eps e
 typedef struct pcb_op pcb_op;       /* one k-point: symbol tables, gamma, shift, (optional) dielectric */
 
 /* dielectric kinds (discretization.py:352 chiral_handle, :368 pseudochiral_trivial_handle,
- * :403 pseudochiral_crossdof_handle; NONE = `Diels = lambda x: x`, numerical_experiments.py:227) */
-enum { PCB_DIEL_KIND_NONE = 0, PCB_DIEL_KIND_CHIRAL = 1, PCB_DIEL_KIND_TRIVIAL = 2, PCB_DIEL_KIND_CROSSDOF = 3 };
+ * :403 pseudochiral_crossdof_handle; NONE = `Diels = lambda x: x`, numerical_experiments.py:227; MATERIALS: several isotropic
+ * materials, one index per edge DoF, created by pcb_diel_create_materials) */
+enum { PCB_DIEL_KIND_NONE = 0, PCB_DIEL_KIND_CHIRAL = 1, PCB_DIEL_KIND_TRIVIAL = 2, PCB_DIEL_KIND_CROSSDOF = 3,
+       PCB_DIEL_KIND_MATERIALS = 4 };
 
 /* pcb_apply modes */
 enum {
@@ -93,6 +95,13 @@ int pcb_fill_uniform(pcb_ctx* ctx, int k, void* const* cols, unsigned long long 
  * stencil: the 2k averaging weights mfd_stencil(k, 0) (crossdof only). */
 int pcb_diel_create(pcb_ctx* ctx, int kind, const int64_t* ind_e, long long n_e, const int64_t* ind_v, long long n_v,
                     const double* ediag, const double* eoff, int k, const double* stencil, pcb_diel** diel);
+/* Several isotropic materials: (M x)_r = inv_eps[mat[r]] x_r.  mat: HOST array of n = 3 N^3 material indices in row order
+ * r = c N^3 + p (index 0: the background, whose inv_eps[0] need not be 1); inv_eps: HOST array of n_mat values 1 / eps, 1 <= n_mat
+ * <= 256.  inv_eps = {1, 1/eps} with mat = 1 on ind_e is the chiral M.  Fails with -1 (nothing allocated) when n != 3 N^3, n_mat is
+ * out of range, some mat[r] >= n_mat or some inv_eps is not finite and > 0; with -2 on a slab context.  A / H run the plane pass
+ * where the plane mode applies (seven sweeps: "mid_five" is ignored) and the five-pass operator elsewhere; pcb_field_energy's
+ * e_in is the energy in the rows with mat[r] != 0. */
+int pcb_diel_create_materials(pcb_ctx* ctx, const uint8_t* mat, long long n, const double* inv_eps, int n_mat, pcb_diel** diel);
 void pcb_diel_destroy(pcb_diel* diel);
 
 /* operator for one k-point (numerical_experiments.py:434-448 pc_mfd_handle).  tables: [3][3][N] complex128,

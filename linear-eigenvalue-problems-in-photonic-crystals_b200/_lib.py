@@ -48,6 +48,7 @@ SIGNATURES = {
     "pcb_fill_uniform": (C.c_int, [C.c_void_p, C.c_int, c_void_pp, C.c_ulonglong]),
     "pcb_diel_create": (C.c_int, [C.c_void_p, C.c_int, c_int64_p, C.c_longlong, c_int64_p, C.c_longlong,
                                   c_double_p, c_double_p, C.c_int, c_double_p, c_void_pp]),
+    "pcb_diel_create_materials": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, c_double_p, C.c_int, c_void_pp]),
     "pcb_diel_destroy": (None, [C.c_void_p]),
     "pcb_op_create": (C.c_int, [C.c_void_p, c_double_p, C.c_double, C.c_double, C.c_double, C.c_void_p, c_void_pp]),
     "pcb_op_update": (C.c_int, [C.c_void_p, c_double_p, C.c_double, C.c_double, C.c_double, C.c_void_p]),
@@ -83,7 +84,7 @@ SIGNATURES = {
 }
 
 APPLY_FFT, APPLY_IFFT, APPLY_A, APPLY_H, APPLY_P, APPLY_M, APPLY_KA, APPLY_KAH, APPLY_KB, APPLY_DFIELD, APPLY_EFIELD, APPLY_EFOURIER = range(12)
-DIEL_NONE, DIEL_CHIRAL, DIEL_TRIVIAL, DIEL_CROSSDOF = range(4)
+DIEL_NONE, DIEL_CHIRAL, DIEL_TRIVIAL, DIEL_CROSSDOF, DIEL_MATERIALS = range(5)
 
 
 class PcbError(RuntimeError):

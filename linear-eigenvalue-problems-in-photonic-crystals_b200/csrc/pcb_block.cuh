@@ -687,6 +687,12 @@ __global__ void __launch_bounds__(256) k_diel_point(PcbOp op, const cplx* __rest
         Y[p] = u[0]; Y[nn + p] = u[1]; Y[2 * nn + p] = u[2];
     }
 }
+// Materials dielectric: Y_r = inv_eps[mat[r]] X_r over the 3 nn rows (in place allowed)
+PCB_D cplx pcb_mat_point(const PcbOp& op, long long r, cplx x) { return cscale(x, __ldg(op.inv_eps + __ldg(op.mat + r))); }
+__global__ void __launch_bounds__(256) k_diel_mat(PcbOp op, const cplx* X, cplx* Y) {
+    for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < 3 * op.nn; r += (long long)gridDim.x * blockDim.x)
+        Y[r] = pcb_mat_point(op, r, X[r]);
+}
 
 // Cross-DoF dielectric (discretization.py:403-453): diagonal + eps_ab * S_ab couplings,
 // S_ab = (I_a T_ab + T_ab I_b)/2,  T_ab = c (x) c^T on two of the three axes (stencil c with 2k taps).
@@ -847,7 +853,7 @@ __global__ void __launch_bounds__(256) k_diel_crossdof_t(PcbOp op, PcbStencil st
 // partial[(blockIdx.x * ncols + j) * 2 + {0: e_in, 1: e_tot}] = this CTA's sums for column j.  The grid-stride loop runs over a
 // grid that does not depend on ncols, and both reduction stages have a fixed order: a column gets the same bits at any width.
 // DIEL: 0 none (e_in = 0, no mask), 1 chiral, 2 trivial (point-wise, pcb_diel_point), 3 cross-DoF (the stencil gather; K as in
-// k_diel_crossdof).
+// k_diel_crossdof), 4 materials (e_in: the rows outside the background, index != 0).
 PCB_D void pcb_energy_block_store(double ein, double etot, double* __restrict__ partial, int ncols) {
     __shared__ double red[8][2];
     ein = pcb_warp_sum(ein);
@@ -860,6 +866,19 @@ PCB_D void pcb_energy_block_store(double ein, double etot, double* __restrict__ 
         for (int w = 0; w < 8; ++w) v += red[w][threadIdx.x];
         partial[((long long)blockIdx.x * ncols + blockIdx.y) * 2 + threadIdx.x] = v;
     }
+}
+// materials: bit c set where row c nn + p is outside the background (index != 0)
+PCB_D unsigned pcb_mat_bits(const PcbOp& op, long long p) {
+    unsigned m = 0u;
+    PCB_UNROLL
+    for (int c = 0; c < 3; ++c) m |= (__ldg(op.mat + c * op.nn + p) != 0 ? 1u : 0u) << c;
+    return m;
+}
+// plane-slot position pt = (i0 N + row) N + col -> natural cell (i2 N + i1) N + i0, i1 = coord(col), i2 = coord_row(row)
+PCB_D long long pcb_slot_to_cell(const PcbOp& op, long long pt) {
+    const int N = op.N;
+    const int col = (int)(pt % N), row = (int)((pt / N) % N), i0 = (int)(pt / ((long long)N * N));
+    return ((long long)__ldg(op.ctab + 2 * N + row) * N + __ldg(op.ctab + col)) * N + i0;
 }
 PCB_D void pcb_energy_point(const cplx d[3], const cplx y[3], unsigned m, double& ein, double& etot) {
     PCB_UNROLL
@@ -878,9 +897,13 @@ __global__ void __launch_bounds__(256) k_field_energy(PcbOp op, PcbStencil st, P
     double ein = 0.0, etot = 0.0;
     for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < nn; p += (long long)gridDim.x * blockDim.x) {
         const cplx d[3] = {X[p], X[nn + p], X[2 * nn + p]};
-        const unsigned m = DIEL ? (unsigned)__ldg(op.mask + p) : 0u;
+        const unsigned m = DIEL == 4 ? pcb_mat_bits(op, p) : DIEL ? (unsigned)__ldg(op.mask + p) : 0u;
         cplx y[3];
         if (DIEL == 3) pcb_crossdof_gather<K>(op, st, X, p, m, d, y);
+        else if (DIEL == 4) {
+            PCB_UNROLL
+            for (int c = 0; c < 3; ++c) y[c] = pcb_mat_point(op, c * nn + p, d[c]);
+        }
         else {
             y[0] = d[0]; y[1] = d[1]; y[2] = d[2];
             if (DIEL) pcb_diel_point(op, DIEL == 1 ? (m & 7u) : m, y);
@@ -899,9 +922,15 @@ __global__ void __launch_bounds__(256) k_field_energy_t(PcbOp op, PcbStencil st,
     double ein = 0.0, etot = 0.0;
     for (long long pt = (long long)blockIdx.x * blockDim.x + threadIdx.x; pt < nn; pt += (long long)gridDim.x * blockDim.x) {
         const cplx d[3] = {X[pt], X[nn + pt], X[2 * nn + pt]};
-        const unsigned m = DIEL ? (unsigned)__ldg(op.maskp + pt) : 0u;
+        // materials: the natural-order position of the slot through the coordinate tables (no slot-ordered copy of the map)
+        const long long p = DIEL == 4 ? pcb_slot_to_cell(op, pt) : 0;
+        const unsigned m = DIEL == 4 ? pcb_mat_bits(op, p) : DIEL ? (unsigned)__ldg(op.maskp + pt) : 0u;
         cplx y[3];
         if (DIEL == 3) pcb_crossdof_gather_t<K>(op, st, X, pt, m, d, y);
+        else if (DIEL == 4) {
+            PCB_UNROLL
+            for (int c = 0; c < 3; ++c) y[c] = pcb_mat_point(op, c * nn + p, d[c]);
+        }
         else {
             y[0] = d[0]; y[1] = d[1]; y[2] = d[2];
             if (DIEL) pcb_diel_point(op, DIEL == 1 ? (m & 7u) : (m & 15u), y);

@@ -117,6 +117,8 @@ struct pcb_diel {
     unsigned char* maskp;   // plane mode, coupled dielectric: byte mask in plane-slot order (k_mask_plane); else null
     unsigned char* maskp_fe; // the same mask for pcb_field_energy where maskp does not exist: built by its first call in the plane layout
     int zsplit;             // the plane-mode form (ctx->zsplit) the slot-ordered masks were built for
+    unsigned char* matp;    // materials, plane mode: the index bytes in the item order of the plane pass (k_mat_bytes); else null
+    double* inv_eps;        // materials: [n_mat] 1 / eps on the device (mask then holds the [3 nn] index bytes); else null
     double ediag[3];
     cplx eoff[3];
     PcbStencil st;
@@ -472,6 +474,7 @@ int pcb_diel_create(pcb_ctx* c, int kind, const int64_t* ind_e, long long n_e, c
     PCB_CUDA_OK(cudaSetDevice(c->device));
     pcb_diel* d = new pcb_diel;
     d->ctx = c; d->kind = kind; d->mask = nullptr; d->mbits = nullptr; d->mbits2 = nullptr; d->maskp = nullptr; d->maskp2 = nullptr; d->maskp_fe = nullptr;
+    d->matp = nullptr; d->inv_eps = nullptr;
     for (int i = 0; i < 3; ++i) { d->ediag[i] = ediag ? ediag[i] : 1.0; d->eoff[i] = eoff ? cmake(eoff[2 * i], eoff[2 * i + 1]) : cmake(0.0, 0.0); }
     d->st.k = 1; for (int i = 0; i < 8; ++i) d->st.w[i] = 0.0;
     if (kind == PCB_DIEL_CROSSDOF) {
@@ -548,6 +551,52 @@ int pcb_diel_create(pcb_ctx* c, int kind, const int64_t* ind_e, long long n_e, c
     *out = d;
     return 0;
 }
+int pcb_diel_create_materials(pcb_ctx* c, const uint8_t* mat, long long n, const double* inv_eps, int n_mat, pcb_diel** out) {
+    PCB_CHECK_ARG(c && mat && inv_eps && out, "null");
+    if (c->nloc != c->nn) {
+        pcb_set_error("pcb_diel_create_materials: needs whole columns; a slab context has no dielectric of this kind");
+        return -2;
+    }
+    // the whole input is checked before anything is allocated
+    if (n != 3 * c->nn) { pcb_set_error("pcb_diel_create_materials: n = %lld, expected 3 N^3 = %lld", n, 3 * c->nn); return -1; }
+    if (n_mat < 1 || n_mat > 256) { pcb_set_error("pcb_diel_create_materials: n_mat = %d, expected 1 ... 256", n_mat); return -1; }
+    for (int i = 0; i < n_mat; ++i)
+        if (!std::isfinite(inv_eps[i]) || !(inv_eps[i] > 0.0)) { pcb_set_error("pcb_diel_create_materials: inv_eps[%d] = %g is not finite and > 0", i, inv_eps[i]); return -1; }
+    unsigned char top = 0;
+    for (long long r = 0; r < n; ++r) top = mat[r] > top ? mat[r] : top;
+    if (top >= n_mat) {
+        long long r = 0;
+        while (mat[r] < n_mat) ++r;
+        pcb_set_error("pcb_diel_create_materials: mat[%lld] = %d >= n_mat = %d", r, (int)mat[r], n_mat);
+        return -1;
+    }
+    PCB_CUDA_OK(cudaSetDevice(c->device));
+    pcb_diel* d = new pcb_diel;
+    d->ctx = c; d->kind = PCB_DIEL_MATERIALS; d->mask = nullptr; d->mbits = nullptr; d->mbits2 = nullptr; d->maskp = nullptr; d->maskp2 = nullptr; d->maskp_fe = nullptr;
+    d->matp = nullptr; d->inv_eps = nullptr; d->zsplit = c->zsplit;
+    for (int i = 0; i < 3; ++i) { d->ediag[i] = 1.0; d->eoff[i] = cmake(0.0, 0.0); }
+    d->st.k = 1; for (int i = 0; i < 8; ++i) d->st.w[i] = 0.0;
+    PCB_CUDA_OK_OR(cudaMalloc(&d->mask, (size_t)n), pcb_diel_destroy(d));
+    PCB_CUDA_OK_OR(cudaMalloc(&d->inv_eps, sizeof(double) * (size_t)n_mat), pcb_diel_destroy(d));
+    PCB_CUDA_OK_OR(cudaMemcpyAsync(d->mask, mat, (size_t)n, cudaMemcpyHostToDevice, c->stream), pcb_diel_destroy(d));
+    PCB_CUDA_OK_OR(cudaMemcpyAsync(d->inv_eps, inv_eps, sizeof(double) * (size_t)n_mat, cudaMemcpyHostToDevice, c->stream), pcb_diel_destroy(d));
+    if (c->plan->plane_mode) {
+        // the index bytes of every z item of the plane pass, padded to pcb_mat_pad(ZR2) bytes (whole or half planes, as mbits)
+        const int zr1 = c->zsplit ? c->plan->zr1 : c->plan->r1, zr2 = c->zsplit ? c->plan->zr2 : c->plan->r2;
+        const size_t bytes = 3 * (size_t)c->N * c->N * (c->zsplit ? 2 : 1) * zr1 * pcb_mat_pad(zr2);
+        PCB_CUDA_OK_OR(cudaMalloc(&d->matp, bytes), pcb_diel_destroy(d));
+        PcbOp tmp;
+        memset(&tmp, 0, sizeof tmp);
+        tmp.N = c->N; tmp.nn = c->nn; tmp.nloc = c->nloc; tmp.mat = d->mask; tmp.matp = d->matp; tmp.zsplit = c->zsplit;
+        PcbCols none;
+        memset(&none, 0, sizeof none);
+        if (c->plan->pass(tmp, none, 1, PCB_PASS_MATBYTES, c->tw, c->stream, c->sms)) { pcb_diel_destroy(d); return -1; }
+        c->launches++;
+    }
+    PCB_CUDA_OK_OR(cudaStreamSynchronize(c->stream), pcb_diel_destroy(d));
+    *out = d;
+    return 0;
+}
 void pcb_diel_destroy(pcb_diel* d) {
     if (!d) return;
     cudaSetDevice(d->ctx->device);
@@ -558,6 +607,8 @@ void pcb_diel_destroy(pcb_diel* d) {
     if (d->mbits2) cudaFree(d->mbits2);
     if (d->maskp2) cudaFree(d->maskp2);
     if (d->maskp_fe) cudaFree(d->maskp_fe);
+    if (d->matp) cudaFree(d->matp);
+    if (d->inv_eps) cudaFree(d->inv_eps);
     delete d;
 }
 
@@ -574,6 +625,7 @@ static void op_fill(pcb_op* o, double gamma, double shift, double pshift, pcb_di
     o->d.maskp = diel ? diel->maskp : nullptr;
     o->d.mbits2 = diel ? diel->mbits2 : nullptr;
     o->d.maskp2 = diel ? diel->maskp2 : nullptr;
+    if (diel && diel->kind == PCB_DIEL_MATERIALS) { o->d.matp = diel->matp; o->d.inv_eps = diel->inv_eps; }
     if (diel) o->d.sten = diel->st; else { o->d.sten.k = 1; for (int i = 0; i < 8; ++i) o->d.sten.w[i] = 0.0; }
     o->d.ctab = c->ctab;
     o->d.zsplit = c->zsplit;
@@ -656,7 +708,7 @@ static int apply_structure(const pcb_op* o) {
     const pcb_ctx* c = o->ctx;
     const int diel = o->d.diel;
     if (plane_layout(c)) {
-        if (diel == PCB_DIEL_NONE || diel == PCB_DIEL_CHIRAL) return PCB_STRUCT_PLANE;
+        if (diel == PCB_DIEL_NONE || diel == PCB_DIEL_CHIRAL || diel == PCB_DIEL_MATERIALS) return PCB_STRUCT_PLANE;
         if (diel == PCB_DIEL_TRIVIAL && c->use_plane_coupled && (c->zsplit ? c->plan->plane_split_coupled : c->plan->plane_coupled)) return PCB_STRUCT_PLANE;
         if (diel == PCB_DIEL_CROSSDOF && c->use_plane_cross) return c->use_plane_cross == 2 ? PCB_STRUCT_CROSS5 : PCB_STRUCT_CROSS4;
     }
@@ -776,6 +828,17 @@ static int apply_AH(pcb_op* o, int mode, const PcbCols& cols, int kc, int j0, in
     return run_steps(o, apply_steps(o, mode, dist), cols, kc);
 }
 
+// Y = M X for one column of a point-wise dielectric (none / chiral / trivial / materials), in place allowed
+static int launch_point_diel(pcb_op* o, const cplx* X, cplx* Y) {
+    pcb_ctx* c = o->ctx;
+    dim3 grid((unsigned)grid_for(c, c->nn, 256, 8), 1, 1);
+    if (o->d.diel == PCB_DIEL_MATERIALS) PCB_LAUNCH(k_diel_mat, grid, dim3(256, 1, 1), 0, c->stream, o->d, X, Y);
+    else PCB_LAUNCH(k_diel_point, grid, dim3(256, 1, 1), 0, c->stream, o->d, X, Y);
+    PCB_CUDA_OK(cudaGetLastError());
+    c->launches++;
+    return 0;
+}
+
 // D = FFT3(K_A^H x) (DFIELD) or E = M D (EFIELD) in the natural layout: the forward half, then for E the point-wise M in place
 // on out, or the cross-DoF stencil from the scratch into out.
 static int apply_field(pcb_op* o, int mode, const PcbCols& cols, int kc) {
@@ -786,12 +849,8 @@ static int apply_field(pcb_op* o, int mode, const PcbCols& cols, int kc) {
     else for (int i = 0; i < p.n; ++i) p.s[i].cols = PCB_COLS_IO;      // D straight into out
     if (run_steps(o, p, cols, kc)) return -1;
     if (mode != PCB_APPLY_EFIELD || o->d.diel == PCB_DIEL_NONE || stencil) return 0;
-    for (int j = 0; j < kc; ++j) {
-        dim3 grid((unsigned)grid_for(c, c->nn, 256, 8), 1, 1);
-        PCB_LAUNCH(k_diel_point, grid, dim3(256, 1, 1), 0, c->stream, o->d, cols.out[j], cols.out[j]);
-        PCB_CUDA_OK(cudaGetLastError());
-        c->launches++;
-    }
+    for (int j = 0; j < kc; ++j)
+        if (launch_point_diel(o, cols.out[j], cols.out[j])) return -1;
     return 0;
 }
 
@@ -833,12 +892,8 @@ int pcb_apply(pcb_op* o, int mode, int ncols, const void* const* in, void* const
             } break;
             case PCB_APPLY_M:
                 if (cross && launch_crossdof(o, kc, cols.in, cols.out)) return -1;      // (in place refused by check_inplace)
-                for (int j = 0; j < kc && !cross; ++j) {
-                    dim3 grid((unsigned)grid_for(c, c->nn, 256, 8), 1, 1);
-                    PCB_LAUNCH(k_diel_point, grid, dim3(256, 1, 1), 0, c->stream, o->d, cols.in[j], cols.out[j]);
-                    PCB_CUDA_OK(cudaGetLastError());
-                    c->launches++;
-                }
+                for (int j = 0; j < kc && !cross; ++j)
+                    if (launch_point_diel(o, cols.in[j], cols.out[j])) return -1;
                 break;
             case PCB_APPLY_DFIELD: case PCB_APPLY_EFIELD:
                 if (int rc = apply_field(o, mode, cols, kc)) return rc;
@@ -921,6 +976,7 @@ static int field_energy_chunk(pcb_op* o, const PcbCols& cols, int kc, bool plane
             case PCB_DIEL_NONE: PCB_LAUNCH((KERN<0, 1>), grid, blk, 0, c->stream, d, st, e, kc, part); break;       \
             case PCB_DIEL_CHIRAL: PCB_LAUNCH((KERN<1, 1>), grid, blk, 0, c->stream, d, st, e, kc, part); break;     \
             case PCB_DIEL_TRIVIAL: PCB_LAUNCH((KERN<2, 1>), grid, blk, 0, c->stream, d, st, e, kc, part); break;    \
+            case PCB_DIEL_MATERIALS: PCB_LAUNCH((KERN<4, 1>), grid, blk, 0, c->stream, d, st, e, kc, part); break;  \
             default:                                                                                                \
                 if (k == 1) PCB_LAUNCH((KERN<3, 1>), grid, blk, 0, c->stream, d, st, e, kc, part);                  \
                 else if (k == 2) PCB_LAUNCH((KERN<3, 2>), grid, blk, 0, c->stream, d, st, e, kc, part);             \
@@ -948,7 +1004,7 @@ int pcb_field_energy(pcb_op* o, int ncols, const void* const* x, double* e_in, d
     PCB_CHECK_ARG(!o->diel || o->diel->zsplit == c->zsplit, "dielectric was created under the other plane-mode form (plane_split); re-create it");
     const bool plane = plane_layout(c);
     const unsigned char* smask = nullptr;
-    if (plane && o->d.diel != PCB_DIEL_NONE && !(smask = energy_slot_mask(o))) return -1;
+    if (plane && o->d.diel != PCB_DIEL_NONE && o->d.diel != PCB_DIEL_MATERIALS && !(smask = energy_slot_mask(o))) return -1;
     const int gx = grid_for(c, c->nn, 256, 4);      // fixed for the context: the same partials for a column at any width
     const int kmax = ncols < PCB_MAXC ? ncols : PCB_MAXC;
     if (ensure_partial(c, sizeof(double) * ((size_t)gx + 1) * 2 * PCB_MAXC)) return -1;

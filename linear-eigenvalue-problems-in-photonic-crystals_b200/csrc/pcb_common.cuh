@@ -98,7 +98,7 @@ void pcb_set_error(const char* fmt, ...);
 //     K_c(i0,i1,i2) = T[c][0][i0] + T[c][1][i1] + T[c][2][i2],
 //     T[c][j][l]    = (CT[c][j]*D1[l] + (j==c) * i*alpha_c*D0[l]) / SCAL
 // replacing the reference's 192*N^3-byte symbol arrays (fft_blocks, discretization.py:301-346).
-enum { PCB_DIEL_NONE = 0, PCB_DIEL_CHIRAL = 1, PCB_DIEL_TRIVIAL = 2, PCB_DIEL_CROSSDOF = 3 };
+enum { PCB_DIEL_NONE = 0, PCB_DIEL_CHIRAL = 1, PCB_DIEL_TRIVIAL = 2, PCB_DIEL_CROSSDOF = 3, PCB_DIEL_MATERIALS = 4 };
 
 // Large-grid mode over peer memory (NVLink): the columns of one distributed apply live as SLABS on all ranks -- rank g holds the
 // i2 planes [zb[g], zb[g+1]) of every column as [c][local cell] -- and the x passes of the operator read / write them in place
@@ -126,9 +126,18 @@ struct PcbOp {
     double pshift;            // shift seen by the preconditioner (= shift / SCAL^2)
     double inv_n3;            // 1 / N^3 (normalisation of the inverse transform)
     int diel;                 // PCB_DIEL_*
-    const unsigned char* mask;  // [nn] bit c: edge DoF of component c in Omega_1; bit 3: volume DoF
-    const unsigned* mbits;      // plane mode: [c][i0][slot][k1] words, bit k2 = component c of (i0, i1 = coord(slot), i2 = lout(k1,k2)) in Omega_1
-    const unsigned* mbits2;     // five-sweep plane pass (k_mid2): [c][i0][d][col] words, bit k2 (k_mask_bits2)
+    union {
+        const unsigned char* mask;  // [nn] bit c: edge DoF of component c in Omega_1; bit 3: volume DoF
+        const unsigned char* mat;   // materials: [3 nn] material index of row r = c nn + p (natural order)
+    };
+    union {
+        const unsigned* mbits;      // plane mode: [c][i0][slot][k1] words, bit k2 = component c of (i0, i1 = coord(slot), i2 = lout(k1,k2)) in Omega_1
+        const unsigned char* matp;  // materials, plane mode: the index bytes of each z item, in the item order of mbits (k_mat_bytes)
+    };
+    union {
+        const unsigned* mbits2;     // five-sweep plane pass (k_mid2): [c][i0][d][col] words, bit k2 (k_mask_bits2)
+        const double* inv_eps;      // materials: [n_mat] 1 / eps of each material (index 0: the background)
+    };
     const unsigned char* maskp2; // the same byte mask in the slot order of the five-sweep plane pass (k_mask_plane2), coupled dielectric
     const unsigned char* maskp; // plane mode, coupled dielectric: the byte mask in plane-slot order, [i0][row][col] = mask(i0, coord(col), coord(row))
     PcbStencil sten;            // cross-DoF dielectric: its averaging stencil (the fused stencil-on-load of the plane pass)

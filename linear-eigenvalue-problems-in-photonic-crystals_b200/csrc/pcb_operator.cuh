@@ -651,9 +651,30 @@ PCB_HD void pcb_diel_point(const PcbOp& op, unsigned m, cplx u[3]) {
     u[0] = y0; u[1] = y1; u[2] = y2;
 }
 
+// Materials dielectric (PCB_DIEL_MATERIALS): M is diagonal, (M x)_r = inv_eps[mat[r]] x_r.  In the plane pass each z item's ZR2
+// index bytes are stored padded to pcb_mat_pad(ZR2) bytes (k_mat_bytes), so that one aligned vector load of ZP / 4 words fetches
+// them; the 2 KB table of 1 / eps is read through __ldg and stays L1-resident (the plane leaves no room for it in shared memory).
+PCB_HD constexpr int pcb_mat_pad(int r2) { return r2 <= 4 ? 4 : (r2 <= 8 ? 8 : 16); }
+template <int W>
+PCB_D void pcb_ldg_words(unsigned* w, const unsigned char* __restrict__ p) {
+#ifdef PCB_EMU
+    memcpy(w, p, 4 * W);
+#else
+    if constexpr (W == 4) { const uint4 u = __ldg(reinterpret_cast<const uint4*>(p)); w[0] = u.x; w[1] = u.y; w[2] = u.z; w[3] = u.w; }
+    else if constexpr (W == 2) { const uint2 u = __ldg(reinterpret_cast<const uint2*>(p)); w[0] = u.x; w[1] = u.y; }
+    else w[0] = __ldg(reinterpret_cast<const unsigned*>(p));
+#endif
+}
+// v[k] *= inv_eps[index byte k of the packed words w]
+template <int R>
+PCB_D void pcb_mat_scale(const PcbOp& op, const unsigned* w, cplx* v) {
+    PCB_UNROLL
+    for (int k = 0; k < R; ++k) v[k] = cscale(v[k], __ldg(op.inv_eps + ((w[k / 4] >> (8 * (k % 4))) & 0xffu)));
+}
+
 // ---------------------------------------------------------------------------------------
 // Pass 3: z-lines: forward FFT, dielectric multiply M in real space, inverse FFT; in place.
-// DIEL: 0 identity, 1 component-wise (chiral), 2 coupled 3x3 at a point (trivial).
+// DIEL: 0 identity, 1 component-wise (chiral), 2 coupled 3x3 at a point (trivial), 4 materials (index bytes gathered per item).
 // Persistent CTAs; tile = 8 consecutive i0 x one i1, all i2, three components (3*N segments of 128 B), streamed into
 // one of two shared-memory stages with cp.async while the previous tile is transformed.  The line element with
 // digits (a, b) always lives in slot P::lin(a, b) of its stage, so all four radix steps exchange in place.
@@ -798,6 +819,19 @@ __global__ void __launch_bounds__(NT, (NT > 256 ? 1 : 2)) k_zmid(PcbOp op, PcbCo
                 if (i0 >= N) continue;
                 const int b1 = P::lin1(k1);
                 cplx* __restrict__ sc = st + c * N * 8 + i0l;
+                // materials: the item's R2 index bytes gathered from the natural-order map and packed four to a word, issued ahead
+                // of the column loads and the radix step (gathered before the barrier as the chiral bits are, the ZI x R2 / 4 words
+                // spill from N = 120 on)
+                constexpr int MW = (DIEL == 4) ? (R2 + 3) / 4 : 1;
+                unsigned mw[MW];
+                if (DIEL == 4) {
+                    PCB_UNROLL
+                    for (int w = 0; w < MW; ++w) mw[w] = 0u;
+                    const unsigned char* __restrict__ mp = op.mat + c * nn + (long long)i1 * N + i0;
+                    const int o1 = P::lout1(k1);      // real-space digits (k1, k2) belong to grid index i2 = lout(k1, k2)
+                    PCB_UNROLL
+                    for (int k2 = 0; k2 < R2; ++k2) mw[k2 / 4] |= (unsigned)__ldg(mp + P::wrap(o1 + P::lout2(k2)) * (N * N)) << (8 * (k2 % 4));
+                }
                 cplx v[R2];
                 PCB_UNROLL
                 for (int n2 = 0; n2 < R2; ++n2) v[n2] = sc[P::wrap(b1 + P::lin2(n2)) * 8];
@@ -808,6 +842,7 @@ __global__ void __launch_bounds__(NT, (NT > 256 ? 1 : 2)) k_zmid(PcbOp op, PcbCo
                     PCB_UNROLL
                     for (int k2 = 0; k2 < R2; ++k2) v[k2] = cscale(v[k2], ((w >> k2) & 1u) ? scl : 1.0);   // branch-free
                 }
+                if (DIEL == 4) pcb_mat_scale<R2>(op, mw, v);
                 Dft<R2, +1>::run(v);
                 PCB_UNROLL
                 for (int n2 = 0; n2 < R2; ++n2) {
@@ -858,6 +893,23 @@ __global__ void k_mask_bits(PcbOp op, unsigned* __restrict__ out) {
     }
     out[t] = w;
 }
+// The same for the materials dielectric: matp[item t of k_mask_bits][k2] = mat[c nn + (i2 N + i1) N + i0], the ZR2 index bytes of
+// the item padded with zeros to pcb_mat_pad(ZR2)
+template <class P, int ZS = 1>
+__global__ void k_mat_bytes(PcbOp op, unsigned char* __restrict__ out) {
+    typedef typename ZSplit<P, ZS>::PZ PZ;
+    constexpr int N = P::N, R1 = PZ::R1, R2 = PZ::R2, ZP = pcb_mat_pad(R2);
+    const long long total = 3LL * N * N * ZS * R1;
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= total) return;
+    const int k1 = (int)(t % R1), h = (int)((t / R1) % ZS), slot = (int)((t / (R1 * ZS)) % N), i0 = (int)((t / ((long long)R1 * ZS * N)) % N),
+              c = (int)(t / ((long long)R1 * ZS * N * N));
+    const int i1 = P::coord(slot), o1 = PZ::lout1(k1);
+    for (int k2 = 0; k2 < ZP; ++k2) {
+        const int i2 = ZS * PZ::wrap(o1 + PZ::lout2(k2 < R2 ? k2 : 0)) + h;
+        out[t * ZP + k2] = k2 < R2 ? op.mat[c * op.nn + ((long long)i2 * N + i1) * N + i0] : (unsigned char)0;
+    }
+}
 
 // ---------------------------------------------------------------------------------------
 // Plane mode, pass 2 of 3: forward y, forward z, M, inverse z, inverse y on one (i1, i2) plane held in shared memory.
@@ -870,7 +922,7 @@ __global__ void k_mask_bits(PcbOp op, unsigned* __restrict__ out) {
 // steps stay conflict-free; N = 120: 232 320 B of the 232 448 B a CTA can have).  Warp w owns rows i2 in [8w, 8w+8) for the
 // y steps and slots i1 in [8w, 8w+8) for the z steps, so only two CTA-wide barriers per plane are needed (row -> column
 // ownership and back); loading, the y steps and storing of different warps overlap each other.  HBM traffic of the whole
-// operator drops from 11 to 7 column transfers per op-apply.  DIEL: 0 identity, 1 component-wise (chiral); the coupled
+// operator drops from 11 to 7 column transfers per op-apply.  DIEL: 0 identity, 1 component-wise (chiral), 4 materials; the coupled
 // 3x3 dielectrics need all three components of a point and stay on the five-pass path.
 // ---------------------------------------------------------------------------------------
 // TMA = 1 (the device build): the rows of a plane are moved by bulk copies -- cp.async.bulk, one elected lane per warp
@@ -1024,7 +1076,7 @@ __global__ void __launch_bounds__(P::N / ZS / 8 * 32, 1) k_mid(PcbOp op, PcbCols
         // word per item (k_mask_bits), fetched now so that its latency hides behind the row loads
         constexpr int ZI = (CW * ZR1 + 31) / 32;
         unsigned mbits[ZI];
-        if (DIEL >= 1) {
+        if (DIEL == 1 || DIEL == 2) {
             PCB_UNROLL
             for (int q = 0; q < ZI; ++q) {
                 const int it = lane + 32 * q;
@@ -1155,6 +1207,12 @@ __global__ void __launch_bounds__(P::N / ZS / 8 * 32, 1) k_mid(PcbOp op, PcbCols
                 if (it >= CW * ZR1) break;
                 cplx* __restrict__ cp = mycols + it % CW;
                 const int k1 = it / CW, b1 = PZ::lin1(k1);
+                // materials: the item's index bytes (k_mat_bytes, same item order as mbits), one vector load issued ahead of the
+                // column loads and the radix step.  (Fetched with the row loads as mbits is, the ZI x 4 words stay live through
+                // the y steps: 68 bytes of spills at N = 120.)
+                constexpr int MW = (DIEL == 4) ? pcb_mat_pad(ZR2) / 4 : 1;
+                unsigned mw[MW];
+                if (DIEL == 4) pcb_ldg_words<MW>(mw, op.matp + (((((long long)c * N + i0) * N + CW * warp + it % CW) * ZS + hz) * ZR1 + k1) * (4 * MW));
                 cplx v[ZR2];
                 PCB_UNROLL
                 for (int n2 = 0; n2 < ZR2; ++n2) v[n2] = cp[PZ::wrap(b1 + PZ::lin2(n2)) * LD];
@@ -1165,6 +1223,7 @@ __global__ void __launch_bounds__(P::N / ZS / 8 * 32, 1) k_mid(PcbOp op, PcbCols
                     PCB_UNROLL
                     for (int k2 = 0; k2 < ZR2; ++k2) v[k2] = cscale(v[k2], ((w >> k2) & 1u) ? scl : 1.0);   // branch-free: no divergence
                 }
+                if (DIEL == 4) pcb_mat_scale<ZR2>(op, mw, v);
                 Dft<ZR2, +1>::run(v);
                 PCB_UNROLL
                 for (int n2 = 0; n2 < ZR2; ++n2) {
@@ -1731,6 +1790,7 @@ enum { PCB_PASS_XFWD_SYM = 0, PCB_PASS_XFWD = 1, PCB_PASS_YFWD = 2, PCB_PASS_ZFW
        // cross-DoF dielectric with the stencil fused into the inverse half of the plane pass (four kernels)
        PCB_PASS_MID_FWD_O = 26 /* forward half, planes -> cols.out */, PCB_PASS_MID_INV_ST = 27 /* stencil on load + inverse half, cols.out -> cols.wrk */,
        PCB_PASS_MASKACTIVE = 28 /* set-up: bits 4-6 of op.maskp */, PCB_PASS_MASKPLANE2 = 29 /* set-up: op.mask -> (unsigned char*)op.maskp2 */,
-       PCB_PASS_XINV_T = 30 /* plane mode: plain inverse x pass (1/N^3, no symbol) from the transposed work column */ };
+       PCB_PASS_XINV_T = 30 /* plane mode: plain inverse x pass (1/N^3, no symbol) from the transposed work column */,
+       PCB_PASS_MATBYTES = 31 /* set-up: op.mat -> (unsigned char*)op.matp (materials dielectric) */ };
 
 const PcbOpLaunch* pcb_find_plan(int N);

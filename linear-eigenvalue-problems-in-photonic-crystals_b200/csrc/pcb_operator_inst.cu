@@ -226,6 +226,12 @@ struct PlanePass<true, PP, ZS> {
             PCB_CUDA_OK(cudaGetLastError());
             return 0;
         }
+        if (pass_id == PCB_PASS_MATBYTES) {
+            const long long total = 3LL * PP::N * PP::N * ZS * ZSplit<PP, ZS>::PZ::R1;
+            PCB_LAUNCH((k_mat_bytes<PP, ZS>), dim3((unsigned)((total + 255) / 256), 1, 1), dim3(256, 1, 1), 0, s, op, const_cast<unsigned char*>(op.matp));
+            PCB_CUDA_OK(cudaGetLastError());
+            return 0;
+        }
         if (pass_id == PCB_PASS_MASKPLANE) {
             const long long total = (long long)PP::N * PP::N * PP::N;
             PCB_LAUNCH((k_mask_plane<PP, ZS>), dim3((unsigned)((total + 255) / 256), 1, 1), dim3(256, 1, 1), 0, s, op, const_cast<unsigned char*>(op.maskp));
@@ -267,6 +273,7 @@ struct PlanePass<true, PP, ZS> {
             else if (pass_id == PCB_PASS_XINV_T) PCB_GO((k_xinv<PP, LX, NT, 0, 1, 0, ZS>), GX, kStageXT);
             else if (pass_id == PCB_PASS_MID && op.diel == PCB_DIEL_NONE) PCB_GO_MID(0, 0, 0);
             else if (pass_id == PCB_PASS_MID && op.diel == PCB_DIEL_CHIRAL) PCB_GO_MID(1, 0, 0);
+            else if (pass_id == PCB_PASS_MID && op.diel == PCB_DIEL_MATERIALS) PCB_GO_MID(4, 0, 0);
             else { pcb_set_error("z-split plane mode: pass %d / dielectric type %d not supported", pass_id, op.diel); return -1; }
             return 0;
         }
@@ -285,6 +292,7 @@ struct PlanePass<true, PP, ZS> {
             if (op.diel == PCB_DIEL_NONE) PCB_GO_MID(0, 0, 0);
             else PCB_GO_MID(1, 0, 0);
         }
+        else if (op.diel == PCB_DIEL_MATERIALS) PCB_GO_MID(4, 0, 0);      // seven sweeps: k_mid2 has no materials form
         else { pcb_set_error("plane mode: dielectric type %d not supported", op.diel); return -1; }
         return 0;
 #undef PCB_GO_MID
@@ -309,12 +317,13 @@ int run_pass(const PcbOp& op, const PcbCols& cols, int ncols, int pass_id, const
             if (op.diel == PCB_DIEL_NONE) PCB_GO_P((k_zmid<P, 0, NTP, NSTZ>), NTP, GL, kSmemZU, 3);
             else if (op.diel == PCB_DIEL_CHIRAL) PCB_GO_P((k_zmid<P, 1, NTP, NSTZ>), NTP, GL, kSmemZU, 3);
             else if (op.diel == PCB_DIEL_TRIVIAL) PCB_GO_P((k_zmid<P, 2, NTP, NSTZ>), NTP, GL, kSmemZU, 2);
+            else if (op.diel == PCB_DIEL_MATERIALS) PCB_GO_P((k_zmid<P, 4, NTP, NSTZ>), NTP, GL, kSmemZU, 3);
             else { pcb_set_error("zmid: dielectric type %d has no fused z pass", op.diel); return -1; }
             break;
         case PCB_PASS_XFWD_SYM_T: case PCB_PASS_MID: case PCB_PASS_XINV_A_T: case PCB_PASS_XINV_H_T: case PCB_PASS_MASKBITS:
         case PCB_PASS_MID_FWD: case PCB_PASS_MID_INV: case PCB_PASS_MASKPLANE: case PCB_PASS_COORDTAB: case PCB_PASS_MASKBITS2:
         case PCB_PASS_XFWD_SYM_TD: case PCB_PASS_XINV_A_TD: case PCB_PASS_XINV_H_TD: case PCB_PASS_MID_FWD_O: case PCB_PASS_MID_INV_ST: case PCB_PASS_MASKPLANE2:
-        case PCB_PASS_XINV_T:
+        case PCB_PASS_XINV_T: case PCB_PASS_MATBYTES:
             if (op.zsplit) return PlanePass<kPlaneSplit, P, 2>::go(op, cols, ncols, pass_id, tw, s, sms);
             return PlanePass<kPlane, P, 1>::go(op, cols, ncols, pass_id, tw, s, sms);
         default: pcb_set_error("unknown pass id %d", pass_id); return -1;

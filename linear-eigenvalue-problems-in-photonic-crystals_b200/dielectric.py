@@ -245,6 +245,16 @@ def device_index_sets(N, d_flag, ctx=None):
     return ind_e, ind_v
 
 
+def material_regions(N, d_flag):
+    """Edge-DoF index sets of the materials of a lattice (discretization.materials_handle): for bcc_dg its two gyroid networks,
+    g > 1.1 (= bcc_sg) and g < -1.1 -- the inversion r -> -r swaps them --, for every other lattice the one set Omega_1."""
+    ind = diel_io_index(N, d_flag, dofs="edge")
+    if d_flag != "bcc_dg":
+        return [ind]
+    sg = diel_io_index(N, "bcc_sg", dofs="edge")
+    return [sg, np.setdiff1d(ind, sg, assume_unique=True)]
+
+
 def diel_io_index(N, d_flag, dofs="edge", gpu=True, cache=True):
     """Indices of the dielectric edge / volume DoFs (dielectric.py:58-97).
 

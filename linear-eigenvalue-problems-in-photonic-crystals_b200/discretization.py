@@ -283,6 +283,31 @@ class DielHandle:
         self._fin = weakref.finalize(self, lib.pcb_diel_destroy, h)
         self._ident_op = None
 
+    @classmethod
+    def materials(cls, n, mat, inv_eps, device=None):
+        """Several isotropic materials (pcb_diel_create_materials): (M x)_r = inv_eps[mat[r]] x_r, with `mat` the material index
+        of each of the 3 n^3 edge DoFs (row order r = c n^3 + p; index 0 is the background) and `inv_eps` one 1 / eps per
+        material (at most 256)."""
+        mat = np.asarray(mat)
+        if mat.dtype != np.uint8 and mat.size and (mat.min() < 0 or mat.max() > 255):
+            raise ValueError("material indices must lie in 0 ... 255")
+        self = cls.__new__(cls)
+        self.n, self.kind = int(n), L.DIEL_MATERIALS
+        self.ctx = devarray.get_context(n, device)
+        self.mat = np.ascontiguousarray(mat, dtype=np.uint8)
+        self.inv_eps = np.ascontiguousarray(inv_eps, dtype=np.float64).ravel()
+        import ctypes as C
+        h = C.c_void_p()
+        lib = L.lib()
+        L.check(lib.pcb_diel_create_materials(self.ctx.h, self.mat.ctypes.data, self.mat.size,
+                                              self.inv_eps.ctypes.data_as(L.c_double_p), len(self.inv_eps), C.byref(h)),
+                "pcb_diel_create_materials")
+        self.h = h
+        import weakref
+        self._fin = weakref.finalize(self, lib.pcb_diel_destroy, h)
+        self._ident_op = None
+        return self
+
     def __call__(self, x):
         from . import pcfft
         return pcfft.diel_apply(self, x)
@@ -294,6 +319,27 @@ def chiral_handle(n, d_flag, eps_opt=0, k=None, device=None):
     eps1 = diel.diel_chiral_const(d_flag) if (eps_opt is None or eps_opt == 0) else eps_opt
     inv = 1.0 / eps1
     return DielHandle(n, L.DIEL_CHIRAL, ind_e, None, [inv, inv, inv], [0, 0, 0], device=device)
+
+
+def materials_handle(n, d_flag, eps_opt=None, regions=None, background=1.0, device=None):
+    """Several isotropic materials: the edge DoFs of regions[i] (index arrays into the 3 n^3 rows; later regions override earlier
+    ones where they overlap) are divided by eps_opt[i], every other row by `background`.  Defaults: the regions of
+    dielectric.material_regions (bcc_dg: its two gyroid networks; every other lattice: Omega_1) and the lattice's chiral eps for
+    each of them -- the same M as chiral_handle(n, d_flag)."""
+    regions = diel.material_regions(n, d_flag) if regions is None else list(regions)
+    if len(regions) > 255:
+        raise ValueError(f"{len(regions)} regions: at most 255 besides the background")
+    if eps_opt is None or (np.isscalar(eps_opt) and eps_opt == 0):
+        eps = np.full(len(regions), float(diel.diel_chiral_const(d_flag)))
+    else:
+        eps = np.atleast_1d(np.asarray(eps_opt, dtype=np.float64))
+        if eps.ndim != 1 or eps.size != len(regions):
+            raise ValueError(f"eps_opt has {eps.size} values for {len(regions)} regions")
+    mat = np.zeros(3 * n ** 3, dtype=np.uint8)
+    for i, reg in enumerate(regions):
+        mat[np.asarray(reg, dtype=np.int64)] = i + 1
+    inv_eps = np.concatenate(([1.0 / background], 1.0 / eps))
+    return DielHandle.materials(n, mat, inv_eps, device=device)
 
 
 def _eps_loc(d_flag, eps_opt, eps_mat):

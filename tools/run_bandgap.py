@@ -1,10 +1,12 @@
 """Full band-structure runs (BASELINE configs 2-4): [torchrun ...] tools/run_bandgap.py N d_flag type [nev] [max_k] [--energy] [--velocity]
+    [--eps e1,e2,...]
 
 Single process: numerical_experiments.bandgap over the whole k-path on one GPU.  Under torch.distributed.run: bandgap_sharded,
 one contiguous k-chunk per GPU, rank 0 merges the rows into the reference-format JSON (output/<type>/bandgap_<d_flag>.json
 under --out).  Prints one JSON line with the wall time, per-k seconds and iteration statistics.  --energy also records, per k-point,
 the fraction of each band's electric energy inside the dielectric ("<d_flag>_<N>_energy_fraction" in the JSON); --velocity the group
-velocity of each band along the path ("<d_flag>_<N>_group_velocity", null for the zero modes at Gamma)."""
+velocity of each band along the path ("<d_flag>_<N>_group_velocity", null for the zero modes at Gamma).  --eps sets eps_opt: one
+permittivity per region for type materials (bcc_dg: its two gyroid networks, e.g. --eps 16,12), else one value."""
 import importlib
 import json
 import os
@@ -20,8 +22,15 @@ os.environ.setdefault("PCB200_QUIET", "1")
 def main():
     energy = "--energy" in sys.argv[1:]
     velocity = "--velocity" in sys.argv[1:]
-    argv = [sys.argv[0]] + [a for a in sys.argv[1:] if a not in ("--energy", "--velocity")]
+    args = sys.argv[1:]
+    eps = None
+    if "--eps" in args:
+        i = args.index("--eps")
+        eps = [float(v) for v in args[i + 1].split(",")]
+        del args[i:i + 2]
+    argv = [sys.argv[0]] + [a for a in args if a not in ("--energy", "--velocity")]
     N, d_flag, typ = int(argv[1]), argv[2], argv[3]
+    eps_opt = 0 if eps is None else (eps if typ == "materials" else eps[0])
     nev = int(argv[4]) if len(argv) > 4 else 10
     max_k = int(argv[5]) if len(argv) > 5 else 0
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -48,8 +57,8 @@ def main():
     if world > 1:
         td.barrier()
     t0 = time.time()
-    rows = ne.bandgap_sharded(N, d_flag, rank, world, type=typ, nev=nev, seed=1000, out_dir=out_dir, indices=indices,
-                              gather=gather if world > 1 else (lambda o: [o]), energy=energy,
+    rows = ne.bandgap_sharded(N, d_flag, rank, world, type=typ, eps_opt=eps_opt, nev=nev, seed=1000, out_dir=out_dir,
+                              indices=indices, gather=gather if world > 1 else (lambda o: [o]), energy=energy,
                               velocity=velocity)
     wall = time.time() - t0
     if world > 1:
