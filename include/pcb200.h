@@ -102,6 +102,12 @@ int pcb_diel_create(pcb_ctx* ctx, int kind, const int64_t* ind_e, long long n_e,
  * where the plane mode applies (seven sweeps: "mid_five" is ignored) and the five-pass operator elsewhere; pcb_field_energy's
  * e_in is the energy in the rows with mat[r] != 0. */
 int pcb_diel_create_materials(pcb_ctx* ctx, const uint8_t* mat, long long n, const double* inv_eps, int n_mat, pcb_diel** diel);
+/* Replace the 1 / eps table of a materials dielectric in place (dispersive materials: eps at a new frequency).  inv_eps: HOST array
+ * of n_mat values.  One copy on the context's stream into the table's own allocation, behind the work already queued: every
+ * operator built on diel sees the new values from its next launch; the index map and the plane-pass index bytes are not rebuilt.
+ * The call waits for the copy, so inv_eps may be reused on return.  Fails with -1, the old table in force, when diel is not of
+ * kind MATERIALS, n_mat differs from the n_mat it was created with, or some value is not finite and > 0. */
+int pcb_diel_set_inv_eps(pcb_diel* diel, const double* inv_eps, int n_mat);
 void pcb_diel_destroy(pcb_diel* diel);
 
 /* operator for one k-point (numerical_experiments.py:434-448 pc_mfd_handle).  tables: [3][3][N] complex128,
@@ -146,6 +152,16 @@ int pcb_apply_timed(pcb_op* op, int mode, int ncols, const void* const* in, void
  * column gives the same bits at any width and on every call.  Runs the forward passes of A (the plane layout where A runs in plane
  * mode, else the natural layout) into the context's scratch and a reduction kernel over them.  A slab context fails with -2. */
 int pcb_field_energy(pcb_op* op, int ncols, const void* const* x, double* e_in, double* e_tot);
+
+/* Electric energy of modes per material (materials dielectric).  With D and E = M D as for pcb_field_energy,
+ *     e_mat[j][m] = Re sum_{r: mat[r] = m} conj(D_r) E_r / N^3,   m < n_mat,
+ * e_mat a HOST array [ncols][n_mat].  sum_m e_mat[j][m] = e_tot and sum_{m != 0} e_mat[j][m] = e_in of pcb_field_energy (to
+ * rounding); since E_r = D_r / eps_m, dlambda/deps_m = -e_m / (eps_m x^H x) (Hellmann-Feynman).  Any ncols, in launches of 32
+ * columns; x is read only.  Runs the forward passes of A into the scratch as pcb_field_energy does, then a kernel that bins the
+ * rows by material without timing-dependent atomics over a grid fixed by the context, and a fixed-order sum: a column's row of
+ * e_mat has the same bits at any width and on every call.  Fails with -1 when op has no dielectric or one of another kind, or
+ * n_mat differs from the dielectric's; with -2 on a slab context.  Nothing is written to e_mat in a refusal. */
+int pcb_material_energy(pcb_op* op, int ncols, const void* const* x, int n_mat, double* e_mat);
 
 /* Band velocity matrices (Hellmann-Feynman).  The symbols depend on the k-point alpha only through the Bloch term of the diagonal
  * tables, dK_c/dalpha_d = delta_cd tau_d[i_d]; dtables = tau as a HOST array [3][N] complex128 (FourierSymbols.dtables).  With

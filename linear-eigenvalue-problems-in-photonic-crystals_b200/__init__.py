@@ -11,7 +11,7 @@ and, to run scripts written against the reference's flat modules unchanged, ``pc
 """
 import sys as _sys
 
-from . import _lib, devarray, environment, dielectric, discretization, pcfft, orthogonalization, lobpcg, numerical_experiments, sharded  # noqa: F401,E501
+from . import _lib, devarray, environment, dielectric, discretization, dispersion, pcfft, orthogonalization, lobpcg, numerical_experiments, sharded  # noqa: F401,E501
 from .devarray import Context, DeviceBlock, get_context, pinned_empty, set_device  # noqa: F401
 from ._lib import PcbError, backend  # noqa: F401
 

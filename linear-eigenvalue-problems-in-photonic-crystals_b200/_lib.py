@@ -49,6 +49,7 @@ SIGNATURES = {
     "pcb_diel_create": (C.c_int, [C.c_void_p, C.c_int, c_int64_p, C.c_longlong, c_int64_p, C.c_longlong,
                                   c_double_p, c_double_p, C.c_int, c_double_p, c_void_pp]),
     "pcb_diel_create_materials": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, c_double_p, C.c_int, c_void_pp]),
+    "pcb_diel_set_inv_eps": (C.c_int, [C.c_void_p, c_double_p, C.c_int]),
     "pcb_diel_destroy": (None, [C.c_void_p]),
     "pcb_op_create": (C.c_int, [C.c_void_p, c_double_p, C.c_double, C.c_double, C.c_double, C.c_void_p, c_void_pp]),
     "pcb_op_update": (C.c_int, [C.c_void_p, c_double_p, C.c_double, C.c_double, C.c_double, C.c_void_p]),
@@ -65,6 +66,7 @@ SIGNATURES = {
     "pcb_update_resid_wait": (C.c_int, [C.c_void_p, C.c_int, c_double_p]),
     "pcb_block_launch_info": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]),
     "pcb_field_energy": (C.c_int, [C.c_void_p, C.c_int, c_void_pp, c_double_p, c_double_p]),
+    "pcb_material_energy": (C.c_int, [C.c_void_p, C.c_int, c_void_pp, C.c_int, c_double_p]),
     "pcb_band_velocity": (C.c_int, [C.c_void_p, C.c_int, c_void_pp, c_double_p, C.c_void_p, c_double_p, c_double_p]),
     "pcb_ctx_trim": (C.c_longlong, [C.c_void_p]),
     "pcb_coldots": (C.c_int, [C.c_void_p, C.c_int, c_void_pp, c_void_pp, C.c_void_p]),

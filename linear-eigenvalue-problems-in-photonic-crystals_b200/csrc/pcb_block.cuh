@@ -940,6 +940,106 @@ __global__ void __launch_bounds__(256) k_field_energy_t(PcbOp op, PcbStencil st,
     pcb_energy_block_store(ein, etot, partial, ncols);
 }
 
+// ---- electric energy per material (pcb_material_energy) ------------------------------------------------------------------
+// Materials dielectric only.  Input: D = FFT3(K_A^H x) in real space, one column per blockIdx.y.  Row r = c nn + p adds
+// Re conj(D_r) E_r, E_r = inv_eps[mat[r]] D_r (pcb_mat_point), to the bin of its material mat[r].
+// partial[(blockIdx.x * ncols + j) * n_mat + m] = this CTA's sum for material m of column j.  No atomics.
+//   S > 0 (n_mat <= S): each thread keeps S bins in registers (one select and add per bin and row), summed by the butterfly of
+//     pcb_warp_sum once at the end: no vote and no warp barrier per row.
+//   S = 0 (any n_mat <= 256): per row component, the lanes of a warp that hold the same material form one group (match_any); a
+//     whole-warp group is summed by the butterfly, any other group by its lowest lane in lane order, into the warp's own bins.  On a
+//     map that changes material from lane to lane every row then pays a vote, two warp barriers and a serial leader sum.
+// Either way the eight warps' bins are added in warp order, and the grid does not depend on ncols: a column gets the same bits at any
+// width.  (A given n_mat always takes the same path.)
+#define PCB_ME_MAX 256      // materials of one dielectric (pcb_diel_create_materials)
+PCB_D unsigned pcb_match_any(unsigned key) {
+#ifdef PCB_EMU
+    unsigned g = 0u;
+    for (int l = 0; l < 32; ++l) g |= (__shfl_sync(0xffffffffu, key, l) == key ? 1u : 0u) << l;
+    return g;
+#else
+    return __match_any_sync(0xffffffffu, key);
+#endif
+}
+// t of every lane into bins[key]; key = PCB_ME_MAX: a lane past the end (nothing added).  All 32 lanes call it.
+PCB_D void pcb_bin_add(double* bins, double* tv, unsigned key, double t, int lane) {
+    const unsigned g = pcb_match_any(key);
+    if (g == 0xffffffffu) {                        // one material across the warp (the usual case: maps are smooth along i0)
+        const double s = pcb_warp_sum(t);
+        if (lane == 0 && key < PCB_ME_MAX) bins[key] += s;
+        return;
+    }
+    tv[lane] = t;
+    __syncwarp();
+    if (key < PCB_ME_MAX && __ffs((int)g) - 1 == lane) {
+        double s = 0.0;
+        for (unsigned q = g; q; q &= q - 1u) s += tv[__ffs((int)q) - 1];
+        bins[key] += s;
+    }
+    __syncwarp();
+}
+#define PCB_ME_REG 16       // materials whose bins a thread keeps in registers (k_material_energy[_t]<PCB_ME_REG>)
+// T = 0: natural layout [c][i2][i1][i0]; T = 1: plane-slot layout W'[c][i0][row][col], the cell found through pcb_slot_to_cell
+template <int T, int S>
+PCB_D void pcb_material_energy_body(const PcbOp& op, const cplx* __restrict__ X, int ncols, int n_mat, double* __restrict__ partial) {
+    __shared__ double bins[8][S ? S : PCB_ME_MAX];
+    __shared__ double tv[8][S ? 1 : 32];
+    const long long nn = op.nn;
+    const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
+    double acc[S ? S : 1];
+    PCB_UNROLL
+    for (int k = 0; k < (S ? S : 1); ++k) acc[k] = 0.0;
+    if (!S) {
+        for (int i = threadIdx.x; i < 8 * n_mat; i += blockDim.x) bins[i / n_mat][i % n_mat] = 0.0;
+        __syncthreads();
+    }
+    // warp-uniform trip count: the lanes past nn take part in the votes with key PCB_ME_MAX
+    for (long long p0 = (long long)blockIdx.x * blockDim.x + 32 * warp; p0 < nn; p0 += (long long)gridDim.x * blockDim.x) {
+        const long long pt = p0 + lane;
+        const bool in = pt < nn;
+        const long long p = !in ? 0 : T ? pcb_slot_to_cell(op, pt) : pt;
+        cplx d[3];
+        unsigned m[3];
+        PCB_UNROLL
+        for (int c = 0; c < 3; ++c) {
+            d[c] = in ? X[c * nn + pt] : cmake(0.0, 0.0);
+            m[c] = in ? (unsigned)__ldg(op.mat + c * nn + p) : (unsigned)PCB_ME_MAX;
+        }
+        PCB_UNROLL
+        for (int c = 0; c < 3; ++c) {
+            const cplx y = in ? cscale(d[c], __ldg(op.inv_eps + m[c])) : cmake(0.0, 0.0);
+            const double t = fma(d[c].x, y.x, d[c].y * y.y);
+            if (S) {
+                PCB_UNROLL
+                for (int k = 0; k < (S ? S : 1); ++k) acc[k] += m[c] == (unsigned)k ? t : 0.0;      // a select: acc stays in registers
+            } else {
+                pcb_bin_add(bins[warp], tv[warp], m[c], t, lane);
+            }
+        }
+    }
+    if (S) {
+        PCB_UNROLL
+        for (int k = 0; k < (S ? S : 1); ++k) {
+            const double v = pcb_warp_sum(acc[k]);
+            if (lane == 0) bins[warp][k] = v;
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < n_mat; i += blockDim.x) {
+        double v = 0.0;
+        for (int w = 0; w < 8; ++w) v += bins[w][i];
+        partial[((long long)blockIdx.x * ncols + blockIdx.y) * n_mat + i] = v;
+    }
+}
+template <int S>
+__global__ void __launch_bounds__(256) k_material_energy(PcbOp op, PcbCols cols, int ncols, int n_mat, double* __restrict__ partial) {
+    pcb_material_energy_body<0, S>(op, cols.in[blockIdx.y], ncols, n_mat, partial);
+}
+template <int S>
+__global__ void __launch_bounds__(256) k_material_energy_t(PcbOp op, PcbCols cols, int ncols, int n_mat, double* __restrict__ partial) {
+    pcb_material_energy_body<1, S>(op, cols.in[blockIdx.y], ncols, n_mat, partial);
+}
+
 // ---- band velocity matrices (pcb_band_velocity) ---------------------------------------------------------------------------
 // Input: X (cols.in) and E^ = IFFT3(M FFT3(K_A^H x)) (cols.out), natural layout; tau = dK_d/dalpha_d, [3][N] complex (device).
 // For d, a, b cyclic:  W_d[i][j] = sum_q conj(x_i,b) F_j,d,a - conj(x_i,a) F_j,d,b  with  F_j,d,c = tau_d[q_d] E^_j,c

@@ -119,6 +119,7 @@ struct pcb_diel {
     int zsplit;             // the plane-mode form (ctx->zsplit) the slot-ordered masks were built for
     unsigned char* matp;    // materials, plane mode: the index bytes in the item order of the plane pass (k_mat_bytes); else null
     double* inv_eps;        // materials: [n_mat] 1 / eps on the device (mask then holds the [3 nn] index bytes); else null
+    int n_mat;              // materials: entries of inv_eps; else 0
     double ediag[3];
     cplx eoff[3];
     PcbStencil st;
@@ -474,7 +475,7 @@ int pcb_diel_create(pcb_ctx* c, int kind, const int64_t* ind_e, long long n_e, c
     PCB_CUDA_OK(cudaSetDevice(c->device));
     pcb_diel* d = new pcb_diel;
     d->ctx = c; d->kind = kind; d->mask = nullptr; d->mbits = nullptr; d->mbits2 = nullptr; d->maskp = nullptr; d->maskp2 = nullptr; d->maskp_fe = nullptr;
-    d->matp = nullptr; d->inv_eps = nullptr;
+    d->matp = nullptr; d->inv_eps = nullptr; d->n_mat = 0;
     for (int i = 0; i < 3; ++i) { d->ediag[i] = ediag ? ediag[i] : 1.0; d->eoff[i] = eoff ? cmake(eoff[2 * i], eoff[2 * i + 1]) : cmake(0.0, 0.0); }
     d->st.k = 1; for (int i = 0; i < 8; ++i) d->st.w[i] = 0.0;
     if (kind == PCB_DIEL_CROSSDOF) {
@@ -573,7 +574,7 @@ int pcb_diel_create_materials(pcb_ctx* c, const uint8_t* mat, long long n, const
     PCB_CUDA_OK(cudaSetDevice(c->device));
     pcb_diel* d = new pcb_diel;
     d->ctx = c; d->kind = PCB_DIEL_MATERIALS; d->mask = nullptr; d->mbits = nullptr; d->mbits2 = nullptr; d->maskp = nullptr; d->maskp2 = nullptr; d->maskp_fe = nullptr;
-    d->matp = nullptr; d->inv_eps = nullptr; d->zsplit = c->zsplit;
+    d->matp = nullptr; d->inv_eps = nullptr; d->n_mat = n_mat; d->zsplit = c->zsplit;
     for (int i = 0; i < 3; ++i) { d->ediag[i] = 1.0; d->eoff[i] = cmake(0.0, 0.0); }
     d->st.k = 1; for (int i = 0; i < 8; ++i) d->st.w[i] = 0.0;
     PCB_CUDA_OK_OR(cudaMalloc(&d->mask, (size_t)n), pcb_diel_destroy(d));
@@ -595,6 +596,20 @@ int pcb_diel_create_materials(pcb_ctx* c, const uint8_t* mat, long long n, const
     }
     PCB_CUDA_OK_OR(cudaStreamSynchronize(c->stream), pcb_diel_destroy(d));
     *out = d;
+    return 0;
+}
+// A new 1 / eps table in the same allocation: the operators built on d read it from their next launch.  Stream-ordered behind the
+// work already queued, and synchronous, so that the host array may be reused on return.
+int pcb_diel_set_inv_eps(pcb_diel* d, const double* inv_eps, int n_mat) {
+    PCB_CHECK_ARG(d && inv_eps, "null");
+    if (d->kind != PCB_DIEL_MATERIALS) { pcb_set_error("pcb_diel_set_inv_eps: dielectric kind %d is not PCB_DIEL_KIND_MATERIALS", d->kind); return -1; }
+    if (n_mat != d->n_mat) { pcb_set_error("pcb_diel_set_inv_eps: n_mat = %d, the dielectric has %d materials", n_mat, d->n_mat); return -1; }
+    for (int i = 0; i < n_mat; ++i)
+        if (!std::isfinite(inv_eps[i]) || !(inv_eps[i] > 0.0)) { pcb_set_error("pcb_diel_set_inv_eps: inv_eps[%d] = %g is not finite and > 0", i, inv_eps[i]); return -1; }
+    pcb_ctx* c = d->ctx;
+    PCB_CUDA_OK(cudaSetDevice(c->device));
+    PCB_CUDA_OK(cudaMemcpyAsync(d->inv_eps, inv_eps, sizeof(double) * (size_t)n_mat, cudaMemcpyHostToDevice, c->stream));
+    PCB_CUDA_OK(cudaStreamSynchronize(c->stream));
     return 0;
 }
 void pcb_diel_destroy(pcb_diel* d) {
@@ -1021,6 +1036,57 @@ int pcb_field_energy(pcb_op* o, int ncols, const void* const* x, double* e_in, d
         PCB_CUDA_OK(cudaStreamSynchronize(c->stream));
         const double* h = (const double*)c->hstage;
         for (int j = 0; j < kc; ++j) { e_in[j0 + j] = h[2 * j] / (double)c->nn; e_tot[j0 + j] = h[2 * j + 1] / (double)c->nn; }
+    }
+    return 0;
+}
+
+// e_m per material of a materials dielectric: the forward passes of pcb_field_energy's layout into the scratch, k_material_energy[_t]
+// over the same fixed grid, the fixed-order sum of the [CTA][column][n_mat] partials.  Every check comes before any output.
+int pcb_material_energy(pcb_op* o, int ncols, const void* const* x, int n_mat, double* e_mat) {
+    PCB_CHECK_ARG(o && x && e_mat && ncols > 0, "bad arguments");
+    pcb_ctx* c = o->ctx;
+    PCB_CUDA_OK(cudaSetDevice(c->device));
+    if (c->nloc != c->nn) {
+        pcb_set_error("pcb_material_energy: needs whole columns; a slab context only supports PCB_APPLY_P (gather with pcb_slab_exchange)");
+        return -2;
+    }
+    if (!o->diel || o->d.diel != PCB_DIEL_MATERIALS) {
+        pcb_set_error("pcb_material_energy: the operator has no materials dielectric (PCB_DIEL_KIND_MATERIALS)");
+        return -1;
+    }
+    if (n_mat != o->diel->n_mat) { pcb_set_error("pcb_material_energy: n_mat = %d, the dielectric has %d materials", n_mat, o->diel->n_mat); return -1; }
+    PCB_CHECK_ARG(o->diel->zsplit == c->zsplit, "dielectric was created under the other plane-mode form (plane_split); re-create it");
+    const bool plane = plane_layout(c);
+    const int gx = grid_for(c, c->nn, 256, 4);      // fixed for the context: the same partials for a column at any width
+    const int kmax = ncols < PCB_MAXC ? ncols : PCB_MAXC;
+    const size_t E = (size_t)PCB_MAXC * (size_t)n_mat;
+    if (ensure_partial(c, sizeof(double) * ((size_t)gx + 1) * E)) return -1;
+    if (ensure_scratch(c, sizeof(cplx) * (size_t)c->R * (size_t)kmax)) return -1;
+    std::vector<double> h(E);
+    double* dout = c->partial + (size_t)gx * E;
+    for (int j0 = 0; j0 < ncols; j0 += PCB_MAXC) {
+        const int kc = (ncols - j0 < PCB_MAXC) ? ncols - j0 : PCB_MAXC;
+        PcbCols cols;
+        memset(&cols, 0, sizeof cols);
+        for (int j = 0; j < kc; ++j) cols.in[j] = (const cplx*)x[j0 + j];
+        if (run_steps(o, forward_steps(plane), cols, kc)) return -1;
+        PcbCols e;
+        memset(&e, 0, sizeof e);
+        for (int j = 0; j < kc; ++j) e.in[j] = c->scratch + (size_t)j * c->R;
+        const int ne = kc * n_mat;
+        dim3 grid((unsigned)gx, (unsigned)kc, 1), blk(256, 1, 1);
+        const bool reg = n_mat <= PCB_ME_REG;      // bins in registers, else the match path
+        if (plane && reg) PCB_LAUNCH(k_material_energy_t<PCB_ME_REG>, grid, blk, 0, c->stream, o->d, e, kc, n_mat, c->partial);
+        else if (plane) PCB_LAUNCH(k_material_energy_t<0>, grid, blk, 0, c->stream, o->d, e, kc, n_mat, c->partial);
+        else if (reg) PCB_LAUNCH(k_material_energy<PCB_ME_REG>, grid, blk, 0, c->stream, o->d, e, kc, n_mat, c->partial);
+        else PCB_LAUNCH(k_material_energy<0>, grid, blk, 0, c->stream, o->d, e, kc, n_mat, c->partial);
+        PCB_CUDA_OK(cudaGetLastError());
+        PCB_LAUNCH(k_sum_partials, dim3((unsigned)((ne + 63) / 64), 1, 1), dim3(64, 1, 1), 0, c->stream, (const double*)c->partial, gx, ne, dout);
+        PCB_CUDA_OK(cudaGetLastError());
+        c->launches += 2;
+        PCB_CUDA_OK(cudaMemcpyAsync(h.data(), dout, sizeof(double) * (size_t)ne, cudaMemcpyDeviceToHost, c->stream));
+        PCB_CUDA_OK(cudaStreamSynchronize(c->stream));
+        for (int i = 0; i < ne; ++i) e_mat[(size_t)j0 * n_mat + i] = h[i] / (double)c->nn;
     }
     return 0;
 }

@@ -308,6 +308,28 @@ class DielHandle:
         self._ident_op = None
         return self
 
+    def set_inv_eps(self, inv_eps):
+        """Replace the 1 / eps table of a materials dielectric in place (pcb_diel_set_inv_eps): every operator built on this
+        handle applies the new values from its next launch.  Refused, with the old table kept, for another kind, a wrong length
+        or a value that is not finite and > 0."""
+        if self.kind != L.DIEL_MATERIALS:
+            raise ValueError("set_inv_eps: only a materials dielectric has a table of 1 / eps")
+        t = np.ascontiguousarray(inv_eps, dtype=np.float64).ravel()
+        L.check(L.lib().pcb_diel_set_inv_eps(self.h, t.ctypes.data_as(L.c_double_p), len(t)), "pcb_diel_set_inv_eps")
+        self.inv_eps = t.copy()
+
+    def at_frequency(self, f):
+        """Set every material's eps to its model's value at frequency f (models: dispersion.Drude / Lorentz / Constant, kept by
+        materials_handle) and return the eps.  Raises ValueError, the table unchanged, when some eps is not finite and > 0 there."""
+        models = getattr(self, "models", None)
+        if models is None:
+            raise ValueError("at_frequency: this handle has no permittivity models (materials_handle keeps them)")
+        eps = np.array([float(m.eps(f)) for m in models])
+        if not np.all(np.isfinite(eps) & (eps > 0.0)):
+            raise ValueError(f"at_frequency({f}): eps = {eps} is not finite and > 0 for every material")
+        self.set_inv_eps(1.0 / eps)
+        return eps
+
     def __call__(self, x):
         from . import pcfft
         return pcfft.diel_apply(self, x)
@@ -325,21 +347,32 @@ def materials_handle(n, d_flag, eps_opt=None, regions=None, background=1.0, devi
     """Several isotropic materials: the edge DoFs of regions[i] (index arrays into the 3 n^3 rows; later regions override earlier
     ones where they overlap) are divided by eps_opt[i], every other row by `background`.  Defaults: the regions of
     dielectric.material_regions (bcc_dg: its two gyroid networks; every other lattice: Omega_1) and the lattice's chiral eps for
-    each of them -- the same M as chiral_handle(n, d_flag)."""
+    each of them -- the same M as chiral_handle(n, d_flag).
+
+    Every entry of eps_opt and `background` may be a number or a dispersion model (dispersion.Drude / Lorentz); the handle keeps
+    one model per material in `models` (index 0: the background) and starts from eps_inf of each; `at_frequency(f)` sets the
+    table to eps(f)."""
+    from . import dispersion as dsp
     regions = diel.material_regions(n, d_flag) if regions is None else list(regions)
     if len(regions) > 255:
         raise ValueError(f"{len(regions)} regions: at most 255 besides the background")
     if eps_opt is None or (np.isscalar(eps_opt) and eps_opt == 0):
-        eps = np.full(len(regions), float(diel.diel_chiral_const(d_flag)))
+        eps = [float(diel.diel_chiral_const(d_flag))] * len(regions)
     else:
-        eps = np.atleast_1d(np.asarray(eps_opt, dtype=np.float64))
-        if eps.ndim != 1 or eps.size != len(regions):
-            raise ValueError(f"eps_opt has {eps.size} values for {len(regions)} regions")
+        eps = np.atleast_1d(np.asarray(eps_opt, dtype=object))      # numbers (0-d arrays too) or models
+        if eps.ndim != 1:
+            raise ValueError(f"eps_opt has shape {eps.shape}: expected one value per region")
+        eps = eps.tolist()
+        if len(eps) != len(regions):
+            raise ValueError(f"eps_opt has {len(eps)} values for {len(regions)} regions")
+    models = [dsp.as_model(background)] + [dsp.as_model(e) for e in eps]
     mat = np.zeros(3 * n ** 3, dtype=np.uint8)
     for i, reg in enumerate(regions):
         mat[np.asarray(reg, dtype=np.int64)] = i + 1
-    inv_eps = np.concatenate(([1.0 / background], 1.0 / eps))
-    return DielHandle.materials(n, mat, inv_eps, device=device)
+    inv_eps = 1.0 / np.array([m.eps_inf for m in models])
+    h = DielHandle.materials(n, mat, inv_eps, device=device)
+    h.models = models
+    return h
 
 
 def _eps_loc(d_flag, eps_opt, eps_mat):

@@ -6,7 +6,9 @@ and bandgap :313-496 keep their names, arguments, printed tables and the JSON ch
 ``kpath_chunks`` / ``bandgap_sharded`` distribute the k-path over the GPUs of a node, one k-chunk per
 process, with no data-path collective (SURVEY.md 8e-i); ``energy_fraction`` / ``mode_fields`` tell where a band's
 electric energy lives (opt-in output of ``eigen_1p`` / ``bandgap`` with ``energy=True``); ``group_velocity`` gives the bands'
-group velocities by Hellmann-Feynman (opt-in output with ``velocity=True``).
+group velocities by Hellmann-Feynman (opt-in output with ``velocity=True``); ``material_energy`` splits that energy per material,
+and a materials dielectric with dispersive models (dispersion.Drude / Lorentz) makes ``eigen_1p`` / ``bandgap`` solve for the
+self-consistent frequencies (dispersion.self_consistent).
 """
 import json
 import os
@@ -19,6 +21,7 @@ from . import _lib as L
 from . import devarray
 from . import dielectric as diel
 from . import discretization as mfd
+from . import dispersion as dsp
 from .devarray import DeviceBlock
 from .environment import (CYAN, GAP, GREEN, K, NEV, OUTPUT_PATH, RED, RESET, SCAL, TOL, TYPE0, YELLOW, owari_cuda, say)
 from .lobpcg import lobpcg_sep_softlock, _residual_helper
@@ -134,6 +137,16 @@ def energy_fraction(x, A_func):
     return e_in / e_tot
 
 
+def material_energy(x, A_func):
+    """(k, n_mat) fractions e_m / e_tot of each column's electric energy per material of a materials dielectric, with
+    e_m = Re sum over the rows of material m of conj(D_r) E_r / N^3 (pcb_material_energy); rows sum to 1.  Index 0 is the
+    background, so the sum over m != 0 is energy_fraction.  For a band that is not degenerate, dlambda/deps_m = -lambda f_m / eps_m;
+    within a degenerate set the sum over the set is basis-independent.  x: DeviceBlock or host array (3n^3, k); A_func: the first
+    callable of pc_mfd_handle."""
+    e = _operator_of(A_func, "material_energy").material_energy(x)
+    return e / e.sum(axis=1, keepdims=True)
+
+
 def mode_fields(x, A_func, which="D"):
     """Real-space fields of the columns of x as a new DeviceBlock in the natural layout: which = "D" gives D = FFT3(K_A^H x),
     "E" gives E = M D.  ``.get()[:, j].reshape(3, n, n, n)`` is column j indexed [c][i2][i1][i0]."""
@@ -226,13 +239,111 @@ def group_velocity(x, A_func, direction=None, side=+1, degen_tol=1e-6):
     return _group_velocity(x, A_func, direction, side, degen_tol)[0]
 
 
+def _dispersive_handle(Diels):
+    return Diels is not None and dsp.is_dispersive(getattr(Diels, "models", None) or [])
+
+
+def _warm_block(ctx, x, m, seed):
+    """A warm start of m columns from the solver's last block x (random columns appended when x is narrower)."""
+    if m <= x.shape[1]:
+        return x[:, 0:m]
+    x0 = ctx.empty(m)
+    x0[:, :x.shape[1]] = x
+    x0[:, x.shape[1]:] = ctx.random_block(m - x.shape[1], _next_seed(seed))
+    return x0
+
+
+def _penalty_ops(a_raw, alpha, Diels):
+    """ops(scale) -> (A_func, H_func, P_func) at k-point alpha (a_raw: the unscaled symbols with alpha), with the penalty of
+    set_relaxation multiplied by scale.  The penalty acts on the gradient modes only (A vanishes there), so A's eigenpairs do not
+    depend on it; a material with eps < 1 lifts the transverse bands by 1 / eps, and the penalty has to follow them."""
+    cache = {}
+
+    def ops(scale):
+        if scale not in cache:
+            relax_opt, pnt = mfd.set_relaxation(alpha, scal=SCAL)
+            pnt = pnt * scale
+            b_fft = mfd.PenaltySymbols(a_raw)
+            inv_fft = mfd.inverse_3_times_3_B(b_fft, pnt, relax_opt[0])
+            cache.clear()
+            cache[scale] = pc_mfd_handle(a_raw / SCAL, (pnt * b_fft[0] / SCAL / SCAL, pnt * b_fft[1] / SCAL / SCAL), Diels,
+                                         (inv_fft[0] * SCAL * SCAL, inv_fft[1] * SCAL * SCAL), relax_opt[0])
+        return cache[scale]
+    return ops
+
+
+def _solve_dispersive(Diels, ops, solver, x0, nev, tol, shift, start=None, window=None, seed=None):
+    """Self-consistent frequencies of the lowest nev bands for a materials dielectric with dispersive models
+    (dispersion.self_consistent).  Every solve is a LOBPCG run warm-started from the previous one's vectors, at the eps of every
+    material at the frequency the iteration asks for (Diels.at_frequency), on the operators ops(max(1, 1 / min_m eps_m))
+    (_penalty_ops).  start None, or one with a NaN (no frequency of that
+    band at the previous point): one solve at eps_inf, and every band starts where the fields of that solve predict its root
+    (dispersion.predict); else the given frequencies.  Bands whose plain-solve frequency is below
+    ZERO_MODE_FREQ (the zero modes at Gamma) get NaN.  Returns a dict: freq, steps, eps (nev, n_mat), frac (nev, n_mat), x, the
+    total LOBPCG iterations and seconds, and the lambdas of the last solve."""
+    m = x0.shape[1]
+    tot = [0.0, 0.0]
+    last = {}
+
+    def run(x_start, A_func, H_func, P_func):
+        lam, x, iters = solver(H_func, P_func, x_start, nev, tol=tol)
+        if lam is None:
+            # a warm start that already holds the eigenvectors (a homogeneous medium only rescales A) leaves [X W] rank
+            # deficient: once more from a random start, as bandgap_sharded does for a failed point
+            lam, x, iters = solver(H_func, P_func, x_start.ctx.random_block(m, _next_seed(seed)), nev, tol=tol)
+        if lam is None:
+            raise RuntimeError("solver returned None (NaN / blow-up)")
+        tot[0] += float(iters[0])
+        tot[1] += float(iters[1])
+        last["lambdas"] = lam
+        _, w_re = recompute_normalize_print(lam[:nev], x[:, :nev], A_func, shift)
+        return np.asarray(w_re, dtype=float), x
+
+    def solve(f, x):
+        eps = Diels.at_frequency(f)
+        A_func, H_func, P_func = ops(max(1.0, 1.0 / float(eps.min())))
+        F, x = run(_warm_block(x.ctx, x, m, seed), A_func, H_func, P_func)
+        frac = material_energy(x[:, :nev], A_func)
+        F = np.where(F < ZERO_MODE_FREQ, 0.0, F)
+        return F, frac, x
+
+    window = dsp.default_window(Diels.models) if window is None else window
+    x = x0
+    if start is None or np.any(np.isnan(start)):
+        eps_inf = np.array([mdl.eps_inf for mdl in Diels.models])
+        Diels.set_inv_eps(1.0 / eps_inf)
+        A_func, H_func, P_func = ops(max(1.0, 1.0 / float(eps_inf.min())))
+        F, x = run(x0, A_func, H_func, P_func)
+        F = np.where(F < ZERO_MODE_FREQ, 0.0, F)
+        start = dsp.predict(F, material_energy(x[:, :nev], A_func), eps_inf, Diels.models, window)
+    start = np.asarray(start, dtype=float)
+    res = dsp.self_consistent(solve, Diels.models, start, window=window, x0=x, zero=ZERO_MODE_FREQ)
+    freq = res["freq"]
+    eps = np.full((nev, len(Diels.models)), np.nan)
+    for j in np.flatnonzero(np.isfinite(freq)):
+        eps[j] = [float(mdl.eps(freq[j])) for mdl in Diels.models]
+    return {"freq": freq, "steps": res["steps"], "eps": eps, "frac": res["frac"], "x": res["x"], "iterations": tot[0],
+            "seconds": tot[1], "lambdas": last.get("lambdas")}
+
+
 def eigen_1p(n, d_flag, alpha, type="chiral", nev=NEV, solver=lobpcg_sep_softlock, cpu_x0=False, x0=None, seed=None,
-             tol=TOL, eps_opt=0, energy=False, velocity=False):
+             tol=TOL, eps_opt=0, energy=False, velocity=False, diel_kw=None, window=None):
     """Eigenvalues at one lattice vector (numerical_experiments.py:209-247).  Prints like the reference and
     additionally returns a dict (lambdas, x, info, omega_pnt, omega_re, residuals, shift); with ``energy=True`` also
     "energy_fraction", the fraction of the electric energy in the dielectric of the first nev bands (energy_fraction); with
     ``velocity=True`` also "group_velocity" (nev, 3), the gradients of group_velocity, and "velocity_cluster", its cluster
-    label per band (bands with the same label are degenerate and report the cluster's trace average)."""
+    label per band (bands with the same label are degenerate and report the cluster's trace average).
+
+    diel_kw: further keyword arguments of the dielectric handle's constructor (e.g. {"regions": [], "background": Drude(1, 0.4)}
+    for materials_handle).  When a material of type="materials" is dispersive (dispersion.Drude / Lorentz in eps_opt or
+    diel_kw), the bands are the self-consistent ones, f_j = F_j(eps(f_j)) (dispersion.self_consistent, starting from one solve at
+    eps_inf), in `window` (default: the highest admissible window); "omega_re" / "omega_pnt" hold those frequencies (NaN where
+    no root was found, and for the zero modes at Gamma), "newton_steps" the solves per band, "eps" (nev, n_mat) the permittivities
+    at each band's own frequency, "info" the total iterations and seconds of all solves; energy=True gives the fractions at each
+    band's own eps.  "x", "lambdas" and "residuals" are those of the LAST solve only, made at the eps of the last band cluster's
+    frequency: they are not the modes of the other bands at their own frequencies (for a band's fields, solve once more at its
+    "eps" row).  velocity=True with a dispersive material raises ValueError (the group velocity needs the d eps / d omega
+    term)."""
     alpha = np.asarray(alpha, dtype=float)
     a_fft, b_fft, inv_fft, x_rand, shift = uniform_initialization(n, d_flag, alpha, nev=nev, seed=seed)
     if x0 is None:
@@ -240,7 +351,20 @@ def eigen_1p(n, d_flag, alpha, type="chiral", nev=NEV, solver=lobpcg_sep_softloc
     del x_rand
     if cpu_x0:
         (x0.get() if isinstance(x0, DeviceBlock) else np.asarray(x0)).tofile("x0_from_single_gpu.bin")
-    Diels = _handle(type, n, d_flag, eps_opt=eps_opt) if type is not None else None
+    Diels = _handle(type, n, d_flag, eps_opt=eps_opt, **(diel_kw or {})) if type is not None else None
+    if _dispersive_handle(Diels):
+        if velocity:
+            raise ValueError("velocity=True with a dispersive material: the group velocity needs the d eps / d omega term")
+        a_raw = mfd.fft_blocks(n, K, diel.diel_info(d_flag, option="ct"), alpha=alpha, scal=SCAL)[0]
+        r = _solve_dispersive(Diels, _penalty_ops(a_raw, alpha, Diels), solver, x0, nev, tol, shift, window=window, seed=seed)
+        say(f"n = {n}, lattice type: {d_flag}, self-consistent frequencies {r['freq']}, solves per band {r['steps']}, "
+            f"iter = {int(r['iterations'])}, runtime = {r['seconds']:<6.3f}s.")
+        out = {"lambdas": r["lambdas"], "x": r["x"], "info": np.array([r["iterations"], r["seconds"]]), "omega_pnt": r["freq"].copy(),
+               "omega_re": r["freq"], "residuals": recompute_normalize_print.last_residuals, "shift": shift,
+               "newton_steps": r["steps"], "eps": r["eps"]}
+        if energy:
+            out["energy_fraction"] = r["frac"][:, 1:].sum(axis=1)
+        return out
     A_func, H_func, P_func = pc_mfd_handle(a_fft, b_fft, Diels, inv_fft, shift)
     lambdas_pnt, x, iters = solver(H_func, P_func, x0, nev, tol=tol)
     del x0
@@ -324,7 +448,7 @@ def _load_or_init_record_its(path_bandgap, var_it, var_fq, n_k, type, d_flag, n)
 
 
 def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indices=None, nev=NEV, seed=None,
-            path=None, tol=TOL / SCAL / SCAL, only=None, energy=False, velocity=False):
+            path=None, tol=TOL / SCAL / SCAL, only=None, energy=False, velocity=False, diel_kw=None, window=None):
     """Band structure along the lattice's k-path, one warm-started LOBPCG solve per point, checkpointed to
     JSON after every point (numerical_experiments.py:313-496).  Returns the list of failed indices.
     `nev` (default NEV), `seed` (reproducible random starts) and `path` (output file) are additions.
@@ -333,7 +457,11 @@ def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indice
     `velocity=True` records under "<d_flag>_<n>_group_velocity", per k-point, d omega / ds of its nev bands along the path
     (group_velocity): point idx lies on segment s = idx // GAP with direction u_s = sym[s+1] - sym[s], and the derivative is
     taken from that segment's start side (side=-1), so segment end points and crossings get the value the path arrives with.
-    Zero modes are written as null; the row sentinels are those of the energy fractions."""
+    Zero modes are written as null; the row sentinels are those of the energy fractions.
+    diel_kw / window: as for eigen_1p.  With a dispersive material each point's frequency row holds the self-consistent
+    frequencies (null where there is none, and for the zero modes at Gamma), warm-started in both the vectors and the frequencies
+    from the previous point; its iteration row holds the total LOBPCG iterations and seconds of all the point's solves;
+    energy=True records the fractions at each band's own eps.  velocity=True is refused there (ValueError)."""
     t_all = time.time()
     timing = {"setup": 0.0, "assemble": 0.0, "solver": 0.0, "postprocess": 0.0, "checkpoint": 0.0}
     if energy:
@@ -344,7 +472,10 @@ def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indice
     ct, sym_points = diel.diel_info(d_flag)
     alphas = diel.kpath(d_flag, GAP)
     n_k = alphas.shape[0]
-    Diels = _handle(type, n, d_flag, eps_opt=eps_opt)
+    Diels = _handle(type, n, d_flag, eps_opt=eps_opt, **(diel_kw or {}))
+    dispersive = _dispersive_handle(Diels)
+    if dispersive and velocity:
+        raise ValueError("velocity=True with a dispersive material: the group velocity needs the d eps / d omega term")
     ctx = Diels.ctx if Diels is not None else devarray.get_context(n)
     d_fft, _ = mfd.fft_blocks(n, K, ct)
     timing["setup"] = time.time() - t_all
@@ -372,7 +503,7 @@ def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indice
     if max(indices) >= n_k or min(indices) < 0:
         raise ValueError("Index is non-positive or is incompatible with gap size.")
 
-    err_index, op, x = [], None, None
+    err_index, op, x, f_prev = [], None, None, None
     for i, idx in enumerate(indices):
         t_h = time.time()
         alpha = alphas[idx] / SCAL
@@ -380,6 +511,7 @@ def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indice
         m = nev + round(nev * relax_opt[1])
         if i == 0 or abs(indices[i] - indices[i - 1]) > 1 or x is None:
             x0 = ctx.random_block(m, _next_seed(None if seed is None else seed + idx))
+            f_prev = None
         elif m <= x.shape[1]:
             x0 = x[:, 0:m]
         else:
@@ -392,39 +524,52 @@ def bandgap(n, d_flag, solver=lobpcg_sep_softlock, type=TYPE0, eps_opt=0, indice
         a_fft = a_fft / SCAL
         b_fft = (pnt * b_fft[0] / SCAL / SCAL, pnt * b_fft[1] / SCAL / SCAL)
         inv_fft = (inv_fft[0] * SCAL * SCAL, inv_fft[1] * SCAL * SCAL)
-        A_func, H_func, P_func = pc_mfd_handle(a_fft, b_fft, Diels, inv_fft, relax_opt[0])
+        # a dispersive point builds its operators per solve (_penalty_ops)
+        A_func, H_func, P_func = (None, None, None) if dispersive else pc_mfd_handle(a_fft, b_fft, Diels, inv_fft, relax_opt[0])
         say(f"Matrix blocks done, {owari() - t_h:<6.3f}s elapsed.")
         timing["assemble"] += time.time() - t_h
         try:
             t_s = time.time()
-            lambdas_pnt, x, iters = solver(H_func, P_func, x0, nev, tol=tol)
-            timing["solver"] += time.time() - t_s
-            if lambdas_pnt is None:
-                raise RuntimeError("solver returned None (NaN / blow-up)")
-            say(f"Gap {idx + 1} out of {n_k} ({d_flag}),"
-                f"alpha = ({alpha[0] / pi:<6.3f}, {alpha[1] / pi:<6.3f}, {alpha[2] / pi:<6.3f})pi is computed.")
-            say(f"Iterations = {int(iters[0])}, runtime = {iters[1]:<6.3f}s.\n")
-            t_s = time.time()
-            _, lambdas_re = recompute_normalize_print(lambdas_pnt, x, A_func, relax_opt[0])
-            timing["postprocess"] += time.time() - t_s
-            if energy:
+            if dispersive:
+                r = _solve_dispersive(Diels, _penalty_ops(d_fft.with_alpha(alpha), alpha, Diels), solver, x0, nev, tol,
+                                      relax_opt[0], start=f_prev, window=window, seed=None if seed is None else seed + idx)
+                timing["solver"] += time.time() - t_s
+                x, f_prev = r["x"], r["freq"]
+                say(f"Gap {idx + 1} out of {n_k} ({d_flag}): self-consistent frequencies {r['freq']}, solves per band "
+                    f"{r['steps']}, iterations = {int(r['iterations'])}, runtime = {r['seconds']:<6.3f}s.\n")
+                if energy:
+                    gap_rec_en[idx] = [None if np.isnan(v) else float(v) for v in r["frac"][:, 1:].sum(axis=1)]
+                gap_rec_it[idx] = [r["iterations"], r["seconds"]]
+                gap_rec_fq[idx] = [None if np.isnan(v) else float(v) for v in r["freq"]]
+            else:
+                lambdas_pnt, x, iters = solver(H_func, P_func, x0, nev, tol=tol)
+                timing["solver"] += time.time() - t_s
+                if lambdas_pnt is None:
+                    raise RuntimeError("solver returned None (NaN / blow-up)")
+                say(f"Gap {idx + 1} out of {n_k} ({d_flag}),"
+                    f"alpha = ({alpha[0] / pi:<6.3f}, {alpha[1] / pi:<6.3f}, {alpha[2] / pi:<6.3f})pi is computed.")
+                say(f"Iterations = {int(iters[0])}, runtime = {iters[1]:<6.3f}s.\n")
                 t_s = time.time()
-                frac = energy_fraction(x[:, :nev], A_func)
-                timing["energy"] += time.time() - t_s
-                gap_rec_en[idx] = [float(v) for v in frac]
-            if velocity:
-                t_s = time.time()
-                seg = sym[idx // GAP + 1] - sym[idx // GAP]
-                vel = group_velocity(x[:, :nev], A_func, direction=seg, side=-1)
-                timing["velocity"] += time.time() - t_s
-                gap_rec_vel[idx] = [None if np.isnan(v) else float(v) for v in vel]
-            gap_rec_it[idx] = [float(v) for v in iters[:2]]
-            gap_rec_fq[idx] = [float(v) for v in lambdas_re]
+                _, lambdas_re = recompute_normalize_print(lambdas_pnt, x, A_func, relax_opt[0])
+                timing["postprocess"] += time.time() - t_s
+                if energy:
+                    t_s = time.time()
+                    frac = energy_fraction(x[:, :nev], A_func)
+                    timing["energy"] += time.time() - t_s
+                    gap_rec_en[idx] = [float(v) for v in frac]
+                if velocity:
+                    t_s = time.time()
+                    seg = sym[idx // GAP + 1] - sym[idx // GAP]
+                    vel = group_velocity(x[:, :nev], A_func, direction=seg, side=-1)
+                    timing["velocity"] += time.time() - t_s
+                    gap_rec_vel[idx] = [None if np.isnan(v) else float(v) for v in vel]
+                gap_rec_it[idx] = [float(v) for v in iters[:2]]
+                gap_rec_fq[idx] = [float(v) for v in lambdas_re]
         except Exception as e:          # same policy as the reference: record [-1,-1], restart from random
             say(f"{RED}WARNING: Error occurs.")
             say(f"Error message: {e}{RESET}")
             err_index.append(idx)
-            x = None
+            x, f_prev = None, None
             gap_rec_it[idx] = [-1.0, -1.0]
             gap_rec_fq[idx] = [-1.0] * nev
             if energy:
@@ -484,12 +629,12 @@ def merge_records(parts, n_k, nev=NEV):
 
 
 def bandgap_sharded(n, d_flag, rank, world, type=TYPE0, eps_opt=0, nev=NEV, seed=1000, out_dir=None, indices=None,
-                    gather=None, tol=TOL / SCAL / SCAL, retry=1, energy=False, velocity=False):
+                    gather=None, tol=TOL / SCAL / SCAL, retry=1, energy=False, velocity=False, diel_kw=None, window=None):
     """k-path sharding over `world` processes (one GPU each): rank r solves chunk r of the path (or of `indices`)
     into its own JSON file; with `gather` (callable: obj -> list of objs on rank 0, e.g. a torch.distributed
     gather_object wrapper) rank 0 merges all rows into the reference-format file.  No collective touches the data path.
     energy=True: bandgap(..., energy=True) on every rank, and the energy-fraction rows are merged as well; velocity=True the
-    same for the group-velocity rows."""
+    same for the group-velocity rows.  diel_kw / window: as for bandgap (dispersive materials)."""
     all_idx = list(range(diel.kpath(d_flag, GAP).shape[0])) if indices is None else list(indices)
     mine = [all_idx[i] for i in kpath_chunks(len(all_idx), world)[rank]]
     out_dir = out_dir or (OUTPUT_PATH + type + "/")
@@ -498,7 +643,7 @@ def bandgap_sharded(n, d_flag, rank, world, type=TYPE0, eps_opt=0, nev=NEV, seed
     if os.path.exists(part_path):
         os.remove(part_path)
     errs = bandgap(n, d_flag, type=type, eps_opt=eps_opt, indices=mine, nev=nev, seed=seed, path=part_path, tol=tol,
-                   energy=energy, velocity=velocity) if mine else []
+                   energy=energy, velocity=velocity, diel_kw=diel_kw, window=window) if mine else []
     # A warm start can make [X W] numerically rank deficient (e.g. the point after Gamma, whose zero modes are pure gradients):
     # the reference records [-1,-1] and recomputes such rows from a random start when bandgap() is called again
     # (numerical_experiments.py:370-390); do that second call here.
@@ -506,7 +651,7 @@ def bandgap_sharded(n, d_flag, rank, world, type=TYPE0, eps_opt=0, nev=NEV, seed
         if not errs:
             break
         errs = bandgap(n, d_flag, type=type, eps_opt=eps_opt, indices=None, nev=nev, seed=seed + 7919 * (attempt + 1),
-                       path=part_path, tol=tol, only=errs, energy=energy, velocity=velocity)
+                       path=part_path, tol=tol, only=errs, energy=energy, velocity=velocity, diel_kw=diel_kw, window=window)
     rows = {"iterations": {}, "frequencies": {}, "errors": errs}
     if energy:
         rows["energy_fraction"] = {}

@@ -115,6 +115,18 @@ class Operator:
                                                e_tot.ctypes.data_as(L.c_double_p)), "pcb_field_energy")
         return e_in, e_tot
 
+    def material_energy(self, X):
+        """(k, n_mat) NumPy array: e_m = Re sum over the rows of material m of conj(D_r) E_r / N^3 per column, for an operator
+        on a materials dielectric -- see pcb_material_energy in include/pcb200.h.  Row sums are e_tot of field_energy.  X: a
+        DeviceBlock on this operator's context (column views welcome) or a host array (3n^3, k) / (3n^3,), uploaded."""
+        X, _ = devarray.as_block(self.ctx, X)
+        n_mat = len(self.diel.inv_eps) if self.diel is not None and hasattr(self.diel, "inv_eps") else 0
+        e = np.zeros((X.k, n_mat))
+        if X.k:
+            L.check(self._lib.pcb_material_energy(self.h, X.k, L.ptr_array(X.ptrs), n_mat, e.ctypes.data_as(L.c_double_p)),
+                    "pcb_material_energy")
+        return e
+
     def band_velocity(self, X):
         """(V, xx, xax) of the columns of X (n <= 32): V (3, n, n) complex, V[d] = X^H (dA/dalpha_d) X (Hermitian), xx[j] =
         x_j^H x_j, xax[j] = Re x_j^H A x_j -- see pcb_band_velocity in include/pcb200.h.  dA/dalpha_d comes from
